@@ -2,7 +2,7 @@
 """Benchmark of the B200 OCT metric suite on the BASELINE.json configurations.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
-                    [--config cfg4|cfg1|cfg2|cfg3|cfg5] [--items M] [--noise f] [--uniform-random]
+                    [--config cfg4|cfg1|cfg2|cfg3|cfg5] [--items M] [--noise f] [--uniform-random] [--dump-outputs DIR]
 
 Default = cfg4 AS STATED in BASELINE.json: the full metric suite (fused label pass + contour metrics + float64
 epilogue) over 100,000 synthetic 496x512 8-class B-scans, sharded over the N ranks (ceil(100000 / N) per GPU:
@@ -14,6 +14,11 @@ host-array API (pinned host buffers, H2D inside the timed region, metrics read b
 
 --config cfg1 / cfg2 / cfg3 / cfg5: the other BASELINE configurations (single volumes; their committed lines live
 under profiles/).  cfg5 shards its 2 K (class, direction) distance transforms over the ranks.
+
+--dump-outputs DIR writes what the last timed step returned to its caller as DIR/<name>.npy (float64): the per-item
+metrics (``item_*``; a fixed, seeded sample of DUMP_ITEMS items of larger batches, ``item_index`` names them) and the
+dataset totals (``dataset_*``); cfg5: the per-class surface integers and metrics.  The inputs depend only on the
+arguments, so two builds of the project can be compared output for output.  With N > 1, rank 0 writes its own shard.
 
 --impl reference times the reference's own CPU path on the box's host cores: the UNMODIFIED Metrics/*.py modules
 (baseline/_ref/Metrics, importable for 4 of the 5 modules) called the only way the reference can be called -- per
@@ -34,8 +39,10 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True        # the benchmark leaves the tree as it found it (it may be read-only)
 
 CFG4_ITEMS = 100_000
+DUMP_ITEMS = 8192                     # per-item rows written by --dump-outputs
 CONFIGS = {
     # name: H, W, K, items of the configuration as BASELINE.json states it, generator, what a step computes
     "cfg1": dict(H=496, W=768, K=8, items=61, gen="layered", noise=0.01, seed=1001, contours=False,
@@ -282,6 +289,36 @@ def run_reference(args):
     }))
 
 
+# ------------------------------------------------------------------------------------ outputs of the timed path
+def step_outputs(name, pend, out):
+    """Host float64 copies of what the last timed step returned: ``pend`` is what ``step()`` returned, ``out`` what
+    ``settle()`` made of it."""
+    import numpy as np
+    from retinal_oct_image_segmentation_via_deep_learning_b200 import suite
+    f64 = lambda v: np.asarray(v, dtype=np.float64)          # noqa: E731
+    if name == "cfg5":
+        ints = {k: v.cpu().numpy() for k, v in out.items()}
+        arrays = {"surface_" + k: f64(v.view(np.uint32) if v.dtype == np.int32 else v) for k, v in ints.items()}
+        arrays.update({k: f64(v) for k, v in suite.surface_metrics_3d(out).items()})
+        return arrays
+    res = pend.res
+    n = res.num_items
+    idx = np.arange(n) if n <= DUMP_ITEMS else np.sort(np.random.default_rng(0).choice(n, DUMP_ITEMS, replace=False))
+    arrays = {"item_index": f64(idx)}
+    arrays.update({"item_" + k: f64(v[idx]) for k, v in res.metrics().items()})
+    arrays.update({"dataset_" + k: f64(v) for k, v in out.items()})
+    return arrays
+
+
+def write_outputs(directory, arrays):
+    import numpy as np
+    total = sum(v.nbytes for v in arrays.values())
+    assert total <= 64 << 20, f"{total} bytes of outputs: lower DUMP_ITEMS"
+    os.makedirs(directory, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(directory, k + ".npy"), v)
+
+
 # ------------------------------------------------------------------------------------ GPU arm
 def run_b200(args):
     import numpy as np
@@ -406,6 +443,7 @@ def run_b200(args):
     ev1.record()
     barrier()
     out = settle(pend)
+    dumped = step_outputs(name, pend, out) if args.dump_outputs and rank == 0 else None
     if keep is not None and len(ring) == 1:
         kh = keep.cpu().numpy()
         assert all((kh[i] == kh[0]).all() for i in range(args.steps)), "steps disagree on the dataset totals"
@@ -596,6 +634,8 @@ def run_b200(args):
         else:
             mm = suite.surface_metrics_3d(out)
             line["hausdorff_distance"] = [float(x) for x in mm["hausdorff_distance"]]
+        if dumped is not None:
+            write_outputs(args.dump_outputs, dumped)
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
@@ -619,7 +659,13 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-secondary", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's outputs to DIR/<name>.npy (float64, seeded sample of large batches)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl b200)")
     if args.impl == "reference":
         run_reference(args)
     else:
