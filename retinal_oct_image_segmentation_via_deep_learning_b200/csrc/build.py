@@ -47,7 +47,7 @@ def build_library(force=False, verbose=False):
 
     def compile_one(src):
         obj = os.path.join(objdir, src.replace(".cu", ".o"))
-        extra = os.environ.get("OCTM_NVCC_EXTRA", "").split()       # tuning builds, e.g. -DOCTM_SEARCH_MINB=6
+        extra = os.environ.get("OCTM_NVCC_EXTRA", "").split()       # debug builds, e.g. -DOCTM_WALK_STATS
         cmd = [nvcc, *NVCC_FLAGS, *extra, "-c", os.path.join(HERE, src), "-o", obj]
         if verbose:
             cmd.insert(1, "-Xptxas=-v")

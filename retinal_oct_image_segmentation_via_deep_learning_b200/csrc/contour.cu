@@ -14,16 +14,15 @@
 //   K5  trace_kernel     one thread per (item, class, map): locate the raster-first mixed square
 //                        from the label pass's first-occurrence table, walk the polyline forward
 //                        (and backward if it is open), emit doubled-lattice vertices.
-//   K6  distance_search_kernel  one CTA per (item, class, direction): source contour staged in shared
-//                        memory tile by tile; exact integer squared distances with the expansion
-//                        |a|^2 - 2 a.q + |q|^2 (2 IMAD + 1 IMNMX per pair), pruned by bounding boxes.
+//   K6  distance_column_kernel  one CTA per (item, class, direction): source contour sorted by column in
+//                        shared memory; exact integer squared distances with the expansion
+//                        |a|^2 - 2 a.q + |q|^2 (2 IMAD + 1 IMNMX per pair), pruned by column span.
+//   K6' distance_search_kernel  the same per unit for contours whose sorted form does not fit shared
+//                        memory: source staged tile by tile, pruned by bounding boxes.
 //   K7  distance_select_kernel  one warp per (item, class, direction): max, sum of sqrt(D2/4) in
 //                        float64, and a radix select of the two order statistics numpy's linear 95th
 //                        percentile interpolates between.
-//       distance_kernel  single-kernel brute-force / per-lane-pruned variants (OCTM_DISTANCE_MODE),
-//                        kept as independent checks of the default path.
 #include <cstdlib>
-#include <cstring>
 #include <numeric>
 #include <type_traits>
 
@@ -94,14 +93,11 @@ __device__ __forceinline__ uint32_t label_of(const uint4& w, uint32_t c) {
 
 // WORDS: W % 16 == 0 and 16-byte aligned maps -> the walk reads aligned 16-byte label groups and keeps the last
 // group of the even and of the odd row in registers (load_rows16).
-#ifndef OCTM_TRACE_MINB
-#define OCTM_TRACE_MINB 8
-#endif
 #ifdef OCTM_WALK_STATS
 __device__ unsigned long long g_walk_stats[8];
 #endif
 template <bool WORDS>
-__global__ void __launch_bounds__(128, OCTM_TRACE_MINB) trace_kernel(const TraceParams prm) {
+__global__ void __launch_bounds__(128, 8) trace_kernel(const TraceParams prm) {
     __shared__ uint32_t s_step[64];      // step_word table: (case, entry edge) -> exit edge, vertex offset, order
     if (prm.todo_count != nullptr && *prm.todo_count == 0) return;
     if (threadIdx.x < 64) s_step[threadIdx.x] = step_word(threadIdx.x);
@@ -251,14 +247,11 @@ __global__ void __launch_bounds__(128, OCTM_TRACE_MINB) trace_kernel(const Trace
 // positions from a warp prefix sum (adjacent lanes write adjacent words).  Everything else (blobs, broken or
 // touching layers, too many vertices) gets n_pts = kTraceTodo and is walked by trace_kernel afterwards, which
 // overwrites whatever part of the list was written before the check failed.
-#ifndef OCTM_LAYERED_MINB
-#define OCTM_LAYERED_MINB 8
-#endif
 // EMIT = false: verification only.  A verified contour gets n_pts = (vertex count | kLayeredBit) and no vertices
 // are written: layered_distance_kernel works from the boundary rows and emits vertices only for the pairs it
 // cannot finish itself.
 template <bool EMIT>
-__global__ void __launch_bounds__(128, OCTM_LAYERED_MINB) trace_layered_kernel(const TraceParams prm) {
+__global__ void __launch_bounds__(128, 8) trace_layered_kernel(const TraceParams prm) {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int K = prm.K, H = prm.H, W = prm.W;
     const uint32_t cap = static_cast<uint32_t>(prm.max_pts);
@@ -428,20 +421,6 @@ __global__ void __launch_bounds__(256) first_pos_kernel(const uint8_t* __restric
 }
 
 // ------------------------------------------------------------------------------ distances
-struct DistParams {
-    const uint32_t* verts;   // [n][K][2][max_pts]
-    const uint32_t* n_pts;   // [n][K][2]
-    long long n_pairs;       // n * K
-    int max_pts;
-    uint32_t* max_sq;        // [n][K][2]
-    uint32_t* p95_sq;        // [n][K][2][2]
-    double* sum_dist;        // [n][K][2]
-    uint32_t* sq_out;        // [n][K][2][max_pts] or null
-};
-
-constexpr int kDistThreads = 128;
-constexpr int kQ = 4;   // queries per thread per sweep
-
 template <int T>
 __device__ __forceinline__ uint32_t block_reduce_max(uint32_t v, uint32_t* scratch) {
     v = __reduce_max_sync(0xffffffffu, v);
@@ -532,7 +511,6 @@ __device__ uint32_t block_select(const uint32_t* vals, int m, uint32_t k, uint32
 }
 
 constexpr int kBox = 16;      // vertices per bounding box (consecutive in trace order => compact)
-constexpr int kSuper = 8;     // boxes per super-box
 
 // squared distance from q to an axis-aligned box {ymin, ymax, xmin, xmax}: exact lower bound of the
 // squared distance to every vertex inside it
@@ -542,178 +520,9 @@ __device__ __forceinline__ int box_lb2(int4 bx, int qy, int qx) {
     return dy * dy + dx * dx;
 }
 
-// PRUNE = false: brute force (every query against every source vertex).
-// PRUNE = true : the same minimum, skipping boxes whose lower bound cannot beat the current best.
-template <bool PRUNE>
-__global__ void __launch_bounds__(kDistThreads) distance_kernel(const DistParams prm) {
-    extern __shared__ __align__(16) uint8_t dsm[];
-    __shared__ uint32_t s_hist[256];
-    __shared__ uint32_t s_scr[8];
-    __shared__ double s_dscr[8];
-    __shared__ uint32_t s_bc[2];
-    const int cap = prm.max_pts;
-    const int capb = (cap + kBox - 1) / kBox, caps = (capb + kSuper - 1) / kSuper;
-    // shared-memory carve-up (offsets, so every access stays an LDS/STS rather than a generic load)
-    int2* const pts0 = reinterpret_cast<int2*>(dsm);                                     // {y<<16|x, y^2+x^2}
-    uint32_t* const d2 = reinterpret_cast<uint32_t*>(dsm + static_cast<size_t>(cap) * 16);
-    int4* const boxes0 = reinterpret_cast<int4*>(dsm + static_cast<size_t>(cap) * 20);
-    int4* const sboxes0 = boxes0 + 2 * capb;
-#define PTS(mm) (pts0 + (mm) * cap)
-#define BOXES(mm) (boxes0 + (mm) * capb)
-#define SBOXES(mm) (sboxes0 + (mm) * caps)
-
-    for (long long pair = blockIdx.x; pair < prm.n_pairs; pair += gridDim.x) {
-        const uint32_t n0 = prm.n_pts[pair * 2 + 0], n1 = prm.n_pts[pair * 2 + 1];
-        const int n[2] = {static_cast<int>(min(n0, (uint32_t)cap)), static_cast<int>(min(n1, (uint32_t)cap))};
-        if (n[0] == 0 || n[1] == 0) {
-            if (threadIdx.x < 2) {
-                prm.max_sq[pair * 2 + threadIdx.x] = 0;
-                prm.p95_sq[pair * 4 + threadIdx.x * 2] = prm.p95_sq[pair * 4 + threadIdx.x * 2 + 1] = 0;
-                prm.sum_dist[pair * 2 + threadIdx.x] = 0.0;
-            }
-            continue;
-        }
-        __syncthreads();
-        for (int mm = 0; mm < 2; ++mm) {
-            const uint32_t* src = prm.verts + (pair * 2 + mm) * static_cast<long long>(cap);
-            for (int i = threadIdx.x; i < n[mm]; i += kDistThreads) {
-                const uint32_t v = src[i];
-                const int y = v >> 16, x = v & 0xffff;
-                PTS(mm)[i] = make_int2(static_cast<int>(v), y * y + x * x);
-            }
-        }
-        __syncthreads();
-        if (PRUNE) {
-            for (int mm = 0; mm < 2; ++mm) {
-                const int nb = (n[mm] + kBox - 1) / kBox;
-                for (int b = threadIdx.x; b < nb; b += kDistThreads) {
-                    int ymin = 0x7fffffff, ymax = -1, xmin = 0x7fffffff, xmax = -1;
-                    const int e = min(n[mm], (b + 1) * kBox);
-                    for (int i = b * kBox; i < e; ++i) {
-                        const uint32_t v = static_cast<uint32_t>(PTS(mm)[i].x);
-                        const int y = v >> 16, x = v & 0xffff;
-                        ymin = min(ymin, y); ymax = max(ymax, y); xmin = min(xmin, x); xmax = max(xmax, x);
-                    }
-                    BOXES(mm)[b] = make_int4(ymin, ymax, xmin, xmax);
-                }
-            }
-            __syncthreads();
-            for (int mm = 0; mm < 2; ++mm) {
-                const int nb = (n[mm] + kBox - 1) / kBox, nsb = (nb + kSuper - 1) / kSuper;
-                for (int sb = threadIdx.x; sb < nsb; sb += kDistThreads) {
-                    int4 acc = BOXES(mm)[sb * kSuper];
-                    const int e = min(nb, (sb + 1) * kSuper);
-                    for (int b = sb * kSuper + 1; b < e; ++b) {
-                        const int4 c = BOXES(mm)[b];
-                        acc.x = min(acc.x, c.x); acc.y = max(acc.y, c.y); acc.z = min(acc.z, c.z); acc.w = max(acc.w, c.w);
-                    }
-                    SBOXES(mm)[sb] = acc;
-                }
-            }
-            __syncthreads();
-        }
-        // direction 0: queries = pred vertices (map 1), sources = true vertices (map 0); direction 1 swapped
-        for (int dir = 0; dir < 2; ++dir) {
-            const int2* qs = PTS(1 - dir);
-            const int2* ss = PTS(dir);
-            const int nq = n[1 - dir], ns = n[dir];
-            if (PRUNE) {
-                const int4* bxs = BOXES(dir);
-                const int4* sbs = SBOXES(dir);
-                const float ratio = static_cast<float>(ns) / static_cast<float>(nq);
-                const int nb = (ns + kBox - 1) / kBox, nsb = (nb + kSuper - 1) / kSuper;
-                for (int j = threadIdx.x; j < nq; j += kDistThreads) {
-                    const int2 q = qs[j];
-                    const int qy = static_cast<uint32_t>(q.x) >> 16, qx = q.x & 0xffff;
-                    const int cy = -2 * qy, cx = -2 * qx;
-                    // prime the bound with the vertex at the same relative position along the other contour
-                    const int2 g = ss[min(ns - 1, static_cast<int>(static_cast<float>(j) * ratio))];
-                    int bm = (g.x & 0xffff) * cx + (static_cast<int>(static_cast<uint32_t>(g.x) >> 16) * cy + g.y);
-                    int bestd = bm + q.y;
-                    for (int sb = 0; sb < nsb; ++sb) {
-                        if (box_lb2(sbs[sb], qy, qx) >= bestd) continue;
-                        const int be = min(nb, (sb + 1) * kSuper);
-                        for (int b = sb * kSuper; b < be; ++b) {
-                            if (box_lb2(bxs[b], qy, qx) >= bestd) continue;
-                            const int e = min(ns, (b + 1) * kBox);
-#pragma unroll 4
-                            for (int i = b * kBox; i < e; ++i) {
-                                const int2 s = ss[i];
-                                const int ay = static_cast<uint32_t>(s.x) >> 16, ax = s.x & 0xffff;
-                                bm = min(bm, ax * cx + (ay * cy + s.y));
-                            }
-                            bestd = bm + q.y;
-                        }
-                    }
-                    d2[j] = static_cast<uint32_t>(bestd);
-                }
-            } else {
-            for (int base = 0; base < nq; base += kDistThreads * kQ) {
-                int cy[kQ], cx[kQ], best[kQ], qn[kQ];
-#pragma unroll
-                for (int t = 0; t < kQ; ++t) {
-                    const int j = min(base + t * kDistThreads + static_cast<int>(threadIdx.x), nq - 1);
-                    const int2 q = qs[j];
-                    cy[t] = -2 * static_cast<int>(static_cast<uint32_t>(q.x) >> 16);
-                    cx[t] = -2 * (q.x & 0xffff);
-                    qn[t] = q.y;
-                    best[t] = 0x7fffffff;
-                }
-#pragma unroll 4
-                for (int i = 0; i < ns; ++i) {
-                    const int2 s = ss[i];
-                    const int ay = static_cast<uint32_t>(s.x) >> 16, ax = s.x & 0xffff;
-#pragma unroll
-                    for (int t = 0; t < kQ; ++t) best[t] = min(best[t], ax * cx[t] + (ay * cy[t] + s.y));
-                }
-#pragma unroll
-                for (int t = 0; t < kQ; ++t) {
-                    const int j = base + t * kDistThreads + static_cast<int>(threadIdx.x);
-                    if (j < nq) d2[j] = static_cast<uint32_t>(best[t] + qn[t]);
-                }
-            }
-            }
-            __syncthreads();
-            // K7: max, sum of sqrt, two order statistics
-            uint32_t vmax = 0;
-            double dsum = 0.0;
-            for (int j = threadIdx.x; j < nq; j += kDistThreads) {
-                const uint32_t v = d2[j];
-                vmax = max(vmax, v);
-                dsum += sqrt(static_cast<double>(v) / 4.0);
-            }
-            vmax = block_reduce_max<kDistThreads>(vmax, s_scr);
-            dsum = block_reduce_add<kDistThreads>(dsum, s_dscr);
-            // numpy linear percentile: virtual index (m - 1) * 0.95, neighbours floor and floor + 1
-            const double pos = __dmul_rn(static_cast<double>(nq - 1), 0.95);
-            const uint32_t lo = static_cast<uint32_t>(floor(pos));
-            const uint32_t v_lo = block_select<kDistThreads>(d2, nq, lo, vmax, s_hist, s_bc);
-            uint32_t cnt_le = 0, next_gt = 0xffffffffu;
-            for (int j = threadIdx.x; j < nq; j += kDistThreads) {
-                const uint32_t v = d2[j];
-                cnt_le += v <= v_lo ? 1u : 0u;
-                if (v > v_lo) next_gt = min(next_gt, v);
-            }
-            cnt_le = block_reduce_add<kDistThreads>(cnt_le, s_scr);
-            next_gt = block_reduce_min<kDistThreads>(next_gt, s_scr);
-            const uint32_t v_hi = (lo + 1 >= static_cast<uint32_t>(nq) || cnt_le >= lo + 2) ? v_lo : next_gt;
-            if (prm.sq_out != nullptr) {
-                uint32_t* o = prm.sq_out + (pair * 2 + dir) * static_cast<long long>(cap);
-                for (int j = threadIdx.x; j < nq; j += kDistThreads) o[j] = d2[j];
-            }
-            if (threadIdx.x == 0) {
-                prm.max_sq[pair * 2 + dir] = vmax;
-                prm.p95_sq[pair * 4 + dir * 2 + 0] = v_lo;
-                prm.p95_sq[pair * 4 + dir * 2 + 1] = v_hi;
-                prm.sum_dist[pair * 2 + dir] = dsum;
-            }
-            __syncthreads();
-        }
-    }
-}
-
 // ------------------------------------------------------------------------------ tiled search + select
-// Default path.  Two kernels, neither of which waits at a CTA barrier inside its hot loop:
+// Used when the column-sorted contour does not fit shared memory (max_pts above ~13k, reached when long contours
+// overflow the default bound).  Two kernels, neither of which waits at a CTA barrier inside its hot loop:
 //
 //   distance_search_kernel   one CTA per (item, class, direction).  The source contour is staged in
 //       shared memory in tiles of `tile` vertices as int4 {y, x, y^2+x^2, -} with one bounding box per
@@ -732,9 +541,6 @@ __global__ void __launch_bounds__(kDistThreads) distance_kernel(const DistParams
 //       (fixed order), and the two order statistics of numpy's linear 95th percentile by an 8-bit
 //       radix select whose histogram updates are aggregated with MATCH.ANY (no atomics, no barriers).
 constexpr int kSearchThreads = 256;
-#ifndef OCTM_SEARCH_MINB
-#define OCTM_SEARCH_MINB 6
-#endif
 
 struct SearchParams {
     const uint32_t* verts;   // [n][K][2][max_pts]
@@ -832,7 +638,7 @@ __device__ __forceinline__ void coop_scan_box(const int4* src4, int bb, int ns, 
     }
 }
 
-__global__ void __launch_bounds__(kSearchThreads, OCTM_SEARCH_MINB) distance_search_kernel(const SearchParams prm) {
+__global__ void __launch_bounds__(kSearchThreads, 6) distance_search_kernel(const SearchParams prm) {
     extern __shared__ __align__(16) uint8_t dsm[];
     __shared__ int s_next;
     __shared__ uint32_t s_bins[kCountBins / 2];      // two 16-bit counters per word: count of squared distance 2 * h
@@ -981,7 +787,7 @@ __global__ void __launch_bounds__(kSearchThreads, OCTM_SEARCH_MINB) distance_sea
 }
 
 // ------------------------------------------------------------------------------ column-sorted search
-// Default search.  One CTA per (item, class, direction).  The source contour is counting-sorted by its doubled
+// Used whenever the sorted contour fits shared memory.  One CTA per (item, class, direction).  The source contour is counting-sorted by its doubled
 // lattice column x2 into shared memory (int4 {y, x, y^2 + x^2, -}; col[c] .. col[c + 1] delimit column c).  A
 // warp owns 32 consecutive query vertices spanning the columns [x0, x1]:
 //   1. all lanes scan the sources of the columns [x0, x1] together (one broadcast LDS.128 per source vertex,
@@ -994,9 +800,6 @@ __global__ void __launch_bounds__(kSearchThreads, OCTM_SEARCH_MINB) distance_sea
 // of a real vertex).  No boxes, no per-candidate tests: ~40 vertex evaluations per query on layered B-scans
 // against ~70 for the tiled search, and the worst case (contours far apart) is a brute-force scan.
 constexpr int kColThreads = 256;
-#ifndef OCTM_COL_MINB
-#define OCTM_COL_MINB 5
-#endif
 
 struct ColumnParams {
     const uint32_t* verts;   // [n][K][2][max_pts]
@@ -1017,10 +820,7 @@ struct ColumnParams {
 // group: 32 / kColGroup distinct LDS.128 addresses per instruction, mostly in different banks).  Smaller groups
 // have narrower spans and a smaller flank radius (fewer vertex evaluations per query), at the price of shuffle
 // reductions inside the group.
-#ifndef OCTM_COL_GROUP
-#define OCTM_COL_GROUP 2
-#endif
-constexpr int kColGroup = OCTM_COL_GROUP;
+constexpr int kColGroup = 2;
 
 __device__ __forceinline__ int group_min(int v) {
     if (kColGroup == 32) return __reduce_min_sync(0xffffffffu, v);
@@ -1037,10 +837,7 @@ __device__ __forceinline__ int group_max(int v) {
 
 // Queries per lane: a lane holds kColQ consecutive query vertices, so one broadcast LDS.128 of a source vertex
 // feeds kColQ evaluations and the per-chunk bookkeeping (spans, look-ups, loops) is shared by 32 * kColQ queries.
-#ifndef OCTM_COL_Q
-#define OCTM_COL_Q 2
-#endif
-constexpr int kColQ = OCTM_COL_Q;
+constexpr int kColQ = 2;
 
 // All lanes fold the sorted source vertices [a, a + len) of THEIR group into bm[]; the trip count is the warp's
 // maximum, so a group with a shorter range runs on into vertices it does not need (harmless: every entry is a
@@ -1139,7 +936,7 @@ __device__ __forceinline__ void column_chunks(const int4* src, const uint32_t* c
     }
 }
 
-__global__ void __launch_bounds__(kColThreads, OCTM_COL_MINB) distance_column_kernel(const ColumnParams prm) {
+__global__ void __launch_bounds__(kColThreads, 5) distance_column_kernel(const ColumnParams prm) {
     extern __shared__ __align__(16) uint8_t dsm[];
     __shared__ uint32_t s_bins[kCountBins / 2];
     __shared__ uint32_t s_vmax, s_big;
@@ -1437,9 +1234,6 @@ constexpr int kLdWarps = 4;           // one CTA = one (item, class) pair: the t
 constexpr int kLdPad = 32;            // empty columns on both sides of a table: the scan needs no clamping up to d = 32
 constexpr int kLdRing = 512;          // odd-column query ring per warp (entries)
 constexpr int kLdShort = 64;          // vertex lists up to this length are searched by brute force in the fused kernel
-#ifndef OCTM_LD_MINB
-#define OCTM_LD_MINB 8
-#endif
 
 struct LayeredDistParams {
     const uint32_t* first_pos;   // [n][2][K]
@@ -1722,7 +1516,7 @@ __device__ __forceinline__ void ld_list_stats(const int* best, int n, int lane, 
 // rings or counters.  Thread t takes columns t, t + 128, ..: the even-column vertex and the run to the next column, every
 // query by brute force over the (at most 64) list vertices; the squared distances go to `vals` in shared memory (any
 // order), the sum of square roots and the maximum are kept per thread.  Order statistics by an 8-bit radix select over
-// the stored values (block_select, as in the single-kernel check modes).
+// the stored values (block_select).
 __device__ __forceinline__ void ld_table_vs_list(const short* qlo, const short* qhi, const int2* pts, int n, int W, int nq, int tid,
                                                  uint32_t* vals, uint32_t* s_nvals, uint32_t* s_scr /*>= 8*/, double* s_dscr /*>= 8*/,
                                                  uint32_t* s_hist /*256*/, uint32_t* s_bc /*2*/, uint32_t* max_sq, uint32_t* p95_sq,
@@ -1880,7 +1674,7 @@ __device__ __forceinline__ void ld_emit(const short* lo, const short* hi, int nc
 //         table, table x short list and short x short list are measured here, the rest gets its tables emitted as
 //         vertex lists and stays marked for distance_column_kernel.
 template <int PASS>
-__global__ void __launch_bounds__(kLdWarps * 32, PASS != 2 ? OCTM_LD_MINB : 8) layered_distance_kernel(const LayeredDistParams prm) {
+__global__ void __launch_bounds__(kLdWarps * 32, 8) layered_distance_kernel(const LayeredDistParams prm) {
     extern __shared__ __align__(16) uint8_t dsm[];
     __shared__ uint32_t s_vmax[2], s_bad, s_ok[2], s_minkey[2], s_cnt[2], s_seed[2];
     __shared__ int2 s_list[2][kLdShort];
@@ -2401,9 +2195,8 @@ extern "C" int octm_first_pos_u8(const uint8_t* labels, int64_t n_items, int64_t
 }
 
 static bool layered_ok(const void* y_true, const void* y_pred, const void* bnd_true, const void* bnd_pred, int H, int W, int K) {
-    // layered fast path (needs the label pass's boundary rows): OCTM_TRACE_LAYERED=0 turns it off
-    static const bool env_layered = [] { const char* e = getenv("OCTM_TRACE_LAYERED"); return !(e && e[0] == '0'); }();
-    return env_layered && bnd_true != nullptr && bnd_pred != nullptr && H >= 2 && W % 2 == 0 && K >= 2 && K <= 32 &&
+    // layered fast path (needs the label pass's boundary rows)
+    return bnd_true != nullptr && bnd_pred != nullptr && H >= 2 && W % 2 == 0 && K >= 2 && K <= 32 &&
            reinterpret_cast<uintptr_t>(y_true) % 2 == 0 && reinterpret_cast<uintptr_t>(y_pred) % 2 == 0 &&
            reinterpret_cast<uintptr_t>(bnd_true) % 8 == 0 && reinterpret_cast<uintptr_t>(bnd_pred) % 8 == 0;
 }
@@ -2448,16 +2241,14 @@ static int launch_walk(const octm::TraceParams& p_in, cudaStream_t s, int force_
     }
     if (force_words >= 0) words = words && force_words == 1;
     const long long threads = p.n_items * p.K * 2;
-    static const int env_ctas = [] { const char* e = getenv("OCTM_TRACE_CTAS"); return e ? atoi(e) : 0; }();
     int fit = 0;       // persistent grid: every CTA that can be resident (the walk is latency-bound: occupancy hides it)
     if ((words ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&fit, octm::trace_kernel<true>, 128, 0)
                : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&fit, octm::trace_kernel<false>, 128, 0)) != cudaSuccess || fit < 1) {
         cudaGetLastError();
         fit = 8;
     }
-    const int ctas_per_sm = env_ctas > 0 ? env_ctas : fit;
     long long grid = (threads + 127) / 128;
-    const long long cap = static_cast<long long>(octm::sm_count()) * ctas_per_sm;
+    const long long cap = static_cast<long long>(octm::sm_count()) * fit;
     if (grid > cap) grid = cap;
     if (words) OCTM_TIMED("trace_kernel", s) octm::trace_kernel<true><<<static_cast<unsigned>(grid), 128, 0, s>>>(p);
     else OCTM_TIMED("trace_kernel", s) octm::trace_kernel<false><<<static_cast<unsigned>(grid), 128, 0, s>>>(p);
@@ -2484,11 +2275,6 @@ extern "C" int octm_contour2d_trace_u8(const uint8_t* y_true, const uint8_t* y_p
     return launch_walk(p, s);
 }
 
-static size_t dist_smem(int max_pts) {
-    const size_t capb = (max_pts + octm::kBox - 1) / octm::kBox, caps = (capb + octm::kSuper - 1) / octm::kSuper;
-    return static_cast<size_t>(max_pts) * 20 + 2 * (capb + caps) * 16;
-}
-
 static int run_distance(const uint32_t* verts, const uint32_t* n_pts, int64_t n_items, int num_classes, int max_pts, int H,
                         int W, uint32_t* max_sq, uint32_t* p95_sq, double* sum_dist, uint32_t* d2, int keep_d2,
                         bool only_marked, const uint32_t* todo_count, void* stream) {
@@ -2496,78 +2282,38 @@ static int run_distance(const uint32_t* verts, const uint32_t* n_pts, int64_t n_
     if (H < 1 || W < 1 || H > 8192 || W > 8192) return octm::fail(OCTM_ERR_INVALID, "H, W outside [1, 8192]");
     if (n_items == 0) return OCTM_OK;
     if (!verts || !n_pts || !max_sq || !p95_sq || !sum_dist) return octm::fail(OCTM_ERR_INVALID, "null pointer");
-    // OCTM_DISTANCE_MODE = column (default: column-sorted cooperative search, falls back to tiled when the sorted
-    // contour does not fit shared memory) | tiled (cooperative box search) | lane (per-lane pruned search) |
-    // brute (no pruning); all produce identical integers (tests run each).
-    static const int env_mode = [] {
-        const char* e = getenv("OCTM_DISTANCE_MODE");
-        if (e && !strcmp(e, "brute")) return 2;
-        if (e && !strcmp(e, "lane")) return 1;
-        if (e && !strcmp(e, "tiled")) return 0;
-        return 3;
-    }();
-    int mode = env_mode;
-    if (only_marked && mode != 3) mode = 0;         // the single-kernel check modes search every unit
+    if (d2 == nullptr) return octm::fail(OCTM_ERR_INVALID, "d2 scratch [n][K][2][max_pts] is required");
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     const long long n_pairs = n_items * num_classes;
-    auto run_select = [&]() -> int {
-        octm::SelectParams kp{n_pts, d2, n_pairs * 2, max_pts, max_sq, p95_sq, sum_dist, todo_count};
-        long long kgrid = (n_pairs * 2 + 3) / 4;
-        const long long kcap = static_cast<long long>(octm::sm_count()) * 16;
-        if (kgrid > kcap) kgrid = kcap;
-        OCTM_TIMED("distance_select_kernel", st) octm::distance_select_kernel<<<static_cast<unsigned>(kgrid), 128, 0, st>>>(kp);
-        return octm::check_launch("distance_select_kernel");
-    };
-    if (mode == 3) {
-        if (d2 == nullptr) return octm::fail(OCTM_ERR_INVALID, "d2 scratch [n][K][2][max_pts] is required");
-        const int ncol = 2 * W;
-        const size_t smem = (static_cast<size_t>(max_pts) + 4) * 16 + (static_cast<size_t>(ncol) + 1) * 4;
-        if (smem + 4096 > static_cast<size_t>(octm::max_optin_smem())) {
-            mode = 0;                                   // long contours: tile the source instead
-        } else {
-            if (cudaFuncSetAttribute(octm::distance_column_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                     static_cast<int>(smem)) != cudaSuccess)
-                return octm::fail(OCTM_ERR_LAUNCH, "cudaFuncSetAttribute(distance_column_kernel) failed");
-            octm::ColumnParams cp{verts, n_pts, n_pairs * 2, max_pts, ncol, d2, max_sq, p95_sq, sum_dist, keep_d2 != 0, only_marked, todo_count};
-            long long grid = n_pairs * 2;
-            const long long cap = static_cast<long long>(octm::sm_count()) * 32;
-            if (grid > cap) grid = cap;
-            OCTM_TIMED("distance_column_kernel", st) octm::distance_column_kernel<<<static_cast<unsigned>(grid), octm::kColThreads, smem, st>>>(cp);
-            if (int e = octm::check_launch("distance_column_kernel")) return e;
-            return run_select();
-        }
-    }
-    if (mode == 0) {
-        if (d2 == nullptr) return octm::fail(OCTM_ERR_INVALID, "d2 scratch [n][K][2][max_pts] is required");
-        static const int env_tile = [] { const char* e = getenv("OCTM_DIST_TILE"); return e ? atoi(e) : 0; }();
-        int tile = env_tile >= octm::kBox ? (env_tile / octm::kBox) * octm::kBox : 2048;
-        if (tile > ((max_pts + octm::kBox - 1) / octm::kBox) * octm::kBox) tile = ((max_pts + octm::kBox - 1) / octm::kBox) * octm::kBox;
-        const size_t smem = static_cast<size_t>(tile) * 16 + static_cast<size_t>(tile / octm::kBox) * 16;
-        if (smem > static_cast<size_t>(octm::max_optin_smem()))
-            return octm::fail(OCTM_ERR_UNSUPPORTED, "tile %d needs %zu B of shared memory", tile, smem);
+    long long grid = n_pairs * 2;
+    const long long cap = static_cast<long long>(octm::sm_count()) * 32;
+    if (grid > cap) grid = cap;
+    // column-sorted search when the sorted contour fits shared memory, tiled box search otherwise (long contours)
+    const int ncol = 2 * W;
+    size_t smem = (static_cast<size_t>(max_pts) + 4) * 16 + (static_cast<size_t>(ncol) + 1) * 4;
+    if (smem + 4096 <= static_cast<size_t>(octm::max_optin_smem())) {
+        if (cudaFuncSetAttribute(octm::distance_column_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                 static_cast<int>(smem)) != cudaSuccess)
+            return octm::fail(OCTM_ERR_LAUNCH, "cudaFuncSetAttribute(distance_column_kernel) failed");
+        octm::ColumnParams cp{verts, n_pts, n_pairs * 2, max_pts, ncol, d2, max_sq, p95_sq, sum_dist, keep_d2 != 0, only_marked, todo_count};
+        OCTM_TIMED("distance_column_kernel", st) octm::distance_column_kernel<<<static_cast<unsigned>(grid), octm::kColThreads, smem, st>>>(cp);
+        if (int e = octm::check_launch("distance_column_kernel")) return e;
+    } else {
+        const int tile = std::min(2048, (max_pts + octm::kBox - 1) / octm::kBox * octm::kBox);
+        smem = static_cast<size_t>(tile) * 16 + static_cast<size_t>(tile / octm::kBox) * 16;
         if (cudaFuncSetAttribute(octm::distance_search_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                  static_cast<int>(smem)) != cudaSuccess)
             return octm::fail(OCTM_ERR_LAUNCH, "cudaFuncSetAttribute(distance_search_kernel) failed");
         octm::SearchParams sp{verts, n_pts, n_pairs * 2, max_pts, tile, d2, max_sq, p95_sq, sum_dist, keep_d2 != 0, only_marked, todo_count};
-        long long grid = n_pairs * 2;
-        const long long cap = static_cast<long long>(octm::sm_count()) * 32;
-        if (grid > cap) grid = cap;
         OCTM_TIMED("distance_search_kernel", st) octm::distance_search_kernel<<<static_cast<unsigned>(grid), octm::kSearchThreads, smem, st>>>(sp);
         if (int e = octm::check_launch("distance_search_kernel")) return e;
-        return run_select();
     }
-    const size_t smem = dist_smem(max_pts);
-    if (smem > static_cast<size_t>(octm::max_optin_smem()) - 4096)
-        return octm::fail(OCTM_ERR_UNSUPPORTED, "max_pts %d needs %zu B of shared memory in this mode", max_pts, smem);
-    octm::DistParams p{verts, n_pts, n_pairs, max_pts, max_sq, p95_sq, sum_dist, d2};
-    long long grid = n_pairs;
-    const long long cap = static_cast<long long>(octm::sm_count()) * 16;
-    if (grid > cap) grid = cap;
-    auto kern = mode == 2 ? octm::distance_kernel<false> : octm::distance_kernel<true>;
-    if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, octm::max_optin_smem() - 4096) != cudaSuccess)
-        return octm::fail(OCTM_ERR_LAUNCH, "cudaFuncSetAttribute(distance_kernel) failed");
-    OCTM_TIMED("distance_kernel", st) kern<<<static_cast<unsigned>(grid), octm::kDistThreads, smem, st>>>(p);
-    return octm::check_launch("distance_kernel");
+    octm::SelectParams kp{n_pts, d2, n_pairs * 2, max_pts, max_sq, p95_sq, sum_dist, todo_count};
+    long long kgrid = (n_pairs * 2 + 3) / 4;
+    const long long kcap = static_cast<long long>(octm::sm_count()) * 16;
+    if (kgrid > kcap) kgrid = kcap;
+    OCTM_TIMED("distance_select_kernel", st) octm::distance_select_kernel<<<static_cast<unsigned>(kgrid), 128, 0, st>>>(kp);
+    return octm::check_launch("distance_select_kernel");
 }
 
 extern "C" int octm_contour2d_distance(const uint32_t* verts, const uint32_t* n_pts, int64_t n_items, int num_classes,
@@ -2628,11 +2374,9 @@ extern "C" int octm_contour2d_metrics_u8(const uint8_t* y_true, const uint8_t* y
     uint32_t* d2 = reinterpret_cast<uint32_t*>(static_cast<uint8_t*>(workspace) + verts_b);
     uint32_t* todo = reinterpret_cast<uint32_t*>(static_cast<uint8_t*>(workspace) + 2 * verts_b);
     cudaStream_t s = static_cast<cudaStream_t>(stream);
-    // OCTM_LAYERED_FUSED=0: always go through vertex lists (the round-1 path; tests compare the two)
-    static const bool env_fused = [] { const char* e = getenv("OCTM_LAYERED_FUSED"); return !(e && e[0] == '0'); }();
     const int tab = (2 * W - 1 + 2 * octm::kLdPad + 7) & ~7;
     const size_t smem = static_cast<size_t>(tab) * 8 + octm::kCountBins * 4 + octm::kLdWarps * octm::kLdRing * 4;
-    const bool fused = env_fused && unsorted != nullptr && layered_ok(y_true, y_pred, bnd_true, bnd_pred, H, W, num_classes) &&
+    const bool fused = unsorted != nullptr && layered_ok(y_true, y_pred, bnd_true, bnd_pred, H, W, num_classes) &&
                        H <= 4095 && max_pts <= 0xffff && smem <= static_cast<size_t>(octm::max_optin_smem());
     if (!fused) {
         if (int e = octm_contour2d_trace_u8(y_true, y_pred, n_items, H, W, num_classes, first_pos, bnd_true, bnd_pred, max_pts,
@@ -2663,8 +2407,6 @@ extern "C" int octm_contour2d_metrics_u8(const uint8_t* y_true, const uint8_t* y
             cudaGetLastError();
             fit = 1;
         }
-        static const int env_ctas = [] { const char* e = getenv("OCTM_LD_CTAS"); return e ? atoi(e) : 0; }();
-        if (env_ctas > 0 && env_ctas < fit) fit = env_ctas;             // co-scheduling experiments
         long long grid = n_pairs;
         const long long cap = static_cast<long long>(octm::sm_count()) * fit;
         if (grid > cap) grid = cap;

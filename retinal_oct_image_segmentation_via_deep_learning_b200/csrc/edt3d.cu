@@ -608,8 +608,7 @@ extern "C" int octm_surface3d_u8(const uint8_t* y_true, const uint8_t* y_pred, i
     const uint32_t nbins = edt3_nbins(D0, D1, D2);
     const int sms = octm::sm_count();
     // near-field path (see above): byte planes inside the general path's g region, bit masks and the flag after the histogram
-    static const bool env_near = [] { const char* e = getenv("OCTM_EDT_NEAR"); return !(e && e[0] == '0'); }();
-    const bool near_ok = env_near && D2 % 16 == 0 && reinterpret_cast<uintptr_t>(y_true) % 16 == 0 &&
+    const bool near_ok = D2 % 16 == 0 && reinterpret_cast<uintptr_t>(y_true) % 16 == 0 &&
                          reinterpret_cast<uintptr_t>(y_pred) % 16 == 0;
     uint8_t* ng2 = reinterpret_cast<uint8_t*>(g);
     uint8_t* nh2 = ng2 + up(vox);

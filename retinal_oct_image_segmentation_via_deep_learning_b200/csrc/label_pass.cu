@@ -42,7 +42,6 @@ namespace octm {
 
 constexpr int kStrip = 128;        // columns per consumer warp
 constexpr int kQueueCap = 64;      // queue entries (16 pixel pairs each) per warp
-constexpr int kMaxStages = 8;
 constexpr uint32_t kPadWord = 0x08080808u;   // label 8: PRMT nibble 8 = "replicate sign of LUT byte 0" = 0x00
 constexpr uint32_t kSkipWord = 0xFFFFFFFFu;  // queue marker: this word holds no pixels
 
@@ -394,9 +393,6 @@ __device__ __forceinline__ void stage_rows(LaneState<NP>& ls, uint32_t at, uint3
     }
 }
 
-#ifndef OCTM_LP_MINB
-#define OCTM_LP_MINB 2
-#endif
 // Shared memory of the fast kernel: a fixed CTA block (kOffWarp bytes), then one private block per warp:
 //   [ S full-barriers, padded to 128 B | histogram 4 KB | queue 1 KB | (H > 504: column totals 4 KB) | ring ]
 // The ring is PRIVATE to the warp: S stages x 2 maps x R rows x strip bytes, filled by 2-D TMA tile copies
@@ -404,7 +400,7 @@ __device__ __forceinline__ void stage_rows(LaneState<NP>& ls, uint32_t at, uint3
 // never wait for each other: each folds its strip's results into the zero-initialised outputs with global
 // reductions (RED.ADD / RED.MIN), so a CTA has no barrier after its start-up.
 template <int NP, bool CONF, bool COLS, bool SEEDS, bool SORT, bool WIDE>
-__global__ void __launch_bounds__(WIDE ? 16 * 32 : 8 * 32, WIDE ? 1 : OCTM_LP_MINB)
+__global__ void __launch_bounds__(WIDE ? 16 * 32 : 8 * 32, WIDE ? 1 : 2)
 label_pass_fast(const LabelPassParams prm, const __grid_constant__ CUtensorMap tm_true, const __grid_constant__ CUtensorMap tm_pred) {
     extern __shared__ __align__(128) uint8_t smem[];
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -683,10 +679,7 @@ label_pass_fast(const LabelPassParams prm, const __grid_constant__ CUtensorMap t
 // the joint code (t, p) comes in long RUNS (a column stays inside a layer for many rows): only a run's length
 // is accumulated per pixel; when the code changes the run goes into the warp's shared-memory confusion
 // histogram (one atomic per run, not per pixel) and into the thread's own per-class column counters.
-#ifndef OCTM_GEN_MINB
-#define OCTM_GEN_MINB 4
-#endif
-__global__ void __launch_bounds__(256, OCTM_GEN_MINB) label_pass_generic(const LabelPassParams prm, const int strips) {
+__global__ void __launch_bounds__(256, 4) label_pass_generic(const LabelPassParams prm, const int strips) {
     __shared__ uint32_t s_counts[8][256];                 // per-warp confusion histogram, code = t * 16 + p
     __shared__ unsigned short s_cls[2][16][256];          // per-thread class counts of the current column
     __shared__ unsigned long long s_sq[16], s_abs[16], s_thick[16];
@@ -848,27 +841,12 @@ __global__ void __launch_bounds__(256, OCTM_GEN_MINB) label_pass_generic(const L
 //     warp-instructions per pixel pair, the same as the byte-wise kernel);
 //   * column arithmetic, boundary rows (16-byte stores) and seeds follow per job; warps never meet: their results
 //     join in zero-initialised outputs through global atomics (a few hundred per 63 k pixel pairs).
-#ifndef OCTM_WIDE_WARPS
-#define OCTM_WIDE_WARPS 2
-#endif
-#ifndef OCTM_WIDE_QUEUE
-#define OCTM_WIDE_QUEUE 48
-#endif
-constexpr int kWideWarps = OCTM_WIDE_WARPS;
-constexpr int kWideQueue = OCTM_WIDE_QUEUE;       // queue entries per lane; a batch of 8 rows pushes at most 32
+constexpr int kWideWarps = 2;
+constexpr int kWideQueue = 48;      // queue entries per lane; a batch of 8 rows pushes at most 32
 // per warp: counts u32 [256] | cls u16 [2][K][128] | queue u32 [kWideQueue][32] | fst u32 [2 K][32] | colstate u32 [4][32]
 // (sized by K: 17 KB per warp at K = 10 -> 12 warps per SM)
 static inline int wide_warp_bytes(int K) { return 1024 + 512 * K + kWideQueue * 128 + 256 * K + 512; }
-#ifndef OCTM_WIDE_MINB
-#define OCTM_WIDE_MINB 7
-#endif
-#ifndef OCTM_WIDE_ROWS
-#define OCTM_WIDE_ROWS 8
-#endif
-#ifndef OCTM_WIDE_PIPE
-#define OCTM_WIDE_PIPE 2
-#endif
-__global__ void __launch_bounds__(kWideWarps * 32, OCTM_WIDE_MINB) label_pass_wide(const LabelPassParams prm, const int strips) {
+__global__ void __launch_bounds__(kWideWarps * 32, 7) label_pass_wide(const LabelPassParams prm, const int strips) {
     extern __shared__ __align__(16) unsigned char s_wide[];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int H = prm.H, W = prm.W, K = prm.K, nthr = K - 1;
@@ -931,7 +909,7 @@ __global__ void __launch_bounds__(kWideWarps * 32, OCTM_WIDE_MINB) label_pass_wi
             const int xc = valid ? x : W - 4;
             const uint8_t* ct = prm.yt + item * H * static_cast<long long>(W) + xc;
             const uint8_t* cp = prm.yp + item * H * static_cast<long long>(W) + xc;
-            constexpr int kRows = OCTM_WIDE_ROWS;
+            constexpr int kRows = 8;
             static_assert(4 * kRows <= kWideQueue, "a batch must fit the queue");
             uint32_t ta[kRows], pa[kRows];
             auto fetch = [&](uint32_t (&tv)[kRows], uint32_t (&pv)[kRows], int y0) {
@@ -967,7 +945,6 @@ __global__ void __launch_bounds__(kWideWarps * 32, OCTM_WIDE_MINB) label_pass_wi
                     }
                 }
             };
-#if OCTM_WIDE_PIPE == 2
             // three register batches: two are in flight while one is worked on
             uint32_t tb[kRows], pb[kRows], tc[kRows], pc[kRows];
             fetch(tb, pb, kRows);
@@ -982,24 +959,6 @@ __global__ void __launch_bounds__(kWideWarps * 32, OCTM_WIDE_MINB) label_pass_wi
                 work(tc, pc, y0 + 2 * kRows);
                 if (__any_sync(0xffffffffu, qn > kWideQueue - 4 * kRows)) drain();
             }
-#elif OCTM_WIDE_PIPE
-            // two register batches: the loads of the next one are in flight while this one is worked on
-            uint32_t tb[kRows], pb[kRows];
-            for (int y0 = 0; y0 < H; y0 += 2 * kRows) {
-                fetch(tb, pb, y0 + kRows);
-                work(ta, pa, y0);
-                if (__any_sync(0xffffffffu, qn > kWideQueue - 4 * kRows)) drain();
-                fetch(ta, pa, y0 + 2 * kRows);
-                work(tb, pb, y0 + kRows);
-                if (__any_sync(0xffffffffu, qn > kWideQueue - 4 * kRows)) drain();
-            }
-#else
-            for (int y0 = 0; y0 < H; y0 += kRows) {
-                if (y0) fetch(ta, pa, y0);
-                work(ta, pa, y0);
-                if (__any_sync(0xffffffffu, qn > kWideQueue - 4 * kRows)) drain();
-            }
-#endif
             if (valid) {                                               // the runs still open at the bottom
                 push(open01 & 0xffffu, st0, H, 0u);
                 push(open01 >> 16, st1, H, 1u);
@@ -1208,21 +1167,13 @@ static int launch_fast(const LabelPassParams& p0, cudaStream_t stream) {
     const int NW = (p.W + kStrip - 1) / kStrip;
     // each warp stages its own 128-column strip: R rows per stage (multiple of 4), S stages.  16 rows x 2 stages =
     // 8 KB of ring per warp; shared memory (occupancy) matters more than ring depth here.
-    // OCTM_LP_ROWS / OCTM_LP_STAGES override for tuning runs.
-    static const int env_rows = [] { const char* e = getenv("OCTM_LP_ROWS"); return e ? atoi(e) : 0; }();
-    static const int env_stages = [] { const char* e = getenv("OCTM_LP_STAGES"); return e ? atoi(e) : 0; }();
-    int R = 16;
-    if (env_rows > 0) R = env_rows & ~3;
-    if (R < 4) R = 4;
-    if (R > 256) R = 256;                                  // TMA box limit
+    const int R = 16, S = 2;
     p.R = R;
+    p.S = S;
     const int srow = p.W < kStrip ? p.W : kStrip;
     const int state = kWarpBars + (p.H > kShortRows ? kWarpBytesTall : kWarpBytesShort);
     const int stage = 2 * R * srow;
     const int budget = max_optin_smem();
-    int S = env_stages >= 2 && env_stages <= kMaxStages ? env_stages : 2;
-    while (S > 2 && kOffWarp + NW * (state + S * stage) > budget) --S;
-    p.S = S;
     const int smem = kOffWarp + NW * (state + S * stage);
     if (smem > budget) return fail(OCTM_ERR_UNSUPPORTED, "label pass: %d B of shared memory needed", smem);
     // the warps of a CTA merge their strips in the outputs by global reductions: start from zero / "no seed"
@@ -1250,9 +1201,6 @@ static int launch_fast(const LabelPassParams& p0, cudaStream_t stream) {
         cudaGetLastError();
         per_sm = 1;
     }
-    // OCTM_LP_CTAS caps the resident CTAs per SM (co-scheduling experiments: leave room for another kernel)
-    static const int env_ctas = [] { const char* e = getenv("OCTM_LP_CTAS"); return e ? atoi(e) : 0; }();
-    if (env_ctas > 0 && env_ctas < per_sm) per_sm = env_ctas;
     long long grid = static_cast<long long>(sm_count()) * per_sm;
     if (grid > p.n_items) grid = p.n_items;
     OCTM_TIMED("label_pass_fast", stream) kern<<<static_cast<unsigned>(grid), threads, smem, stream>>>(p, tm_true, tm_pred);
@@ -1281,8 +1229,7 @@ static int dispatch_np(const LabelPassParams& p, cudaStream_t stream) {
 
 static int launch_generic(const LabelPassParams& p, cudaStream_t stream) {
     // K <= 16 with 4-byte rows: the warp-per-strip kernel; anything else the byte-wise one
-    static const bool env_wide = [] { const char* e = getenv("OCTM_LP_WIDE"); return !(e && e[0] == '0'); }();
-    const bool wide = env_wide && p.W % 4 == 0 && reinterpret_cast<uintptr_t>(p.yt) % 4 == 0 && reinterpret_cast<uintptr_t>(p.yp) % 4 == 0 &&
+    const bool wide = p.W % 4 == 0 && reinterpret_cast<uintptr_t>(p.yt) % 4 == 0 && reinterpret_cast<uintptr_t>(p.yp) % 4 == 0 &&
                       (p.bnd_t == nullptr || (reinterpret_cast<uintptr_t>(p.bnd_t) % 16 == 0 && reinterpret_cast<uintptr_t>(p.bnd_p) % 16 == 0)) &&
                       p.H <= 16383 && static_cast<long long>(p.H) * p.W < (1ll << 32) &&
                       // a handful of items (one volume) is latency-bound either way: the byte-wise kernel's 32-column warps
