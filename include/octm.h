@@ -222,6 +222,32 @@ OCTM_API int octm_contour2d_distance(const uint32_t* verts, const uint32_t* n_pt
                             void* stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * All-contour distances (build-defined, no reference counterpart): hausdorff / hd95 / assd over EVERY contour of
+ * each class mask instead of contour [0] only -- the whole boundary, as MONAI, medpy and surface-distance measure it.
+ * Per (item i, class c, map m) the vertex set is
+ *   V(i, c, m) = doubled-lattice midpoints of every crack between two 4-adjacent pixels of the image exactly one of
+ *                which is class c  (= unique(concatenate(find_contours(L == c, 0.5))) * 2)
+ * each vertex ONCE: no closing repeats.  Lattice row 2y holds the cracks (y, x) | (y, x + 1) at x2 = 2x + 1, row
+ * 2y + 1 the cracks (y, x) | (y + 1, x) at x2 = 2x.  Outputs as for octm_contour2d_u8 with these sets in place of
+ * contour [0]: direction 0 queries every pred vertex against the true set, direction 1 the other way.
+ *   verts   uint32 [n][K][2][max_pts]  packed (y2 << 16 | x2), in raster order of the doubled lattice (y2, then x2):
+ *                                      deterministic, so sum_dist is bit-reproducible
+ *   n_pts   uint32 [n][K][2]           |V| EXACTLY, also when it exceeds max_pts (then only the first max_pts
+ *                                      vertices are stored and the OCTM_CF_*_OVERFLOW bit is set: redo the item with
+ *                                      max_pts >= n_pts).  0 = class absent from the map or filling it (metrics NaN).
+ *   flags   uint32 [n][K]              OCTM_CF_*_OVERFLOW only; the *_CLOSED bits are never set.
+ * |V| <= (H - 1) * W + H * (W - 1) (every crack).  One read of each label map emits all K classes. */
+OCTM_API int octm_contour2d_all_vertices_u8(const uint8_t* y_true, const uint8_t* y_pred, int64_t n_items, int H, int W,
+                                   int num_classes, int max_pts, uint32_t* verts, uint32_t* n_pts,
+                                   uint32_t* flags, void* stream);
+/* One call: octm_contour2d_all_vertices_u8 + octm_contour2d_distance; max_sq / p95_sq / sum_dist as for
+ * octm_contour2d_u8.  workspace >= octm_contour2d_workspace_bytes(n_items, H, W, num_classes, max_pts). */
+OCTM_API int octm_contour2d_all_u8(const uint8_t* y_true, const uint8_t* y_pred, int64_t n_items, int H, int W,
+                          int num_classes, int max_pts, uint32_t* n_pts, uint32_t* flags, uint32_t* max_sq,
+                          uint32_t* p95_sq, double* sum_dist, void* workspace, size_t workspace_bytes,
+                          void* stream);
+
+/* ---------------------------------------------------------------------------------------------
  * Boundary rows -> label maps (SURVEY.md 8f-4: the layer datasets catalogued in the reference's
  * Datasets.md:3-26 annotate boundary curves, while Metrics/*.py score masks).  The inverse of the label
  * pass's boundary rows on layered maps:

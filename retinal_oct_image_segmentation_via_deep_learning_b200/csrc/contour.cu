@@ -2171,7 +2171,7 @@ __global__ void __launch_bounds__(kLdWarps * 32, 8) layered_distance_kernel(cons
 }  // namespace octm
 
 // ----------------------------------------------------------------------------------- C ABI
-static int check_shape(int64_t n, int H, int W, int K, int max_pts) {
+int check_shape(int64_t n, int H, int W, int K, int max_pts) {     // also used by contour_all.cu
     if (n < 0) return octm::fail(OCTM_ERR_INVALID, "n_items < 0");
     if (K < 2 || K > OCTM_MAX_CLASSES) return octm::fail(OCTM_ERR_INVALID, "num_classes %d outside [2, 16]", K);
     if (H < 1 || W < 1) return octm::fail(OCTM_ERR_INVALID, "H, W must be >= 1");

@@ -27,6 +27,20 @@ def default_max_pts(width):
     synthetic layers), so the bound grows with the width -- 2048 up to W = 512, 4 W beyond (a 1024-wide HC-MS B-scan would
     otherwise overflow on every contour and be redone)."""
     return max(DEFAULT_MAX_PTS, min(MAX_MAX_PTS, 4 * int(width)))
+
+
+def default_max_pts_all(width):
+    """First-attempt vertex bound of ``mode="all"``: a layer band has two boundaries (its upper and its lower one, each
+    about 2.7 W vertices on the synthetic layers), hence 8 W."""
+    return max(DEFAULT_MAX_PTS, 8 * int(width))
+
+
+def crack_bound(height, width):
+    """Largest possible all-contour vertex count of one class: every crack between 4-adjacent pixels."""
+    return (int(height) - 1) * int(width) + int(height) * (int(width) - 1)
+
+
+CONTOUR_MODES = ("first", "all")
 CONTOUR_CHUNK_BYTES = 4 << 30   # vertex + squared-distance scratch per chunk of items (grow-only, reused)
 
 
@@ -227,6 +241,7 @@ class ContourOut:
     verts: torch.Tensor | None = None     # [N, K, 2, max_pts] when requested
     sq: torch.Tensor | None = None        # [N, K, 2, max_pts] when requested
     max_pts: int = 0
+    mode: str = "first"                   # "first": contour [0] only; "all": every contour of each class
 
 
 _SCRATCH = {}      # (device, stream) -> grow-only int32 scratch for contour vertices (pure workspace, never returned)
@@ -260,7 +275,10 @@ def _vertex_scratch(dev, numel):
     return buf[:numel]
 
 
-def _contour_chunk(yt, yp, k, first_pos, max_pts, want_verts, want_sq, timers=None, bnd=None, unsorted=None):
+def _contour_chunk(yt, yp, k, first_pos, max_pts, want_verts, want_sq, timers=None, bnd=None, unsorted=None,
+                   mode="first"):
+    if mode == "all":
+        return _contour_chunk_all(yt, yp, k, max_pts, want_verts, want_sq, timers)
     n, h, w = yt.shape
     max_pts = (int(max_pts) + 3) & ~3          # vertices are stored in 16-byte groups
     dev = yt.device
@@ -293,9 +311,47 @@ def _contour_chunk(yt, yp, k, first_pos, max_pts, want_verts, want_sq, timers=No
     return ContourOut(n_pts, flags, max_sq, p95, sums, verts if want_verts else None, sq if want_sq else None, max_pts)
 
 
+def _contour_chunk_all(yt, yp, k, max_pts, want_verts, want_sq, timers=None):
+    """``mode="all"``: every boundary vertex of every class (octm_contour2d_all_*), then the same distance stage."""
+    n, h, w = yt.shape
+    dev = yt.device
+    i32 = dict(dtype=torch.int32, device=dev)
+    numel = (n * k * 2 * max_pts + 63) & ~63          # 256-byte multiples (the workspace layout of the C ABI)
+    nv = n * k * 2 * max_pts
+    n_pts = torch.empty((n, k, 2), **i32)
+    flags = torch.empty((n, k), **i32)
+    max_sq = torch.empty((n, k, 2), **i32)
+    p95 = torch.empty((n, k, 2, 2), **i32)
+    sums = torch.empty((n, k, 2), dtype=torch.float64, device=dev)
+    if not want_verts and not want_sq:
+        ws_bytes = int(_lib.load().octm_contour2d_workspace_bytes(n, h, w, k, max_pts))
+        scratch = _vertex_scratch(dev, (ws_bytes + 3) // 4)
+        with _Timed(timers, "contour"):
+            _lib.call("octm_contour2d_all_u8", _ptr(yt), _ptr(yp), n, h, w, k, max_pts, _ptr(n_pts), _ptr(flags),
+                      _ptr(max_sq), _ptr(p95), _ptr(sums), _ptr(scratch), scratch.numel() * 4, _stream())
+        return ContourOut(n_pts, flags, max_sq, p95, sums, None, None, max_pts, "all")
+    scratch = None if (want_verts and want_sq) else _vertex_scratch(dev, 2 * numel + 64)
+    verts = torch.empty((n, k, 2, max_pts), **i32) if want_verts else scratch[:nv].view(n, k, 2, max_pts)
+    sq = torch.empty((n, k, 2, max_pts), **i32) if want_sq else scratch[numel:numel + nv].view(n, k, 2, max_pts)
+    with _Timed(timers, "contour_trace"):
+        _lib.call("octm_contour2d_all_vertices_u8", _ptr(yt), _ptr(yp), n, h, w, k, max_pts, _ptr(verts), _ptr(n_pts),
+                  _ptr(flags), _stream())
+    with _Timed(timers, "contour_distance"):
+        _lib.call("octm_contour2d_distance", _ptr(verts), _ptr(n_pts), n, k, max_pts, h, w, _ptr(max_sq), _ptr(p95),
+                  _ptr(sums), _ptr(sq), 1 if want_sq else 0, _stream())
+    return ContourOut(n_pts, flags, max_sq, p95, sums, verts if want_verts else None, sq if want_sq else None, max_pts,
+                      "all")
+
+
 def contour_pass(y_true, y_pred, num_classes, first_pos=None, *, max_pts=None, return_vertices=False,
-                 return_sq=False, timers=None, check_overflow=True, boundaries=None, unsorted=None):
+                 return_sq=False, timers=None, check_overflow=True, boundaries=None, unsorted=None, mode="first"):
     """Contour ``[0]`` of every class mask of both maps, then hausdorff / hd95 / assd integers.
+
+    ``mode="all"`` measures EVERY contour of each class instead (build-defined, no reference counterpart): the vertex
+    set of a class is the midpoint of every crack between two 4-adjacent pixels exactly one of which is in the class,
+    each once, in raster order of the doubled lattice (``octm_contour2d_all_vertices_u8``); ``n_pts`` is its exact
+    size.  ``first_pos``, ``boundaries`` and ``unsorted`` are not used then, and the default bound is
+    ``default_max_pts_all(W)``.
 
     ``boundaries``: optional ``(bnd_true, bnd_pred)`` int32 ``[N, K-1, W]`` of the label pass; with them the
     contours of layered maps are verified and emitted in parallel instead of walked (same vertices).
@@ -304,15 +360,21 @@ def contour_pass(y_true, y_pred, num_classes, first_pos=None, *, max_pts=None, r
 
     Items are processed in chunks so the vertex workspace stays under ~1 GiB; items whose contour is
     longer than ``max_pts`` are re-run on their own with a larger bound."""
+    if mode not in CONTOUR_MODES:
+        raise ValueError(f"mode must be one of {CONTOUR_MODES}, got {mode!r}")
     yt, yp = _check_pair(y_true, y_pred)
     n, h, w = yt.shape
     k = int(num_classes)
-    max_pts = (int(default_max_pts(w) if max_pts is None else max_pts) + 3) & ~3
+    if max_pts is None:
+        max_pts = default_max_pts_all(w) if mode == "all" else default_max_pts(w)
+    max_pts = (int(max_pts) + 3) & ~3
     if h < 2 or w < 2:
         raise ValueError("Input array must be at least 2x2.")     # skimage's message for find_contours
     dev = yt.device
+    if mode == "all":
+        first_pos = boundaries = unsorted = None
     with torch.cuda.device(dev):
-        if first_pos is None:
+        if first_pos is None and mode == "first":
             first_pos = torch.empty((n, 2, k), dtype=torch.int32, device=dev)
             tmp = torch.empty((n, k), dtype=torch.int32, device=dev)
             for m, src in enumerate((yt, yp)):
@@ -323,21 +385,22 @@ def contour_pass(y_true, y_pred, num_classes, first_pos=None, *, max_pts=None, r
             i32 = dict(dtype=torch.int32, device=dev)
             return ContourOut(torch.empty((0, k, 2), **i32), torch.empty((0, k), **i32), torch.empty((0, k, 2), **i32),
                               torch.empty((0, k, 2, 2), **i32), torch.empty((0, k, 2), dtype=torch.float64, device=dev),
-                              None, None, max_pts)
+                              None, None, max_pts, mode)
         per_item = k * 2 * max_pts * 4 * 2          # vertices + squared-distance scratch
         chunk = n if keep else max(1, min(n, CONTOUR_CHUNK_BYTES // per_item))
         parts = []
         for s in range(0, n, chunk):
             e = min(n, s + chunk)
-            parts.append(_contour_chunk(yt[s:e], yp[s:e], k, first_pos[s:e], max_pts, return_vertices, return_sq, timers,
+            parts.append(_contour_chunk(yt[s:e], yp[s:e], k, None if first_pos is None else first_pos[s:e], max_pts,
+                                        return_vertices, return_sq, timers,
                                         None if boundaries is None else (boundaries[0][s:e], boundaries[1][s:e]),
-                                        None if unsorted is None else unsorted[s:e]))
+                                        None if unsorted is None else unsorted[s:e], mode))
         if len(parts) == 1:
             out = parts[0]
         else:
             cat = lambda f: torch.cat([getattr(p, f) for p in parts])      # noqa: E731
             out = ContourOut(cat("n_pts"), cat("flags"), cat("max_sq"), cat("p95_sq"), cat("sum_dist"), None, None,
-                             max_pts)
+                             max_pts, mode)
         if check_overflow:
             _retry_overflow(out, yt, yp, k, first_pos, keep)
     return out
@@ -347,11 +410,16 @@ def _retry_overflow(out, yt, yp, k, first_pos, keep=False):
     """Re-run, with a larger vertex bound, the (rare) items whose contour overflowed ``max_pts``.  The bound
     escalates geometrically (x8 per round, up to MAX_MAX_PTS) and every round is chunked so that its vertex and
     distance scratch stays below CONTOUR_CHUNK_BYTES, like the first pass.  Returns True when something was
-    redone.  Costs one device->host sync per round."""
+    redone.  Costs one device->host sync per round.
+
+    ``mode="all"`` counts every vertex even past the bound, so a single round redoes the overflowed items with the
+    largest count (rounded up to a multiple of 4) as the bound; no count exceeds ``crack_bound(H, W)``."""
     over_bits = _lib.CF_TRUE_OVERFLOW | _lib.CF_PRED_OVERFLOW
     over = ((out.flags & over_bits) != 0).any(dim=1)
     if not bool(over.any()):
         return False
+    if out.mode == "all":
+        return _retry_overflow_all(out, yt, yp, k, over, keep)
     if keep:
         raise _lib.OctmError(f"a contour has more than max_pts={out.max_pts} vertices; raise max_pts")
     idx = torch.nonzero(over).flatten()
@@ -370,6 +438,21 @@ def _retry_overflow(out, yt, yp, k, first_pos, keep=False):
                 getattr(out, f)[sub] = getattr(redo, f)
             still.append(sub[((redo.flags & over_bits) != 0).any(dim=1)])
         idx = torch.cat(still)
+    return True
+
+
+def _retry_overflow_all(out, yt, yp, k, over, keep):
+    idx = torch.nonzero(over).flatten()
+    need = (int(out.n_pts[idx].max()) + 3) & ~3
+    if keep:
+        raise _lib.OctmError(f"a class has {need} boundary vertices (rounded up to a multiple of 4), more than "
+                             f"max_pts={out.max_pts}; pass max_pts >= {need}")
+    chunk = max(1, CONTOUR_CHUNK_BYTES // (k * 2 * need * 4 * 2))
+    for s0 in range(0, idx.numel(), chunk):
+        sub = idx[s0:s0 + chunk]
+        redo = _contour_chunk_all(yt[sub].contiguous(), yp[sub].contiguous(), k, need, False, False)
+        for f in ("n_pts", "flags", "max_sq", "p95_sq", "sum_dist"):
+            getattr(out, f)[sub] = getattr(redo, f)
     return True
 
 
@@ -405,6 +488,7 @@ class SuiteResult:
     _final: bool = field(default=False, repr=False)
     _host: dict | None = field(default=None, repr=False)
     _totals_host: np.ndarray | None = field(default=None, repr=False)
+    contour_mode: str | None = "first"     # "first" / "all" (contour_pass modes), None without contour metrics
 
     def settle_overflow(self, vec):
         """Redo (with a larger vertex bound) this batch's items whose contour overflowed ``max_pts`` and
@@ -499,9 +583,21 @@ class SuiteResult:
         return m
 
 
+def _contour_mode(contours):
+    if not isinstance(contours, str):
+        return "first" if contours else None
+    if contours not in CONTOUR_MODES:
+        raise ValueError(f"contours must be True, False, 'first' or 'all', got {contours!r}")
+    return contours
+
+
 def evaluate(y_true, y_pred, num_classes, *, contours=True, boundaries=False, max_pts=None, timers=None,
              validate=True):
     """The full suite on a batch of label maps: fused label pass, contour kernels, float64 epilogue.
+
+    ``contours``: ``True`` / ``"first"`` = hausdorff / hd95 / assd on contour ``[0]`` of each class mask, as the
+    reference computes them; ``"all"`` = on every contour of each class (the whole boundary, see ``contour_pass``);
+    ``False`` = no contour metrics.
 
     Everything is launched asynchronously on the current stream; nothing is read back until
     ``totals_host()`` / ``metrics()`` / ``integers()`` is called on the result.
@@ -509,7 +605,14 @@ def evaluate(y_true, y_pred, num_classes, *, contours=True, boundaries=False, ma
     ``validate``: a label >= num_classes (an ignore label such as 255, a wrong class count) raises ValueError when
     the results are read.  The check costs nothing extra: the label pass never aliases such a pixel into another
     class but drops it, so the item's confusion counts do not add up to H * W, which the totals kernel counts."""
+    mode = _contour_mode(contours)
     yt, yp = _check_pair(y_true, y_pred)
+    if mode == "all":
+        lp = label_pass(yt, yp, num_classes, counts=True, columns=True, boundaries=boundaries, timers=timers)
+        ct = contour_pass(yt, yp, num_classes, max_pts=max_pts, timers=timers, check_overflow=False, mode="all")
+        cls, bnd, tot = derive_on_device(lp, ct, yt.shape[0], timers)
+        return SuiteResult(yt.shape[0], lp, ct, cls, bnd, tot, (yt, yp), validate=bool(validate), contour_mode="all")
+    contours = mode == "first"
     # the contour stage uses the label pass's boundary rows to skip the walk on layered maps
     lp = label_pass(yt, yp, num_classes, counts=True, columns=True, seeds=contours, boundaries=boundaries or contours,
                     timers=timers, certify=contours)
@@ -520,7 +623,8 @@ def evaluate(y_true, y_pred, num_classes, *, contours=True, boundaries=False, ma
         if not boundaries:
             lp.bnd_true = lp.bnd_pred = None
     cls, bnd, tot = derive_on_device(lp, ct, yt.shape[0], timers)
-    return SuiteResult(yt.shape[0], lp, ct, cls, bnd, tot, (yt, yp) if contours else None, validate=bool(validate))
+    return SuiteResult(yt.shape[0], lp, ct, cls, bnd, tot, (yt, yp) if contours else None, validate=bool(validate),
+                       contour_mode=mode)
 
 
 def _cat_results(parts):
@@ -537,10 +641,10 @@ def _cat_results(parts):
     if parts[0].contours is not None:
         cts = [p.contours for p in parts]
         ct = ContourOut(*[cat(cts, f) for f in ("n_pts", "flags", "max_sq", "p95_sq", "sum_dist")], None, None,
-                        cts[0].max_pts)
+                        cts[0].max_pts, cts[0].mode)
     n = sum(p.num_items for p in parts)
     cls, bnd, tot = derive_on_device(lp, ct, n)            # per-item values again + totals of the whole batch
-    res = SuiteResult(n, lp, ct, cls, bnd, tot, validate=parts[0].validate)
+    res = SuiteResult(n, lp, ct, cls, bnd, tot, validate=parts[0].validate, contour_mode=parts[0].contour_mode)
     res._final = True
     return res
 
