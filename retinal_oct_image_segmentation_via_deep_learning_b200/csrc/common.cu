@@ -1,4 +1,4 @@
-// Process-wide state of the octm library: error string, launch counter, device properties.
+// Process-wide state of the octm library: error string, launch counter, device properties, host-mapped report cells.
 #include "common.cuh"
 
 #include <cstring>
@@ -62,6 +62,27 @@ int max_optin_smem() {
         cached_dev = dev;
     }
     return cached;
+}
+
+HostReport* host_report(int slot) {
+    static HostReport cells[64][2];
+    static std::mutex mu;
+    int dev = -1;
+    if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) { cudaGetLastError(); return nullptr; }
+    std::lock_guard<std::mutex> lk(mu);
+    HostReport& r = cells[dev][slot];
+    if (r.host == nullptr) {
+        void* h = nullptr;
+        void* d = nullptr;
+        if (cudaHostAlloc(&h, 2 * sizeof(uint32_t), cudaHostAllocMapped) != cudaSuccess || cudaHostGetDevicePointer(&d, h, 0) != cudaSuccess) {
+            cudaGetLastError();
+            return nullptr;
+        }
+        r.host = static_cast<uint32_t*>(h);
+        r.dev = static_cast<uint32_t*>(d);
+        r.host[0] = r.host[1] = 0;
+    }
+    return &r;
 }
 
 }  // namespace octm

@@ -65,6 +65,41 @@ int sm_count();            // SMs of the current device (cached per device)
 bool stream_mostly_rejected();
 int max_optin_smem();      // cudaDevAttrMaxSharedMemoryPerBlockOptin of the current device
 
+// Persistent grid: min(want, the CTAs of `kern` resident at once on the current device); `fallback` CTAs per SM when the
+// occupancy query fails.
+template <class Kernel>
+long long resident_grid(long long want, Kernel kern, int threads, size_t smem, int fallback) {
+    int fit = 0;
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&fit, kern, threads, smem) != cudaSuccess || fit < 1) {
+        cudaGetLastError();
+        fit = fallback;
+    }
+    const long long cap = static_cast<long long>(sm_count()) * fit;
+    return want < cap ? want : cap;
+}
+
+// A zeroed, host-mapped uint32[2] per device and slot, allocated on first use: a one-thread kernel leaves a report in it
+// and a later call reads it on the host without synchronisation.  nullptr when no cell can be had.
+enum { kReportSeeds = 0, kReportWalks = 1 };      // label_pass.cu: rejected maps / maps; contour.cu: walks / contours
+struct HostReport {
+    uint32_t* host = nullptr;      // mapped, pinned
+    uint32_t* dev = nullptr;       // the device's view of it
+};
+HostReport* host_report(int slot);
+
+// contour.cu: the argument checks every contour entry point shares
+int check_shape(int64_t n, int H, int W, int K, int max_pts);
+
+// contour.cu: the contour workspace holds the vertices [n][K][2][max_pts] and the squared distances (same shape), each
+// rounded up to 256 bytes, then a tail of words at tail_offset.  Without a workspace only tail_offset is set.
+struct ContourWorkspace {
+    size_t tail_offset;
+    uint32_t* verts = nullptr;
+    uint32_t* d2 = nullptr;
+    uint32_t* tail = nullptr;
+};
+ContourWorkspace contour_workspace(int64_t n_items, int K, int max_pts, void* workspace = nullptr);
+
 #ifdef __CUDACC__
 // ---------------------------------------------------------------- device-side PTX helpers
 __device__ __forceinline__ uint32_t smem_u32(const void* p) {

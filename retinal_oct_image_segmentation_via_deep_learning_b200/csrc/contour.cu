@@ -26,8 +26,6 @@
 #include <numeric>
 #include <type_traits>
 
-#include <mutex>
-
 #include "common.cuh"
 #include "trace_core.h"
 
@@ -2171,15 +2169,38 @@ __global__ void __launch_bounds__(kLdWarps * 32, 8) layered_distance_kernel(cons
 }  // namespace octm
 
 // ----------------------------------------------------------------------------------- C ABI
-int check_shape(int64_t n, int H, int W, int K, int max_pts) {     // also used by contour_all.cu
-    if (n < 0) return octm::fail(OCTM_ERR_INVALID, "n_items < 0");
-    if (K < 2 || K > OCTM_MAX_CLASSES) return octm::fail(OCTM_ERR_INVALID, "num_classes %d outside [2, 16]", K);
-    if (H < 1 || W < 1) return octm::fail(OCTM_ERR_INVALID, "H, W must be >= 1");
+namespace octm {
+int check_shape(int64_t n, int H, int W, int K, int max_pts) {
+    if (n < 0) return fail(OCTM_ERR_INVALID, "n_items < 0");
+    if (K < 2 || K > OCTM_MAX_CLASSES) return fail(OCTM_ERR_INVALID, "num_classes %d outside [2, 16]", K);
+    if (H < 1 || W < 1) return fail(OCTM_ERR_INVALID, "H, W must be >= 1");
     if (H > 8192 || W > 8192)
-        return octm::fail(OCTM_ERR_UNSUPPORTED, "image side > 8192: squared lattice distances leave the int32 kernel range");
-    if (static_cast<long long>(H) * W >= (1ll << 32) - 1) return octm::fail(OCTM_ERR_UNSUPPORTED, "H*W >= 2^32");
-    if (max_pts < 8 || max_pts % 4 != 0) return octm::fail(OCTM_ERR_INVALID, "max_pts must be >= 8 and a multiple of 4");
+        return fail(OCTM_ERR_UNSUPPORTED, "image side > 8192: squared lattice distances leave the int32 kernel range");
+    if (static_cast<long long>(H) * W >= (1ll << 32) - 1) return fail(OCTM_ERR_UNSUPPORTED, "H*W >= 2^32");
+    if (max_pts < 8 || max_pts % 4 != 0) return fail(OCTM_ERR_INVALID, "max_pts must be >= 8 and a multiple of 4");
     return OCTM_OK;
+}
+
+ContourWorkspace contour_workspace(int64_t n_items, int K, int max_pts, void* workspace) {
+    const size_t verts_b = (static_cast<size_t>(n_items) * K * 2 * max_pts * sizeof(uint32_t) + 255) & ~static_cast<size_t>(255);
+    ContourWorkspace ws{2 * verts_b};
+    if (workspace != nullptr) {
+        uint8_t* base = static_cast<uint8_t*>(workspace);
+        ws.verts = reinterpret_cast<uint32_t*>(base);
+        ws.d2 = reinterpret_cast<uint32_t*>(base + verts_b);
+        ws.tail = reinterpret_cast<uint32_t*>(base + 2 * verts_b);
+    }
+    return ws;
+}
+}  // namespace octm
+
+// first occurrences of the classes of one label map per item, at first_pos[i * out_stride + c]
+static int launch_first_pos(const uint8_t* labels, int64_t n_items, int64_t item_elems, int num_classes, uint32_t* first_pos,
+                            long long out_stride, cudaStream_t s) {
+    const long long grid = n_items < 148 * 8 ? n_items : 148 * 8;
+    OCTM_TIMED("first_pos_kernel", s) octm::first_pos_kernel<<<static_cast<unsigned>(grid), 256, 0, s>>>(
+        labels, n_items, item_elems, num_classes, first_pos, out_stride);
+    return octm::check_launch("first_pos_kernel");
 }
 
 extern "C" int octm_first_pos_u8(const uint8_t* labels, int64_t n_items, int64_t item_elems, int num_classes,
@@ -2188,10 +2209,7 @@ extern "C" int octm_first_pos_u8(const uint8_t* labels, int64_t n_items, int64_t
         return octm::fail(OCTM_ERR_INVALID, "bad shape");
     if (n_items == 0) return OCTM_OK;
     if (!labels || !first_pos) return octm::fail(OCTM_ERR_INVALID, "null pointer");
-    const long long grid = n_items < 148 * 8 ? n_items : 148 * 8;
-    OCTM_TIMED("first_pos_kernel", static_cast<cudaStream_t>(stream)) octm::first_pos_kernel<<<static_cast<unsigned>(grid), 256, 0, static_cast<cudaStream_t>(stream)>>>(
-        labels, n_items, item_elems, num_classes, first_pos, num_classes);
-    return octm::check_launch("first_pos_kernel");
+    return launch_first_pos(labels, n_items, item_elems, num_classes, first_pos, num_classes, static_cast<cudaStream_t>(stream));
 }
 
 static bool layered_ok(const void* y_true, const void* y_pred, const void* bnd_true, const void* bnd_pred, int H, int W, int K) {
@@ -2203,14 +2221,7 @@ static bool layered_ok(const void* y_true, const void* y_pred, const void* bnd_t
 
 template <bool EMIT>
 static int launch_layered_trace(const octm::TraceParams& p, cudaStream_t s) {
-    int fit = 0;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&fit, octm::trace_layered_kernel<EMIT>, 128, 0) != cudaSuccess || fit < 1) {
-        cudaGetLastError();
-        fit = 8;
-    }
-    long long grid = (p.n_items * p.K * 2 + 3) / 4;
-    const long long cap = static_cast<long long>(octm::sm_count()) * fit;
-    if (grid > cap) grid = cap;
+    const long long grid = octm::resident_grid((p.n_items * p.K * 2 + 3) / 4, octm::trace_layered_kernel<EMIT>, 128, 0, 8);
     OCTM_TIMED("trace_layered_kernel", s) octm::trace_layered_kernel<EMIT><<<static_cast<unsigned>(grid), 128, 0, s>>>(p);
     return octm::check_launch("trace_layered_kernel");
 }
@@ -2240,16 +2251,10 @@ static int launch_walk(const octm::TraceParams& p_in, cudaStream_t s, int force_
         return launch_walk(p, s, 0);
     }
     if (force_words >= 0) words = words && force_words == 1;
-    const long long threads = p.n_items * p.K * 2;
-    int fit = 0;       // persistent grid: every CTA that can be resident (the walk is latency-bound: occupancy hides it)
-    if ((words ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&fit, octm::trace_kernel<true>, 128, 0)
-               : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&fit, octm::trace_kernel<false>, 128, 0)) != cudaSuccess || fit < 1) {
-        cudaGetLastError();
-        fit = 8;
-    }
-    long long grid = (threads + 127) / 128;
-    const long long cap = static_cast<long long>(octm::sm_count()) * fit;
-    if (grid > cap) grid = cap;
+    // persistent grid: every CTA that can be resident (the walk is latency-bound: occupancy hides it)
+    const long long want = (p.n_items * p.K * 2 + 127) / 128;
+    const long long grid = words ? octm::resident_grid(want, octm::trace_kernel<true>, 128, 0, 8)
+                                 : octm::resident_grid(want, octm::trace_kernel<false>, 128, 0, 8);
     if (words) OCTM_TIMED("trace_kernel", s) octm::trace_kernel<true><<<static_cast<unsigned>(grid), 128, 0, s>>>(p);
     else OCTM_TIMED("trace_kernel", s) octm::trace_kernel<false><<<static_cast<unsigned>(grid), 128, 0, s>>>(p);
     return octm::check_launch("trace_kernel");
@@ -2259,7 +2264,7 @@ extern "C" int octm_contour2d_trace_u8(const uint8_t* y_true, const uint8_t* y_p
                                        int num_classes, const uint32_t* first_pos, const int32_t* bnd_true,
                                        const int32_t* bnd_pred, int max_pts, uint32_t* verts, uint32_t* n_pts,
                                        uint32_t* flags, void* stream) {
-    if (int e = check_shape(n_items, H, W, num_classes, max_pts)) return e;
+    if (int e = octm::check_shape(n_items, H, W, num_classes, max_pts)) return e;
     if (n_items == 0) return OCTM_OK;
     if (!y_true || !y_pred || !first_pos || !verts || !n_pts || !flags) return octm::fail(OCTM_ERR_INVALID, "null pointer");
     if ((bnd_true == nullptr) != (bnd_pred == nullptr)) return octm::fail(OCTM_ERR_INVALID, "bnd_true/bnd_pred: both or neither");
@@ -2331,30 +2336,6 @@ __global__ void walk_report_kernel(const uint32_t* walk_count, uint32_t contours
     out[1] = contours;
     out[0] = *walk_count;
 }
-struct WalkReport {
-    uint32_t* host = nullptr;
-    uint32_t* dev = nullptr;
-};
-static WalkReport g_walk_report[64];
-static std::mutex g_walk_mu;
-static WalkReport* walk_report() {
-    int dev = -1;
-    if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) { cudaGetLastError(); return nullptr; }
-    std::lock_guard<std::mutex> lk(g_walk_mu);
-    WalkReport& r = g_walk_report[dev];
-    if (r.host == nullptr) {
-        void* h = nullptr;
-        void* d = nullptr;
-        if (cudaHostAlloc(&h, 2 * sizeof(uint32_t), cudaHostAllocMapped) != cudaSuccess || cudaHostGetDevicePointer(&d, h, 0) != cudaSuccess) {
-            cudaGetLastError();
-            return nullptr;
-        }
-        r.host = static_cast<uint32_t*>(h);
-        r.dev = static_cast<uint32_t*>(d);
-        r.host[0] = r.host[1] = 0;
-    }
-    return &r;
-}
 }  // namespace octm
 
 extern "C" int octm_contour2d_metrics_u8(const uint8_t* y_true, const uint8_t* y_pred, int64_t n_items, int H, int W,
@@ -2362,17 +2343,17 @@ extern "C" int octm_contour2d_metrics_u8(const uint8_t* y_true, const uint8_t* y
                                          const int32_t* bnd_pred, const uint32_t* unsorted, int max_pts, uint32_t* n_pts,
                                          uint32_t* flags, uint32_t* max_sq, uint32_t* p95_sq, double* sum_dist,
                                          void* workspace, size_t workspace_bytes, void* stream) {
-    if (int e = check_shape(n_items, H, W, num_classes, max_pts)) return e;
+    if (int e = octm::check_shape(n_items, H, W, num_classes, max_pts)) return e;
     if (n_items == 0) return OCTM_OK;
     if (!y_true || !y_pred || !first_pos || !n_pts || !flags || !max_sq || !p95_sq || !sum_dist)
         return octm::fail(OCTM_ERR_INVALID, "null pointer");
     if ((bnd_true == nullptr) != (bnd_pred == nullptr)) return octm::fail(OCTM_ERR_INVALID, "bnd_true/bnd_pred: both or neither");
-    const size_t verts_b = (static_cast<size_t>(n_items) * num_classes * 2 * max_pts * sizeof(uint32_t) + 255) & ~static_cast<size_t>(255);
-    if (workspace == nullptr || workspace_bytes < 2 * verts_b + 256)
-        return octm::fail(OCTM_ERR_WORKSPACE, "workspace too small: need %zu B", 2 * verts_b + 256);
-    uint32_t* verts = static_cast<uint32_t*>(workspace);
-    uint32_t* d2 = reinterpret_cast<uint32_t*>(static_cast<uint8_t*>(workspace) + verts_b);
-    uint32_t* todo = reinterpret_cast<uint32_t*>(static_cast<uint8_t*>(workspace) + 2 * verts_b);
+    const octm::ContourWorkspace ws = octm::contour_workspace(n_items, num_classes, max_pts, workspace);
+    if (workspace == nullptr || workspace_bytes < ws.tail_offset + 256)       // the tail: the pass counters
+        return octm::fail(OCTM_ERR_WORKSPACE, "workspace too small: need %zu B", ws.tail_offset + 256);
+    uint32_t* verts = ws.verts;
+    uint32_t* d2 = ws.d2;
+    uint32_t* todo = ws.tail;
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     const int tab = (2 * W - 1 + 2 * octm::kLdPad + 7) & ~7;
     const size_t smem = static_cast<size_t>(tab) * 8 + octm::kCountBins * 4 + octm::kLdWarps * octm::kLdRing * 4;
@@ -2402,14 +2383,7 @@ extern "C" int octm_contour2d_metrics_u8(const uint8_t* y_true, const uint8_t* y
         const size_t smem = smem_pass;
         if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)) != cudaSuccess)
             return octm::fail(OCTM_ERR_LAUNCH, "cudaFuncSetAttribute(layered_distance_kernel) failed");
-        int fit = 0;
-        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&fit, kern, octm::kLdWarps * 32, smem) != cudaSuccess || fit < 1) {
-            cudaGetLastError();
-            fit = 1;
-        }
-        long long grid = n_pairs;
-        const long long cap = static_cast<long long>(octm::sm_count()) * fit;
-        if (grid > cap) grid = cap;
+        long long grid = octm::resident_grid(n_pairs, kern, octm::kLdWarps * 32, smem, 1);
         // a CTA strides over the pairs by the grid size: keep the stride coprime to the class count, or every CTA would
         // meet one class only (and the classes differ: the class after pixel (0, 0)'s is usually a copy, not a search)
         while (grid > 1 && std::gcd(grid, static_cast<long long>(num_classes)) != 1) --grid;
@@ -2421,7 +2395,7 @@ extern "C" int octm_contour2d_metrics_u8(const uint8_t* y_true, const uint8_t* y
                         bnd_true, bnd_pred, true, todo, d2, todo + 2, 0, unsorted, 0};     // the walk list borrows the distance scratch
     // The order of the first two steps follows the data (the label pass's report of how many maps its certificate
     // rejected, octm_label_pass_seed_policy): same results either way.
-    octm::WalkReport* wr = octm::stream_mostly_rejected() ? octm::walk_report() : nullptr;
+    octm::HostReport* wr = octm::stream_mostly_rejected() ? octm::host_report(octm::kReportWalks) : nullptr;
     // (pinned "noisy": always rows first, so that tests reach this order whatever ran before them)
     const bool few_walks = wr != nullptr && (octm_label_pass_seed_policy(-1) == 2 ||
                                              static_cast<unsigned long long>(*static_cast<volatile uint32_t*>(wr->host)) * 4ull <=
@@ -2460,39 +2434,31 @@ extern "C" int octm_contour2d_metrics_u8(const uint8_t* y_true, const uint8_t* y
 extern "C" size_t octm_contour2d_workspace_bytes(int64_t n_items, int H, int W, int num_classes, int max_pts) {
     (void)H; (void)W;
     if (n_items <= 0 || num_classes < 1 || max_pts < 1) return 0;
-    const size_t verts = static_cast<size_t>(n_items) * num_classes * 2 * max_pts * sizeof(uint32_t);
     const size_t first = static_cast<size_t>(n_items) * 2 * num_classes * sizeof(uint32_t);
-    // vertices, squared-distance scratch (same shape), first occurrences
-    return 2 * ((verts + 255) & ~static_cast<size_t>(255)) + ((first + 255) & ~static_cast<size_t>(255));
+    // vertices, squared-distance scratch, then the first occurrences of octm_contour2d_u8 in the tail
+    return octm::contour_workspace(n_items, num_classes, max_pts).tail_offset + ((first + 255) & ~static_cast<size_t>(255));
 }
 
 extern "C" int octm_contour2d_u8(const uint8_t* y_true, const uint8_t* y_pred, int64_t n_items, int H, int W,
                                  int num_classes, const uint32_t* first_pos, int max_pts, uint32_t* n_pts,
                                  uint32_t* flags, uint32_t* max_sq, uint32_t* p95_sq, double* sum_dist, void* workspace,
                                  size_t workspace_bytes, void* stream) {
-    if (int e = check_shape(n_items, H, W, num_classes, max_pts)) return e;
+    if (int e = octm::check_shape(n_items, H, W, num_classes, max_pts)) return e;
     if (n_items == 0) return OCTM_OK;
     if (workspace == nullptr || workspace_bytes < octm_contour2d_workspace_bytes(n_items, H, W, num_classes, max_pts))
         return octm::fail(OCTM_ERR_WORKSPACE, "workspace too small: need %zu B",
                           octm_contour2d_workspace_bytes(n_items, H, W, num_classes, max_pts));
-    uint32_t* verts = static_cast<uint32_t*>(workspace);
-    const size_t verts_b = (static_cast<size_t>(n_items) * num_classes * 2 * max_pts * sizeof(uint32_t) + 255) & ~static_cast<size_t>(255);
-    uint32_t* d2_ws = reinterpret_cast<uint32_t*>(static_cast<uint8_t*>(workspace) + verts_b);
-    uint32_t* fp_ws = reinterpret_cast<uint32_t*>(static_cast<uint8_t*>(workspace) + 2 * verts_b);
+    const octm::ContourWorkspace ws = octm::contour_workspace(n_items, num_classes, max_pts, workspace);
     if (first_pos == nullptr) {
         // no label pass ran: find the first occurrences of both maps here, interleaved [n][2][K]
-        const long long grid = n_items < 148 * 8 ? n_items : 148 * 8;
         cudaStream_t s = static_cast<cudaStream_t>(stream);
-        OCTM_TIMED("first_pos_kernel", s) octm::first_pos_kernel<<<static_cast<unsigned>(grid), 256, 0, s>>>(y_true, n_items, static_cast<long long>(H) * W,
-                                                                         num_classes, fp_ws, 2 * num_classes);
-        if (int e = octm::check_launch("first_pos_kernel")) return e;
-        OCTM_TIMED("first_pos_kernel", s) octm::first_pos_kernel<<<static_cast<unsigned>(grid), 256, 0, s>>>(y_pred, n_items, static_cast<long long>(H) * W,
-                                                                         num_classes, fp_ws + num_classes, 2 * num_classes);
-        if (int e = octm::check_launch("first_pos_kernel")) return e;
-        first_pos = fp_ws;
+        if (int e = launch_first_pos(y_true, n_items, static_cast<long long>(H) * W, num_classes, ws.tail, 2 * num_classes, s)) return e;
+        if (int e = launch_first_pos(y_pred, n_items, static_cast<long long>(H) * W, num_classes, ws.tail + num_classes, 2 * num_classes, s))
+            return e;
+        first_pos = ws.tail;
     }
-    if (int e = octm_contour2d_trace_u8(y_true, y_pred, n_items, H, W, num_classes, first_pos, nullptr, nullptr, max_pts, verts, n_pts,
-                                        flags, stream))
+    if (int e = octm_contour2d_trace_u8(y_true, y_pred, n_items, H, W, num_classes, first_pos, nullptr, nullptr, max_pts, ws.verts,
+                                        n_pts, flags, stream))
         return e;
-    return octm_contour2d_distance(verts, n_pts, n_items, num_classes, max_pts, H, W, max_sq, p95_sq, sum_dist, d2_ws, 0, stream);
+    return octm_contour2d_distance(ws.verts, n_pts, n_items, num_classes, max_pts, H, W, max_sq, p95_sq, sum_dist, ws.d2, 0, stream);
 }

@@ -18,9 +18,6 @@
 // The distance stage is the one of the contour [0] path (octm_contour2d_distance): it takes any vertex lists.
 #include "common.cuh"
 
-// contour.cu: the shape checks every contour entry point shares
-int check_shape(int64_t n, int H, int W, int K, int max_pts);
-
 namespace octm {
 
 constexpr int kAllWarps = 8;
@@ -191,7 +188,7 @@ __global__ void __launch_bounds__(kAllWarps * 32, 3) contour_all_vertices_kernel
 extern "C" int octm_contour2d_all_vertices_u8(const uint8_t* y_true, const uint8_t* y_pred, int64_t n_items, int H, int W,
                                               int num_classes, int max_pts, uint32_t* verts, uint32_t* n_pts,
                                               uint32_t* flags, void* stream) {
-    if (int e = check_shape(n_items, H, W, num_classes, max_pts)) return e;
+    if (int e = octm::check_shape(n_items, H, W, num_classes, max_pts)) return e;
     if (n_items == 0) return OCTM_OK;
     if (!y_true || !y_pred || !verts || !n_pts || !flags) return octm::fail(OCTM_ERR_INVALID, "null pointer");
     cudaStream_t s = static_cast<cudaStream_t>(stream);
@@ -210,17 +207,14 @@ extern "C" int octm_contour2d_all_u8(const uint8_t* y_true, const uint8_t* y_pre
                                      int num_classes, int max_pts, uint32_t* n_pts, uint32_t* flags, uint32_t* max_sq,
                                      uint32_t* p95_sq, double* sum_dist, void* workspace, size_t workspace_bytes,
                                      void* stream) {
-    if (int e = check_shape(n_items, H, W, num_classes, max_pts)) return e;
+    if (int e = octm::check_shape(n_items, H, W, num_classes, max_pts)) return e;
     if (n_items == 0) return OCTM_OK;
     if (!y_true || !y_pred || !n_pts || !flags || !max_sq || !p95_sq || !sum_dist)
         return octm::fail(OCTM_ERR_INVALID, "null pointer");
     const size_t need = octm_contour2d_workspace_bytes(n_items, H, W, num_classes, max_pts);
     if (workspace == nullptr || workspace_bytes < need) return octm::fail(OCTM_ERR_WORKSPACE, "workspace too small: need %zu B", need);
-    // workspace layout of octm_contour2d_u8: vertices, then the squared-distance scratch
-    uint32_t* verts = static_cast<uint32_t*>(workspace);
-    const size_t verts_b = (static_cast<size_t>(n_items) * num_classes * 2 * max_pts * sizeof(uint32_t) + 255) & ~static_cast<size_t>(255);
-    uint32_t* d2 = reinterpret_cast<uint32_t*>(static_cast<uint8_t*>(workspace) + verts_b);
-    if (int e = octm_contour2d_all_vertices_u8(y_true, y_pred, n_items, H, W, num_classes, max_pts, verts, n_pts, flags, stream))
+    const octm::ContourWorkspace ws = octm::contour_workspace(n_items, num_classes, max_pts, workspace);
+    if (int e = octm_contour2d_all_vertices_u8(y_true, y_pred, n_items, H, W, num_classes, max_pts, ws.verts, n_pts, flags, stream))
         return e;
-    return octm_contour2d_distance(verts, n_pts, n_items, num_classes, max_pts, H, W, max_sq, p95_sq, sum_dist, d2, 0, stream);
+    return octm_contour2d_distance(ws.verts, n_pts, n_items, num_classes, max_pts, H, W, max_sq, p95_sq, sum_dist, ws.d2, 0, stream);
 }

@@ -34,7 +34,6 @@
 #include <cuda.h>      // CUtensorMap (type only; the encoder is fetched through cudaGetDriverEntryPoint)
 
 #include <cstdlib>
-#include <mutex>
 
 #include "common.cuh"
 
@@ -1196,13 +1195,7 @@ static int launch_fast(const LabelPassParams& p0, cudaStream_t stream) {
     if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, budget) != cudaSuccess)
         return fail(OCTM_ERR_LAUNCH, "cudaFuncSetAttribute(label_pass_fast) failed");
     const int threads = NW * 32;
-    int per_sm = 0;      // persistent grid: exactly the CTAs that are resident at once
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, threads, smem) != cudaSuccess || per_sm < 1) {
-        cudaGetLastError();
-        per_sm = 1;
-    }
-    long long grid = static_cast<long long>(sm_count()) * per_sm;
-    if (grid > p.n_items) grid = p.n_items;
+    const long long grid = resident_grid(p.n_items, kern, threads, smem, 1);      // persistent: the CTAs resident at once
     OCTM_TIMED("label_pass_fast", stream) kern<<<static_cast<unsigned>(grid), threads, smem, stream>>>(p, tm_true, tm_pred);
     if (int e = check_launch("label_pass_fast")) return e;
     if (SORT && !SEEDS && p.first_pos != nullptr) {
@@ -1251,17 +1244,11 @@ static int launch_generic(const LabelPassParams& p, cudaStream_t stream) {
     if (p.unsorted != nullptr && cudaMemsetAsync(p.unsorted, 0, static_cast<size_t>(p.n_items) * 4, stream) != cudaSuccess)
         return fail(OCTM_ERR_LAUNCH, "memset of the label-pass outputs failed");
     if (wide) {
-        int fit = 0;
         const int kWideSmem = kWideWarps * wide_warp_bytes(p.K);
         if (cudaFuncSetAttribute(label_pass_wide, cudaFuncAttributeMaxDynamicSharedMemorySize, kWideWarps * wide_warp_bytes(16)) != cudaSuccess)
             return fail(OCTM_ERR_LAUNCH, "cudaFuncSetAttribute(label_pass_wide) failed");
-        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&fit, label_pass_wide, kWideWarps * 32, kWideSmem) != cudaSuccess || fit < 1) {
-            cudaGetLastError();
-            fit = 3;
-        }
-        long long grid = (p.n_items * strips + kWideWarps - 1) / kWideWarps;
-        const long long cap = static_cast<long long>(sm_count()) * fit;
-        if (grid > cap) grid = cap;
+        const long long grid = resident_grid((p.n_items * strips + kWideWarps - 1) / kWideWarps, label_pass_wide, kWideWarps * 32,
+                                             kWideSmem, 3);
         OCTM_TIMED("label_pass_wide", stream) label_pass_wide<<<static_cast<unsigned>(grid), kWideWarps * 32, kWideSmem, stream>>>(p, strips);
         return check_launch("label_pass_wide");
     }
@@ -1279,33 +1266,8 @@ static int launch_generic(const LabelPassParams& p, cudaStream_t stream) {
 // leaves "maps rejected / maps seen" in a host-mapped word (one tiny kernel, no synchronisation: the next call reads
 // whatever has arrived), and a call tracks per pixel when more than a fifth of the maps of the last report were
 // rejected.  Both ways give the same seeds (tests run both); octm_label_pass_seed_policy pins one.
-struct SeedFeedback {
-    uint32_t* host = nullptr;      // mapped, pinned: [0] rejected maps, [1] maps
-    uint32_t* dev = nullptr;       // the device's view of it
-};
-static SeedFeedback g_seed_fb[64];
-static std::mutex g_seed_mu;
+// The report: host_report(kReportSeeds), [0] rejected maps, [1] maps.
 static std::atomic<int> g_seed_policy{0};      // 0 follow the data, 1 column totals + rescan, 2 per pixel
-
-static SeedFeedback* seed_feedback() {
-    int dev = -1;
-    if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) { cudaGetLastError(); return nullptr; }
-    std::lock_guard<std::mutex> lk(g_seed_mu);
-    SeedFeedback& f = g_seed_fb[dev];
-    if (f.host == nullptr) {
-        void* h = nullptr;
-        void* d = nullptr;
-        if (cudaHostAlloc(&h, 2 * sizeof(uint32_t), cudaHostAllocMapped) != cudaSuccess ||
-            cudaHostGetDevicePointer(&d, h, 0) != cudaSuccess) {
-            cudaGetLastError();
-            return nullptr;
-        }
-        f.host = static_cast<uint32_t*>(h);
-        f.dev = static_cast<uint32_t*>(d);
-        f.host[0] = f.host[1] = 0;
-    }
-    return &f;
-}
 
 __global__ void __launch_bounds__(1024) seed_feedback_kernel(const uint32_t* __restrict__ unsorted, long long n, uint32_t* out) {
     __shared__ uint32_t s_sum[32];
@@ -1328,14 +1290,14 @@ static bool seeds_per_pixel() { return stream_mostly_rejected(); }
 bool stream_mostly_rejected() {
     const int policy = g_seed_policy.load();
     if (policy != 0) return policy == 2;
-    SeedFeedback* f = seed_feedback();
+    HostReport* f = host_report(kReportSeeds);
     if (f == nullptr) return false;
     const uint32_t rejected = *static_cast<volatile uint32_t*>(f->host), maps = *static_cast<volatile uint32_t*>(f->host + 1);
     return maps != 0 && static_cast<unsigned long long>(rejected) * 5ull > maps;
 }
 
 static int report_rejected(const LabelPassParams& p, cudaStream_t stream) {
-    SeedFeedback* f = seed_feedback();
+    HostReport* f = host_report(kReportSeeds);
     if (f == nullptr) return OCTM_OK;
     OCTM_TIMED("seed_feedback_kernel", stream) seed_feedback_kernel<<<1, 1024, 0, stream>>>(p.unsorted, p.n_items, f->dev);
     return check_launch("seed_feedback_kernel");

@@ -275,72 +275,47 @@ def _vertex_scratch(dev, numel):
     return buf[:numel]
 
 
-def _contour_chunk(yt, yp, k, first_pos, max_pts, want_verts, want_sq, timers=None, bnd=None, unsorted=None,
-                   mode="first"):
-    if mode == "all":
-        return _contour_chunk_all(yt, yp, k, max_pts, want_verts, want_sq, timers)
-    n, h, w = yt.shape
-    max_pts = (int(max_pts) + 3) & ~3          # vertices are stored in 16-byte groups
-    dev = yt.device
+def _contour_outputs(n, k, dev):
+    """Empty ``n_pts``, ``flags``, ``max_sq``, ``p95_sq``, ``sum_dist`` of ``n`` items (the ``ContourOut`` order)."""
     i32 = dict(dtype=torch.int32, device=dev)
-    numel = (n * k * 2 * max_pts + 63) & ~63          # 256-byte multiples (octm_contour2d_metrics_u8's workspace layout)
-    # stream-ordered reuse: every consumer of the scratch is enqueued on the same stream
-    scratch = None if (want_verts and want_sq) else _vertex_scratch(dev, 2 * numel + 64)
-    nv = n * k * 2 * max_pts
-    verts = torch.empty((n, k, 2, max_pts), **i32) if want_verts else scratch[:nv].view(n, k, 2, max_pts)
-    sq = torch.empty((n, k, 2, max_pts), **i32) if want_sq else scratch[numel:numel + nv].view(n, k, 2, max_pts)
-    n_pts = torch.empty((n, k, 2), **i32)
-    flags = torch.empty((n, k), **i32)
-    max_sq = torch.empty((n, k, 2), **i32)
-    p95 = torch.empty((n, k, 2, 2), **i32)
-    sums = torch.empty((n, k, 2), dtype=torch.float64, device=dev)
-    if bnd is not None and not want_verts and not want_sq:
-        # the production path: layered pairs are measured from the boundary rows, the rest through vertex lists
-        with _Timed(timers, "contour"):
-            _lib.call("octm_contour2d_metrics_u8", _ptr(yt), _ptr(yp), n, h, w, k, _ptr(first_pos), _ptr(bnd[0]),
-                      _ptr(bnd[1]), _ptr(unsorted), max_pts, _ptr(n_pts), _ptr(flags), _ptr(max_sq), _ptr(p95), _ptr(sums),
-                      _ptr(scratch), scratch.numel() * 4, _stream())
-        return ContourOut(n_pts, flags, max_sq, p95, sums, None, None, max_pts)
-    with _Timed(timers, "contour_trace"):
-        _lib.call("octm_contour2d_trace_u8", _ptr(yt), _ptr(yp), n, h, w, k, _ptr(first_pos),
-                  _ptr(bnd[0]) if bnd else None, _ptr(bnd[1]) if bnd else None, max_pts, _ptr(verts),
-                  _ptr(n_pts), _ptr(flags), _stream())
-    with _Timed(timers, "contour_distance"):
-        _lib.call("octm_contour2d_distance", _ptr(verts), _ptr(n_pts), n, k, max_pts, h, w, _ptr(max_sq), _ptr(p95),
-                  _ptr(sums), _ptr(sq), 1 if want_sq else 0, _stream())
-    return ContourOut(n_pts, flags, max_sq, p95, sums, verts if want_verts else None, sq if want_sq else None, max_pts)
+    return (torch.empty((n, k, 2), **i32), torch.empty((n, k), **i32), torch.empty((n, k, 2), **i32),
+            torch.empty((n, k, 2, 2), **i32), torch.empty((n, k, 2), dtype=torch.float64, device=dev))
 
 
-def _contour_chunk_all(yt, yp, k, max_pts, want_verts, want_sq, timers=None):
-    """``mode="all"``: every boundary vertex of every class (octm_contour2d_all_*), then the same distance stage."""
+def _contour_chunk(yt, yp, k, max_pts, mode, want_verts, want_sq, timers=None, first_pos=None, bnd=None, unsorted=None):
+    """One chunk of ``contour_pass``.  Metrics alone take the one-call entry point of ``mode`` on the shared scratch;
+    requested vertices or squared distances take the vertex emitter of ``mode``, then ``octm_contour2d_distance``."""
     n, h, w = yt.shape
     dev = yt.device
-    i32 = dict(dtype=torch.int32, device=dev)
-    numel = (n * k * 2 * max_pts + 63) & ~63          # 256-byte multiples (the workspace layout of the C ABI)
-    nv = n * k * 2 * max_pts
-    n_pts = torch.empty((n, k, 2), **i32)
-    flags = torch.empty((n, k), **i32)
-    max_sq = torch.empty((n, k, 2), **i32)
-    p95 = torch.empty((n, k, 2, 2), **i32)
-    sums = torch.empty((n, k, 2), dtype=torch.float64, device=dev)
+    n_pts, flags, max_sq, p95, sums = _contour_outputs(n, k, dev)
+    bt, bp = (None, None) if bnd is None else bnd
     if not want_verts and not want_sq:
-        ws_bytes = int(_lib.load().octm_contour2d_workspace_bytes(n, h, w, k, max_pts))
-        scratch = _vertex_scratch(dev, (ws_bytes + 3) // 4)
+        # stream-ordered reuse: every consumer of the scratch is enqueued on the same stream
+        scratch = _vertex_scratch(dev, (int(_lib.load().octm_contour2d_workspace_bytes(n, h, w, k, max_pts)) + 3) // 4)
         with _Timed(timers, "contour"):
-            _lib.call("octm_contour2d_all_u8", _ptr(yt), _ptr(yp), n, h, w, k, max_pts, _ptr(n_pts), _ptr(flags),
-                      _ptr(max_sq), _ptr(p95), _ptr(sums), _ptr(scratch), scratch.numel() * 4, _stream())
-        return ContourOut(n_pts, flags, max_sq, p95, sums, None, None, max_pts, "all")
-    scratch = None if (want_verts and want_sq) else _vertex_scratch(dev, 2 * numel + 64)
-    verts = torch.empty((n, k, 2, max_pts), **i32) if want_verts else scratch[:nv].view(n, k, 2, max_pts)
-    sq = torch.empty((n, k, 2, max_pts), **i32) if want_sq else scratch[numel:numel + nv].view(n, k, 2, max_pts)
+            if mode == "first":
+                # layered pairs (with boundary rows and certificate) are measured from the rows, the rest from vertex lists
+                _lib.call("octm_contour2d_metrics_u8", _ptr(yt), _ptr(yp), n, h, w, k, _ptr(first_pos), _ptr(bt), _ptr(bp),
+                          _ptr(unsorted), max_pts, _ptr(n_pts), _ptr(flags), _ptr(max_sq), _ptr(p95), _ptr(sums),
+                          _ptr(scratch), scratch.numel() * 4, _stream())
+            else:
+                _lib.call("octm_contour2d_all_u8", _ptr(yt), _ptr(yp), n, h, w, k, max_pts, _ptr(n_pts), _ptr(flags),
+                          _ptr(max_sq), _ptr(p95), _ptr(sums), _ptr(scratch), scratch.numel() * 4, _stream())
+        return ContourOut(n_pts, flags, max_sq, p95, sums, None, None, max_pts, mode)
+    verts = torch.empty((n, k, 2, max_pts), dtype=torch.int32, device=dev)
+    sq = torch.empty((n, k, 2, max_pts), dtype=torch.int32, device=dev)
     with _Timed(timers, "contour_trace"):
-        _lib.call("octm_contour2d_all_vertices_u8", _ptr(yt), _ptr(yp), n, h, w, k, max_pts, _ptr(verts), _ptr(n_pts),
-                  _ptr(flags), _stream())
+        if mode == "first":
+            _lib.call("octm_contour2d_trace_u8", _ptr(yt), _ptr(yp), n, h, w, k, _ptr(first_pos), _ptr(bt), _ptr(bp),
+                      max_pts, _ptr(verts), _ptr(n_pts), _ptr(flags), _stream())
+        else:
+            _lib.call("octm_contour2d_all_vertices_u8", _ptr(yt), _ptr(yp), n, h, w, k, max_pts, _ptr(verts),
+                      _ptr(n_pts), _ptr(flags), _stream())
     with _Timed(timers, "contour_distance"):
         _lib.call("octm_contour2d_distance", _ptr(verts), _ptr(n_pts), n, k, max_pts, h, w, _ptr(max_sq), _ptr(p95),
                   _ptr(sums), _ptr(sq), 1 if want_sq else 0, _stream())
     return ContourOut(n_pts, flags, max_sq, p95, sums, verts if want_verts else None, sq if want_sq else None, max_pts,
-                      "all")
+                      mode)
 
 
 def contour_pass(y_true, y_pred, num_classes, first_pos=None, *, max_pts=None, return_vertices=False,
@@ -382,19 +357,16 @@ def contour_pass(y_true, y_pred, num_classes, first_pos=None, *, max_pts=None, r
                 first_pos[:, m, :] = tmp
         keep = return_vertices or return_sq
         if n == 0:
-            i32 = dict(dtype=torch.int32, device=dev)
-            return ContourOut(torch.empty((0, k, 2), **i32), torch.empty((0, k), **i32), torch.empty((0, k, 2), **i32),
-                              torch.empty((0, k, 2, 2), **i32), torch.empty((0, k, 2), dtype=torch.float64, device=dev),
-                              None, None, max_pts, mode)
+            return ContourOut(*_contour_outputs(0, k, dev), None, None, max_pts, mode)
         per_item = k * 2 * max_pts * 4 * 2          # vertices + squared-distance scratch
         chunk = n if keep else max(1, min(n, CONTOUR_CHUNK_BYTES // per_item))
         parts = []
         for s in range(0, n, chunk):
             e = min(n, s + chunk)
-            parts.append(_contour_chunk(yt[s:e], yp[s:e], k, None if first_pos is None else first_pos[s:e], max_pts,
-                                        return_vertices, return_sq, timers,
+            parts.append(_contour_chunk(yt[s:e], yp[s:e], k, max_pts, mode, return_vertices, return_sq, timers,
+                                        None if first_pos is None else first_pos[s:e],
                                         None if boundaries is None else (boundaries[0][s:e], boundaries[1][s:e]),
-                                        None if unsorted is None else unsorted[s:e], mode))
+                                        None if unsorted is None else unsorted[s:e]))
         if len(parts) == 1:
             out = parts[0]
         else:
@@ -418,41 +390,31 @@ def _retry_overflow(out, yt, yp, k, first_pos, keep=False):
     over = ((out.flags & over_bits) != 0).any(dim=1)
     if not bool(over.any()):
         return False
-    if out.mode == "all":
-        return _retry_overflow_all(out, yt, yp, k, over, keep)
-    if keep:
-        raise _lib.OctmError(f"a contour has more than max_pts={out.max_pts} vertices; raise max_pts")
     idx = torch.nonzero(over).flatten()
     big = max(int(out.max_pts), 8)
     while idx.numel():
-        if big >= MAX_MAX_PTS:
-            raise _lib.OctmError(f"a contour has more than {MAX_MAX_PTS} vertices: pass a larger max_pts")
-        big = min(big * 8, MAX_MAX_PTS)
-        per_item = k * 2 * big * 4 * 2
-        chunk = max(1, CONTOUR_CHUNK_BYTES // per_item)
+        if out.mode == "all":
+            big = (int(out.n_pts[idx].max()) + 3) & ~3
+            if keep:
+                raise _lib.OctmError(f"a class has {big} boundary vertices (rounded up to a multiple of 4), more than "
+                                     f"max_pts={out.max_pts}; pass max_pts >= {big}")
+        else:
+            if keep:
+                raise _lib.OctmError(f"a contour has more than max_pts={out.max_pts} vertices; raise max_pts")
+            if big >= MAX_MAX_PTS:
+                raise _lib.OctmError(f"a contour has more than {MAX_MAX_PTS} vertices: pass a larger max_pts")
+            big = min(big * 8, MAX_MAX_PTS)
+        chunk = max(1, CONTOUR_CHUNK_BYTES // (k * 2 * big * 4 * 2))
         still = []
         for s0 in range(0, idx.numel(), chunk):
             sub = idx[s0:s0 + chunk]
-            redo = _contour_chunk(yt[sub].contiguous(), yp[sub].contiguous(), k, first_pos[sub].contiguous(), big, False, False)
+            redo = _contour_chunk(yt[sub].contiguous(), yp[sub].contiguous(), k, big, out.mode, False, False,
+                                  first_pos=None if first_pos is None else first_pos[sub].contiguous())
             for f in ("n_pts", "flags", "max_sq", "p95_sq", "sum_dist"):
                 getattr(out, f)[sub] = getattr(redo, f)
-            still.append(sub[((redo.flags & over_bits) != 0).any(dim=1)])
-        idx = torch.cat(still)
-    return True
-
-
-def _retry_overflow_all(out, yt, yp, k, over, keep):
-    idx = torch.nonzero(over).flatten()
-    need = (int(out.n_pts[idx].max()) + 3) & ~3
-    if keep:
-        raise _lib.OctmError(f"a class has {need} boundary vertices (rounded up to a multiple of 4), more than "
-                             f"max_pts={out.max_pts}; pass max_pts >= {need}")
-    chunk = max(1, CONTOUR_CHUNK_BYTES // (k * 2 * need * 4 * 2))
-    for s0 in range(0, idx.numel(), chunk):
-        sub = idx[s0:s0 + chunk]
-        redo = _contour_chunk_all(yt[sub].contiguous(), yp[sub].contiguous(), k, need, False, False)
-        for f in ("n_pts", "flags", "max_sq", "p95_sq", "sum_dist"):
-            getattr(out, f)[sub] = getattr(redo, f)
+            if out.mode == "first":
+                still.append(sub[((redo.flags & over_bits) != 0).any(dim=1)])
+        idx = torch.cat(still) if still else idx[:0]      # "all": no count exceeds the bound of this round
     return True
 
 
@@ -607,24 +569,20 @@ def evaluate(y_true, y_pred, num_classes, *, contours=True, boundaries=False, ma
     class but drops it, so the item's confusion counts do not add up to H * W, which the totals kernel counts."""
     mode = _contour_mode(contours)
     yt, yp = _check_pair(y_true, y_pred)
-    if mode == "all":
-        lp = label_pass(yt, yp, num_classes, counts=True, columns=True, boundaries=boundaries, timers=timers)
-        ct = contour_pass(yt, yp, num_classes, max_pts=max_pts, timers=timers, check_overflow=False, mode="all")
-        cls, bnd, tot = derive_on_device(lp, ct, yt.shape[0], timers)
-        return SuiteResult(yt.shape[0], lp, ct, cls, bnd, tot, (yt, yp), validate=bool(validate), contour_mode="all")
-    contours = mode == "first"
-    # the contour stage uses the label pass's boundary rows to skip the walk on layered maps
-    lp = label_pass(yt, yp, num_classes, counts=True, columns=True, seeds=contours, boundaries=boundaries or contours,
-                    timers=timers, certify=contours)
+    first = mode == "first"
+    # contour [0] is seeded by the label pass, and its boundary rows and certificate skip the walk on layered maps
+    lp = label_pass(yt, yp, num_classes, counts=True, columns=True, seeds=first, boundaries=boundaries or first,
+                    timers=timers, certify=first)
     ct = None
-    if contours:
+    if mode is not None:
         ct = contour_pass(yt, yp, num_classes, lp.first_pos, max_pts=max_pts, timers=timers, check_overflow=False,
-                          boundaries=(lp.bnd_true, lp.bnd_pred), unsorted=lp.unsorted)
-        if not boundaries:
+                          boundaries=(lp.bnd_true, lp.bnd_pred) if first else None,
+                          unsorted=lp.unsorted if first else None, mode=mode)
+        if first and not boundaries:
             lp.bnd_true = lp.bnd_pred = None
     cls, bnd, tot = derive_on_device(lp, ct, yt.shape[0], timers)
-    return SuiteResult(yt.shape[0], lp, ct, cls, bnd, tot, (yt, yp) if contours else None, validate=bool(validate),
-                       contour_mode=mode)
+    return SuiteResult(yt.shape[0], lp, ct, cls, bnd, tot, (yt, yp) if ct is not None else None,
+                       validate=bool(validate), contour_mode=mode)
 
 
 def _cat_results(parts):
