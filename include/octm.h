@@ -248,6 +248,27 @@ OCTM_API int octm_contour2d_all_u8(const uint8_t* y_true, const uint8_t* y_pred,
                           void* stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * Normalized surface Dice at tolerance tau (build-defined, no reference counterpart; MONAI compute_surface_dice,
+ * surface-distance compute_surface_dice_at_tolerance): the share of both boundaries that lies within tau of the other.
+ * The surfaces are the all-contour vertex sets V_t, V_p of octm_contour2d_all_vertices_u8, whatever contour mode the
+ * other metrics use.  Per (item i, class c) and integer threshold T_j (squared doubled-lattice distance; for a
+ * tolerance of tau pixels, T = max{D : sqrt(D / 4.0) <= tau}, the expression every contour distance here is reported
+ * through):
+ *   n_surf    uint32 [n][K][2]             (|V_t|, |V_p|), as n_pts of octm_contour2d_all_vertices_u8
+ *   n_within  uint32 [n][K][2][n_thresholds]  [..][0][j] = #{v in V_p : min_{u in V_t} |v - u|^2 <= T_j} (pred -> true,
+ *                                          direction 0 as elsewhere), [..][1][j] the same for V_t against V_p
+ *   NSD_j = (n_within[..][0][j] + n_within[..][1][j]) / (|V_t| + |V_p|): NaN when both sets are empty, 0 when one is.
+ * thresholds_sq is a HOST array of parameters, not data (the exception to the device-pointer rule): 1 to
+ * OCTM_SURFACE_DICE_MAX_TOL values in ascending order, each <= OCTM_SURFACE_DICE_MAX_SQ (tau <= 8 px), read before the
+ * call returns.  Counts are exact (no workspace, no overflow); one read of each label map. */
+#define OCTM_SURFACE_DICE_MAX_TOL 4
+#define OCTM_SURFACE_DICE_MAX_SQ 256      /* T(8 px) */
+OCTM_API int octm_surface_dice_u8(const uint8_t* y_true, const uint8_t* y_pred, int64_t n_items, int H, int W,
+                                  int num_classes, const uint32_t* thresholds_sq /* HOST array, ascending */,
+                                  int n_thresholds, uint32_t* n_surf /* [n][K][2] */,
+                                  uint32_t* n_within /* [n][K][2][n_thresholds] */, void* stream);
+
+/* ---------------------------------------------------------------------------------------------
  * Boundary rows -> label maps (SURVEY.md 8f-4: the layer datasets catalogued in the reference's
  * Datasets.md:3-26 annotate boundary curves, while Metrics/*.py score masks).  The inverse of the label
  * pass's boundary rows on layered maps:

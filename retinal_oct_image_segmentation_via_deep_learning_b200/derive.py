@@ -106,3 +106,51 @@ def contour_metrics(n_pts, max_sq, p95_sq, sum_dist, lattice=4.0):
             "hausdorff_distance_95": np.where(valid, hd95, nan),
             "assd": np.where(valid, assd, nan),
             "contour_valid": valid}
+
+
+SURFACE_DICE_MAX_TOL = 4         # OCTM_SURFACE_DICE_MAX_TOL: tolerances per call
+SURFACE_DICE_MAX_TAU = 8.0       # pixels; T(8) = OCTM_SURFACE_DICE_MAX_SQ = 256
+
+
+def surface_dice_threshold(tau):
+    """Integer threshold of tolerance ``tau`` (pixels): the largest squared doubled-lattice distance D with
+    ``sqrt(D / 4.0) <= tau``, tested with the expression every contour distance of the suite is reported through, so
+    that "within tau" means what a user computes from those distances, boundary cases included."""
+    t = float(tau)
+    d = int(np.floor(4.0 * t * t))
+    while d > 0 and not np.sqrt(d / 4.0) <= t:
+        d -= 1
+    while np.sqrt((d + 1) / 4.0) <= t:
+        d += 1
+    return d
+
+
+def surface_dice_tolerances(tolerances):
+    """A tolerance or a sequence of 1 to 4 of them -> tuple of floats; ValueError outside ``0 <= tau <= 8`` (NaN
+    included) or for an empty or longer list."""
+    taus = (tolerances,) if np.ndim(tolerances) == 0 else tuple(tolerances)
+    if not 1 <= len(taus) <= SURFACE_DICE_MAX_TOL:
+        raise ValueError(f"surface_dice takes 1 to {SURFACE_DICE_MAX_TOL} tolerances, got {len(taus)}")
+    out = []
+    for t in taus:
+        try:
+            v = float(t)
+        except (TypeError, ValueError):
+            raise ValueError(f"surface_dice tolerance {t!r} is not a number") from None
+        if not 0.0 <= v <= SURFACE_DICE_MAX_TAU:          # False for NaN
+            raise ValueError(f"surface_dice tolerance {v} outside [0, {SURFACE_DICE_MAX_TAU}] pixels")
+        out.append(v)
+    return tuple(out)
+
+
+def surface_dice(n_surf, n_within):
+    """Normalized surface Dice per tolerance from the exact counts of ``octm_surface_dice_u8``: ``n_surf [..., 2]``
+    (|V_t|, |V_p|) and ``n_within [..., 2, T]`` -> float64 ``[..., T]`` = (n_within[..., 0, :] + n_within[..., 1, :]) /
+    (|V_t| + |V_p|).  NaN when both boundaries are empty (class absent from or filling both maps), 0 when exactly one
+    is (as MONAI)."""
+    ns = np.asarray(n_surf).astype(np.int64)
+    nw = np.asarray(n_within).astype(np.int64)
+    tot = (ns[..., 0] + ns[..., 1])[..., None]
+    num = (nw[..., 0, :] + nw[..., 1, :]).astype(np.float64)
+    with np.errstate(divide="ignore", invalid="ignore"):
+        return np.where(tot > 0, num / np.maximum(tot, 1), np.nan)

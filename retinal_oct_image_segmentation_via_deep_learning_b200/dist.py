@@ -187,6 +187,26 @@ def dataset_totals_async(res, world, group=None, want_max=False):
     return PendingTotals(res, world, group, want_max, local, reduced)
 
 
+def surface_dice_totals(res, world, device=None, group=None):
+    """Dataset-level normalized surface Dice over all ranks' shards from one ``evaluate(surface_dice=...)`` result per
+    rank: per class and tolerance, ``surface_dice_mean`` = mean over the items where NSD is defined (as
+    ``hausdorff_distance_mean``) and ``surface_dice_items`` = their exact count, both ``[K, T]``.  One float64 SUM
+    all-reduce of its own small vector; the totals vector of ``dataset_totals`` is not touched."""
+    taus = res.surface_dice_tolerances
+    if taus is None:
+        raise ValueError("the result has no surface Dice counts: evaluate with surface_dice=...")
+    ints = res.integers()
+    nsd = derive.surface_dice(ints["surface_dice_n_surf"], ints["surface_dice_n_within"])      # [N, K, T]
+    defined = ~np.isnan(nsd)
+    vec = np.concatenate([defined.sum(0).reshape(-1).astype(np.float64), np.where(defined, nsd, 0.0).sum(0).reshape(-1)])
+    vec = all_reduce_sum(vec, world, device=device, group=group)
+    k, t = nsd.shape[1:]
+    items = np.rint(vec[:k * t]).astype(np.int64).reshape(k, t)
+    with np.errstate(invalid="ignore", divide="ignore"):
+        mean = vec[k * t:].reshape(k, t) / items
+    return {"surface_dice_mean": mean, "surface_dice_items": items, "tolerances": tuple(taus)}
+
+
 def surface_distance_3d_sharded(vol_true, vol_pred, num_classes, rank, world, group=None):
     """BASELINE config 5 on several GPUs: the volume pair is replicated (it is small), the ``2 * K``
     independent (class, direction) distance transforms are split into contiguous unit ranges per rank,

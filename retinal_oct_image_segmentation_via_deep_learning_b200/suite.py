@@ -433,6 +433,44 @@ def derive_on_device(lp, ct, n, timers=None):
 
 
 @dataclass
+class SurfaceDiceOut:
+    """Exact counts of the surface Dice pass (device tensors, uint32 stored as int32 bits)."""
+    n_surf: torch.Tensor       # [N, K, 2]      (|V_t|, |V_p|): all-contour vertices of y_true / y_pred
+    n_within: torch.Tensor     # [N, K, 2, T]   vertices within tolerance j of the other boundary; direction 0: pred -> true
+    tolerances: tuple          # T tolerances in pixels, in the caller's order
+
+
+def surface_dice(y_true, y_pred, num_classes, tolerances=(1.0,), *, timers=None):
+    """Normalized surface Dice counts of every class at 1 to 4 tolerances ``0 <= tau <= 8`` pixels (build-defined,
+    no reference counterpart; MONAI ``compute_surface_dice``, surface-distance ``compute_surface_dice_at_tolerance``).
+
+    The surfaces are the whole boundaries, the all-contour vertex sets of ``contour_pass(mode="all")``; a vertex counts
+    as within ``tau`` when the nearest vertex of the other map lies at ``sqrt(D2 / 4.0) <= tau``, the expression every
+    contour distance of the suite is reported through.  One read of each label map (``octm_surface_dice_u8``).
+    Tolerances may come in any order; the counts come back in that order.  ``derive.surface_dice`` turns them into
+    float64 NSD values."""
+    taus = derive.surface_dice_tolerances(tolerances)
+    thr = [derive.surface_dice_threshold(t) for t in taus]
+    order = sorted(range(len(taus)), key=lambda j: thr[j])
+    yt, yp = _check_pair(y_true, y_pred)
+    n, h, w = yt.shape
+    k = int(num_classes)
+    dev = yt.device
+    n_surf = torch.empty((n, k, 2), dtype=torch.int32, device=dev)
+    n_within = torch.empty((n, k, 2, len(taus)), dtype=torch.int32, device=dev)
+    sorted_thr = (ctypes.c_uint32 * len(taus))(*[thr[j] for j in order])
+    with torch.cuda.device(dev), _Timed(timers, "surface_dice"):
+        _lib.call("octm_surface_dice_u8", _ptr(yt), _ptr(yp), n, h, w, k, sorted_thr, len(taus), _ptr(n_surf),
+                  _ptr(n_within), _stream())
+    if order != sorted(order):
+        n_within = n_within[..., [order.index(j) for j in range(len(taus))]]
+    return SurfaceDiceOut(n_surf, n_within, taus)
+
+
+_surface_dice_pass = surface_dice      # evaluate()'s keyword argument of the same name shadows it there
+
+
+@dataclass
 class SuiteResult:
     """Everything one evaluation produced, still on the device.
 
@@ -451,6 +489,12 @@ class SuiteResult:
     _host: dict | None = field(default=None, repr=False)
     _totals_host: np.ndarray | None = field(default=None, repr=False)
     contour_mode: str | None = "first"     # "first" / "all" (contour_pass modes), None without contour metrics
+    surface: SurfaceDiceOut | None = None  # evaluate(surface_dice=...) only
+
+    @property
+    def surface_dice_tolerances(self):
+        """The tolerances (pixels) of ``metrics()["surface_dice"]``, or None when it was not requested."""
+        return None if self.surface is None else self.surface.tolerances
 
     def settle_overflow(self, vec):
         """Redo (with a larger vertex bound) this batch's items whose contour overflowed ``max_pts`` and
@@ -507,6 +551,9 @@ class SuiteResult:
             d["contour_max_sq"] = ct.max_sq.cpu().numpy().view(np.uint32)
             d["contour_p95_sq"] = ct.p95_sq.cpu().numpy().view(np.uint32)
             d["contour_sum_dist"] = ct.sum_dist.cpu().numpy()
+        if self.surface is not None:
+            d["surface_dice_n_surf"] = self.surface.n_surf.cpu().numpy().view(np.uint32)
+            d["surface_dice_n_within"] = self.surface.n_within.cpu().numpy().view(np.uint32)
         return d
 
     def metrics(self):
@@ -526,6 +573,9 @@ class SuiteResult:
             if self.boundary_metrics is not None:
                 b = self.boundary_metrics.cpu().numpy()
                 m.update({name: b[:, :, i] for i, name in enumerate(_lib.BOUNDARY_METRICS)})
+            if self.surface is not None:        # a ratio of exact counts, evaluated on the host
+                m["surface_dice"] = derive.surface_dice(self.surface.n_surf.cpu().numpy().view(np.uint32),
+                                                        self.surface.n_within.cpu().numpy().view(np.uint32))
             self._host = m
         return self._host
 
@@ -542,6 +592,8 @@ class SuiteResult:
         if "contour_n_pts" in ints:
             m.update(derive.contour_metrics(ints["contour_n_pts"], ints["contour_max_sq"],
                                             ints["contour_p95_sq"], ints["contour_sum_dist"]))
+        if "surface_dice_n_surf" in ints:
+            m["surface_dice"] = derive.surface_dice(ints["surface_dice_n_surf"], ints["surface_dice_n_within"])
         return m
 
 
@@ -554,12 +606,17 @@ def _contour_mode(contours):
 
 
 def evaluate(y_true, y_pred, num_classes, *, contours=True, boundaries=False, max_pts=None, timers=None,
-             validate=True):
+             validate=True, surface_dice=None):
     """The full suite on a batch of label maps: fused label pass, contour kernels, float64 epilogue.
 
     ``contours``: ``True`` / ``"first"`` = hausdorff / hd95 / assd on contour ``[0]`` of each class mask, as the
     reference computes them; ``"all"`` = on every contour of each class (the whole boundary, see ``contour_pass``);
     ``False`` = no contour metrics.
+
+    ``surface_dice``: ``None`` (default, nothing extra runs) or a tolerance or 1 to 4 tolerances in pixels
+    (``0 <= tau <= 8``): adds ``metrics()["surface_dice"]``, float64 ``[N, K, T]``, the normalized surface Dice of the
+    whole boundary of each class at each tolerance (see ``surface_dice``; independent of ``contours``), the counts
+    ``integers()["surface_dice_n_surf"]`` / ``["surface_dice_n_within"]`` and ``surface_dice_tolerances``.
 
     Everything is launched asynchronously on the current stream; nothing is read back until
     ``totals_host()`` / ``metrics()`` / ``integers()`` is called on the result.
@@ -568,11 +625,13 @@ def evaluate(y_true, y_pred, num_classes, *, contours=True, boundaries=False, ma
     the results are read.  The check costs nothing extra: the label pass never aliases such a pixel into another
     class but drops it, so the item's confusion counts do not add up to H * W, which the totals kernel counts."""
     mode = _contour_mode(contours)
+    taus = None if surface_dice is None else derive.surface_dice_tolerances(surface_dice)
     yt, yp = _check_pair(y_true, y_pred)
     first = mode == "first"
     # contour [0] is seeded by the label pass, and its boundary rows and certificate skip the walk on layered maps
     lp = label_pass(yt, yp, num_classes, counts=True, columns=True, seeds=first, boundaries=boundaries or first,
                     timers=timers, certify=first)
+    sd = None if taus is None else _surface_dice_pass(yt, yp, num_classes, taus, timers=timers)
     ct = None
     if mode is not None:
         ct = contour_pass(yt, yp, num_classes, lp.first_pos, max_pts=max_pts, timers=timers, check_overflow=False,
@@ -582,7 +641,7 @@ def evaluate(y_true, y_pred, num_classes, *, contours=True, boundaries=False, ma
             lp.bnd_true = lp.bnd_pred = None
     cls, bnd, tot = derive_on_device(lp, ct, yt.shape[0], timers)
     return SuiteResult(yt.shape[0], lp, ct, cls, bnd, tot, (yt, yp) if ct is not None else None,
-                       validate=bool(validate), contour_mode=mode)
+                       validate=bool(validate), contour_mode=mode, surface=sd)
 
 
 def _cat_results(parts):
@@ -602,7 +661,12 @@ def _cat_results(parts):
                         cts[0].max_pts, cts[0].mode)
     n = sum(p.num_items for p in parts)
     cls, bnd, tot = derive_on_device(lp, ct, n)            # per-item values again + totals of the whole batch
-    res = SuiteResult(n, lp, ct, cls, bnd, tot, validate=parts[0].validate, contour_mode=parts[0].contour_mode)
+    sd = None
+    if parts[0].surface is not None:
+        sds = [p.surface for p in parts]
+        sd = SurfaceDiceOut(cat(sds, "n_surf"), cat(sds, "n_within"), sds[0].tolerances)
+    res = SuiteResult(n, lp, ct, cls, bnd, tot, validate=parts[0].validate, contour_mode=parts[0].contour_mode,
+                      surface=sd)
     res._final = True
     return res
 
@@ -620,7 +684,7 @@ def _pinned(nbytes):
 
 
 def evaluate_host(y_true, y_pred, num_classes, *, contours=True, device=None, chunk_items=None,
-                  max_pts=None, pack=False, pack_threads=0, validate=True):
+                  max_pts=None, pack=False, pack_threads=0, validate=True, surface_dice=None):
     """The full suite on HOST label maps (numpy arrays or CPU torch tensors, ideally pinned).
 
     Items are streamed to the GPU in chunks through two staging buffers: the host->device copy of
@@ -718,7 +782,7 @@ def evaluate_host(y_true, y_pred, num_classes, *, contours=True, device=None, ch
             if use_pack:
                 expand(ci)
             parts.append(evaluate(bt[:e0 - s0], bp[:e0 - s0], num_classes, contours=contours, max_pts=max_pts,
-                                  validate=validate))
+                                  validate=validate, surface_dice=surface_dice))
             done = torch.cuda.Event()
             done.record(compute)
             freed[ci & 1] = done
