@@ -127,7 +127,7 @@ OCTM_API int octm_label_pass_u8(const uint8_t* y_true, const uint8_t* y_pred, in
  *                          bottom (0 = every A-scan of both maps crosses the classes in order).  For an item with
  *                          unsorted == 0 every class contour is a function of the boundary rows alone, which is what
  *                          lets octm_contour2d_metrics_u8 measure it without reading the label maps again.
- *                          Items taller than 504 rows are reported as unsorted (not certified). */
+ *                          Items taller than 500 rows are reported as unsorted (not certified). */
 OCTM_API int octm_label_pass_sorted_u8(const uint8_t* y_true, const uint8_t* y_pred, int64_t n_items, int H, int W,
                               int num_classes, uint64_t* counts, int64_t* thick_absdiff, int64_t* bnd_sq,
                               int64_t* bnd_abs, int32_t* bnd_true, int32_t* bnd_pred, uint32_t* first_pos,

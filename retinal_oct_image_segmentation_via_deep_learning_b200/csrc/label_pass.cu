@@ -17,7 +17,7 @@
 //   * column scan: labels of 4 pixels x 2 maps are interleaved into a PRMT selector; one PRMT against
 //     an 8-entry byte LUT (immediate) yields the flags of a PAIR of thresholds; flags accumulate in
 //     nibble counters (IMAD adds on the FMA pipe), flushed every 28 rows into byte counters, those every
-//     504 rows into uint16 column totals in shared memory.
+//     504 rows (126 four-row groups) into uint16 column totals in shared memory.
 //   * confusion matrix: joint code t*8+p per pixel.  A lane whose 16 pixel pairs share one code (the
 //     common case in segmentation maps) extends a run counted in a register; runs reach the lane's
 //     private uint16 histogram column when the code changes.  The rare mixed lanes are compacted
@@ -71,9 +71,12 @@ constexpr int kWarpHist = 64 * 32 * 2;             // u16 [code][lane]
 constexpr int kWarpQueue = kQueueCap * 16;         // uint4 entries
 constexpr int kWarpBars = 768;                     // the warp's S "stage full" mbarriers (64 B), flags (at +64), first-position
                                                    // table (128 B at +128), last rows of the lanes' mixed passes (512 B at +256)
-constexpr int kWarpBytesShort = kWarpHist + kWarpQueue;              // H <= 504: totals alias the histogram block
+constexpr int kWarpBytesShort = kWarpHist + kWarpQueue;              // H <= 500: totals alias the histogram block
 constexpr int kWarpBytesTall = kWarpHist + kWarpQueue + kWarpTotals;
-constexpr int kShortRows = 504;   // 18 byte flushes x 7 nibble flushes x 4 rows
+// The byte counters are flushed after every 18 x 7 four-row groups, the last of which may be partial: an item of more
+// than 500 rows (126 groups) is flushed before its epilogue, and the flush would land in the histogram block the
+// totals of shorter items alias (and leave nothing for the certificate's byte-counter check).
+constexpr int kShortRows = 500;
 
 // PRMT look-up words for threshold pair q (k1 = 2q+1, k2 = 2q+2); byte i describes label v0 + i.
 //   q <  2 : flags [v <  k1] | [v <  k2] << 4  -- non-zero only for labels 0-3
@@ -393,7 +396,7 @@ __device__ __forceinline__ void stage_rows(LaneState<NP>& ls, uint32_t at, uint3
 }
 
 // Shared memory of the fast kernel: a fixed CTA block (kOffWarp bytes), then one private block per warp:
-//   [ S full-barriers, padded to 128 B | histogram 4 KB | queue 1 KB | (H > 504: column totals 4 KB) | ring ]
+//   [ S full-barriers, padded to 128 B | histogram 4 KB | queue 1 KB | (H > 500: column totals 4 KB) | ring ]
 // The ring is PRIVATE to the warp: S stages x 2 maps x R rows x strip bytes, filled by 2-D TMA tile copies
 // (one box of R rows x 128 columns per map) that the warp issues for itself.  Warps of a CTA therefore
 // never wait for each other: each folds its strip's results into the zero-initialised outputs with global
@@ -473,7 +476,7 @@ label_pass_fast(const LabelPassParams prm, const __grid_constant__ CUtensorMap t
         ls.reset(COLS);
         if (CONF && lane == 0) *warp_bad = 0;
         if (SORT) {
-            if (lane == 0) *warp_unsorted = tall ? 3u : 0u;      // items taller than one byte-counter period: not certified
+            if (lane == 0) *warp_unsorted = tall ? 3u : 0u;      // items that flush their byte counters: not certified
             prev_rows[lane] = make_uint4(0, 0, 0, 0);
         }
         if (SEEDS) warp_first[lane] = OCTM_NO_SEED;
@@ -500,7 +503,7 @@ label_pass_fast(const LabelPassParams prm, const __grid_constant__ CUtensorMap t
 
         // ------------------------------------------------------------------ item epilogue
         // The histogram fold runs first and leaves its shared-memory block zeroed: for items of at most
-        // 504 rows (no mid-item byte flush) the column totals reuse that block.
+        // kShortRows rows (no byte flush before the epilogue) the column totals reuse that block.
         if (CONF) {
             // leftover queue entries, then fold the 32 private histogram columns
             if (ls.last_b != 0xffffffffu) hist_add(hist_lane, ls.last_b & 0x3fu, ls.run);      // the open run

@@ -48,7 +48,7 @@ def _check_one(yt, yp, k, cuda, certify):
     fp = out.first_pos.cpu().numpy().view(np.uint32)
     np.testing.assert_array_equal(fp[:, 0], _first_pos_oracle(yt, k))
     np.testing.assert_array_equal(fp[:, 1], _first_pos_oracle(yp, k))
-    if certify and yt.shape[1] <= 504:          # (the strip kernel reports taller items unsorted without looking)
+    if certify and yt.shape[1] <= 500:          # (the strip kernel reports taller items unsorted without looking)
         want = ((np.diff(yt.astype(np.int16), axis=1) < 0).any(axis=(1, 2)).astype(np.uint32)
                 | ((np.diff(yp.astype(np.int16), axis=1) < 0).any(axis=(1, 2)).astype(np.uint32) << 1))
         np.testing.assert_array_equal(out.unsorted.cpu().numpy().view(np.uint32), want)

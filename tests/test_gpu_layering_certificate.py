@@ -9,14 +9,14 @@ from retinal_oct_image_segmentation_via_deep_learning_b200 import synth
 pytestmark = pytest.mark.gpu
 
 
-def _expected(yt, yp, tall_limit=504, fast=True):
+def _expected(yt, yp, tall_limit=500, fast=True):
     out = np.zeros(len(yt), np.uint32)
     for i in range(len(yt)):
         for m, a in enumerate((yt[i], yp[i])):
             if (np.diff(a.astype(np.int16), axis=0) < 0).any():
                 out[i] |= 1 << m
     if fast and yt.shape[1] > tall_limit:
-        out[:] = 3                                  # the strip kernel does not certify items taller than 504 rows
+        out[:] = 3                                  # the strip kernel does not certify items taller than 500 rows
     return out
 
 
@@ -54,7 +54,7 @@ def test_certificate_matches_numpy(cuda, shape, k):
         yt[5, rows, rng.integers(0, w, size=8)] = rng.integers(0, k, size=8)         # sparse salt in y_true only
     got, fast = _run(yt, yp, k, cuda)
     np.testing.assert_array_equal(got, _expected(yt, yp, fast=fast))
-    assert got[0] == (3 if (fast and h > 504) else 0)
+    assert got[0] == (3 if (fast and h > 500) else 0)
 
 
 def test_interleaving_defects(cuda):
