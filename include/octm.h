@@ -269,6 +269,17 @@ OCTM_API int octm_surface_dice_u8(const uint8_t* y_true, const uint8_t* y_pred, 
                                   uint32_t* n_within /* [n][K][2][n_thresholds] */, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * Connected components per class (build-defined, no reference counterpart; scipy.ndimage.label, skimage.measure.label).
+ * Per (item i, class c, map m: 0 = y_true, 1 = y_pred; o the other map), connectivity 4 or 8:
+ *   n_comp  uint32 [n][K][2]   number of connected components of (L_m == c)
+ *   n_hit   uint32 [n][K][2]   how many of them share at least one pixel with (L_o == c): detected (m = 0), matched (m = 1)
+ * Labels >= num_classes belong to no class and are never counted.  Counts are exact with no upper bound (no workspace,
+ * no overflow, no host synchronisation); each (item, map) is one row-streaming union-find over runs of equal labels. */
+OCTM_API int octm_components_u8(const uint8_t* y_true, const uint8_t* y_pred, int64_t n_items, int H, int W,
+                                int num_classes, int connectivity /* 4 or 8 */,
+                                uint32_t* n_comp /* [n][K][2] */, uint32_t* n_hit /* [n][K][2] */, void* stream);
+
+/* ---------------------------------------------------------------------------------------------
  * Boundary rows -> label maps (SURVEY.md 8f-4: the layer datasets catalogued in the reference's
  * Datasets.md:3-26 annotate boundary curves, while Metrics/*.py score masks).  The inverse of the label
  * pass's boundary rows on layered maps:

@@ -18,7 +18,7 @@ import os as _os
 METRICS_DIR = _os.path.join(_os.path.dirname(_os.path.abspath(__file__)), "Metrics")
 
 _LAZY = {"evaluate", "label_pass", "contour_pass", "confusion", "boundary_error", "validate_labels", "SuiteResult",
-         "surface_dice"}
+         "surface_dice", "components"}
 
 
 def __getattr__(name):          # keep `import package.synth` free of torch / the CUDA library

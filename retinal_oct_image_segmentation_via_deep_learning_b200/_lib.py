@@ -51,6 +51,7 @@ SIGNATURES = {
     "octm_contour2d_all_vertices_u8": (_INT, [_P, _P, _I64, _INT, _INT, _INT, _INT, _P, _P, _P, _P]),
     "octm_contour2d_all_u8": (_INT, [_P, _P, _I64, _INT, _INT, _INT, _INT, _P, _P, _P, _P, _P, _P, _c.c_size_t, _P]),
     "octm_surface_dice_u8": (_INT, [_P, _P, _I64, _INT, _INT, _INT, _P, _INT, _P, _P, _P]),
+    "octm_components_u8": (_INT, [_P, _P, _I64, _INT, _INT, _INT, _INT, _P, _P, _P]),
     "octm_argmax_labels": (_INT, [_P, _INT, _I64, _INT, _I64, _INT, _P, _P]),
     "octm_auc_workspace_bytes": (_c.c_size_t, [_I64, _I64, _INT]),
     "octm_auc_u8": (_INT, [_P, _P, _INT, _I64, _I64, _c.c_double, _P, _P, _c.c_size_t, _P]),

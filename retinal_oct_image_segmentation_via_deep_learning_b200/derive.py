@@ -154,3 +154,31 @@ def surface_dice(n_surf, n_within):
     num = (nw[..., 0, :] + nw[..., 1, :]).astype(np.float64)
     with np.errstate(divide="ignore", invalid="ignore"):
         return np.where(tot > 0, num / np.maximum(tot, 1), np.nan)
+
+
+COMPONENT_METRICS = ("component_count_error", "component_recall", "component_precision", "component_f1")
+
+
+def component_metrics(n_comp, n_hit):
+    """Lesion-wise detection scores from the exact counts of ``octm_components_u8``: ``n_comp [..., 2]`` (components of
+    y_true, y_pred) and ``n_hit [..., 2]`` (of those, the ones that share a pixel with the other map's class) -> float64
+    ``[...]`` arrays keyed by ``COMPONENT_METRICS``:
+
+    - ``component_count_error`` = |n_t - n_p|;
+    - ``component_recall`` = hit_t / n_t, NaN when n_t == 0;
+    - ``component_precision`` = hit_p / n_p, NaN when n_p == 0;
+    - ``component_f1`` = 2 P R / (P + R): NaN when n_t == n_p == 0, 0 when exactly one of them is 0 or P + R == 0.
+    """
+    nc = np.asarray(n_comp).astype(np.int64)
+    nh = np.asarray(n_hit).astype(np.int64)
+    nt, npred = nc[..., 0], nc[..., 1]
+    with np.errstate(divide="ignore", invalid="ignore"):
+        rec = np.where(nt > 0, nh[..., 0] / np.maximum(nt, 1), np.nan)
+        prec = np.where(npred > 0, nh[..., 1] / np.maximum(npred, 1), np.nan)
+        both = (nt > 0) & (npred > 0)
+        r0, p0 = np.where(both, rec, 0.0), np.where(both, prec, 0.0)
+        s = r0 + p0
+        f1 = np.where(s > 0, 2.0 * p0 * r0 / np.where(s > 0, s, 1.0), 0.0)
+    f1 = np.where((nt == 0) & (npred == 0), np.nan, f1)
+    return {"component_count_error": np.abs(nt - npred).astype(np.float64), "component_recall": rec,
+            "component_precision": prec, "component_f1": f1}

@@ -207,6 +207,32 @@ def surface_dice_totals(res, world, device=None, group=None):
     return {"surface_dice_mean": mean, "surface_dice_items": items, "tolerances": tuple(taus)}
 
 
+def component_totals(res, world, device=None, group=None):
+    """Dataset-level component scores over all ranks' shards from one ``evaluate(components=4 or 8)`` result per rank.
+    The counts of every item are summed (one float64 SUM all-reduce of its own small vector; each sum is exact below
+    2**53, and the totals vector of ``dataset_totals`` is not touched).  Per class: pooled (micro) ``component_recall``,
+    ``component_precision`` and ``component_f1`` by the rules of ``derive.component_metrics`` applied to the summed
+    counts, ``component_count_error`` = the mean of |n_t - n_p| over all items, and the summed integers
+    ``component_count`` / ``component_hits`` ``[K, 2]`` and ``items``."""
+    if res.component_connectivity is None:
+        raise ValueError("the result has no component counts: evaluate with components=4 or 8")
+    ints = res.integers()
+    nc = ints["component_count"].astype(np.int64)                 # [N, K, 2]
+    nh = ints["component_hits"].astype(np.int64)
+    err = np.abs(nc[..., 0] - nc[..., 1]).sum(0)
+    vec = np.concatenate([nc.sum(0).reshape(-1), nh.sum(0).reshape(-1), err, [nc.shape[0]]]).astype(np.float64)
+    vec = all_reduce_sum(vec, world, device=device, group=group)
+    k = nc.shape[1]
+    tot = np.rint(vec).astype(np.int64)
+    count, hits = tot[:2 * k].reshape(k, 2), tot[2 * k:4 * k].reshape(k, 2)
+    items = int(tot[-1])
+    out = derive.component_metrics(count, hits)
+    with np.errstate(invalid="ignore", divide="ignore"):
+        out["component_count_error"] = tot[4 * k:5 * k] / np.float64(items) if items else np.full(k, np.nan)
+    out.update(component_count=count, component_hits=hits, items=items, connectivity=res.component_connectivity)
+    return out
+
+
 def surface_distance_3d_sharded(vol_true, vol_pred, num_classes, rank, world, group=None):
     """BASELINE config 5 on several GPUs: the volume pair is replicated (it is small), the ``2 * K``
     independent (class, direction) distance transforms are split into contiguous unit ranges per rank,

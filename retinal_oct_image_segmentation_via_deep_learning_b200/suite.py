@@ -471,6 +471,44 @@ _surface_dice_pass = surface_dice      # evaluate()'s keyword argument of the sa
 
 
 @dataclass
+class ComponentsOut:
+    """Exact counts of the connected-component pass (device tensors, uint32 stored as int32 bits)."""
+    n_comp: torch.Tensor       # [N, K, 2]   components of (y_true == c), (y_pred == c)
+    n_hit: torch.Tensor        # [N, K, 2]   of those, the ones sharing a pixel with the other map's class c
+    connectivity: int          # 4 or 8
+
+
+def _connectivity(connectivity):
+    if connectivity is True or connectivity is False or connectivity not in (4, 8):
+        raise ValueError(f"components must be None, 4 or 8, got {connectivity!r}")
+    return int(connectivity)
+
+
+def components(y_true, y_pred, num_classes, connectivity=4, *, timers=None):
+    """Connected components of every class of both maps (build-defined, no reference counterpart;
+    ``scipy.ndimage.label`` at connectivity 4, ``skimage.measure.label``'s default at 8).
+
+    ``n_comp[i, c, m]`` counts the components of ``(L_m == c)`` (m = 0: y_true, 1: y_pred) and ``n_hit[i, c, m]`` those
+    of them that share at least one pixel with ``(L_o == c)`` of the other map: detected true lesions (m = 0) and
+    matched predicted ones (m = 1).  Labels >= num_classes are never counted.  One row-streaming union-find per
+    (item, map) (``octm_components_u8``), launched asynchronously on the current stream; ``derive.component_metrics``
+    turns the counts into float64 scores."""
+    conn = _connectivity(connectivity)
+    yt, yp = _check_pair(y_true, y_pred)
+    n, h, w = yt.shape
+    k = int(num_classes)
+    dev = yt.device
+    n_comp = torch.empty((n, k, 2), dtype=torch.int32, device=dev)
+    n_hit = torch.empty((n, k, 2), dtype=torch.int32, device=dev)
+    with torch.cuda.device(dev), _Timed(timers, "components"):
+        _lib.call("octm_components_u8", _ptr(yt), _ptr(yp), n, h, w, k, conn, _ptr(n_comp), _ptr(n_hit), _stream())
+    return ComponentsOut(n_comp, n_hit, conn)
+
+
+_components_pass = components          # evaluate()'s keyword argument of the same name shadows it there
+
+
+@dataclass
 class SuiteResult:
     """Everything one evaluation produced, still on the device.
 
@@ -490,11 +528,17 @@ class SuiteResult:
     _totals_host: np.ndarray | None = field(default=None, repr=False)
     contour_mode: str | None = "first"     # "first" / "all" (contour_pass modes), None without contour metrics
     surface: SurfaceDiceOut | None = None  # evaluate(surface_dice=...) only
+    components: ComponentsOut | None = None  # evaluate(components=...) only
 
     @property
     def surface_dice_tolerances(self):
         """The tolerances (pixels) of ``metrics()["surface_dice"]``, or None when it was not requested."""
         return None if self.surface is None else self.surface.tolerances
+
+    @property
+    def component_connectivity(self):
+        """The connectivity (4 or 8) of the component metrics, or None when they were not requested."""
+        return None if self.components is None else self.components.connectivity
 
     def settle_overflow(self, vec):
         """Redo (with a larger vertex bound) this batch's items whose contour overflowed ``max_pts`` and
@@ -554,6 +598,9 @@ class SuiteResult:
         if self.surface is not None:
             d["surface_dice_n_surf"] = self.surface.n_surf.cpu().numpy().view(np.uint32)
             d["surface_dice_n_within"] = self.surface.n_within.cpu().numpy().view(np.uint32)
+        if self.components is not None:
+            d["component_count"] = self.components.n_comp.cpu().numpy().view(np.uint32)
+            d["component_hits"] = self.components.n_hit.cpu().numpy().view(np.uint32)
         return d
 
     def metrics(self):
@@ -576,6 +623,9 @@ class SuiteResult:
             if self.surface is not None:        # a ratio of exact counts, evaluated on the host
                 m["surface_dice"] = derive.surface_dice(self.surface.n_surf.cpu().numpy().view(np.uint32),
                                                         self.surface.n_within.cpu().numpy().view(np.uint32))
+            if self.components is not None:     # ratios of exact counts, evaluated on the host
+                m.update(derive.component_metrics(self.components.n_comp.cpu().numpy().view(np.uint32),
+                                                  self.components.n_hit.cpu().numpy().view(np.uint32)))
             self._host = m
         return self._host
 
@@ -594,6 +644,8 @@ class SuiteResult:
                                             ints["contour_p95_sq"], ints["contour_sum_dist"]))
         if "surface_dice_n_surf" in ints:
             m["surface_dice"] = derive.surface_dice(ints["surface_dice_n_surf"], ints["surface_dice_n_within"])
+        if "component_count" in ints:
+            m.update(derive.component_metrics(ints["component_count"], ints["component_hits"]))
         return m
 
 
@@ -606,7 +658,7 @@ def _contour_mode(contours):
 
 
 def evaluate(y_true, y_pred, num_classes, *, contours=True, boundaries=False, max_pts=None, timers=None,
-             validate=True, surface_dice=None):
+             validate=True, surface_dice=None, components=None):
     """The full suite on a batch of label maps: fused label pass, contour kernels, float64 epilogue.
 
     ``contours``: ``True`` / ``"first"`` = hausdorff / hd95 / assd on contour ``[0]`` of each class mask, as the
@@ -618,6 +670,12 @@ def evaluate(y_true, y_pred, num_classes, *, contours=True, boundaries=False, ma
     whole boundary of each class at each tolerance (see ``surface_dice``; independent of ``contours``), the counts
     ``integers()["surface_dice_n_surf"]`` / ``["surface_dice_n_within"]`` and ``surface_dice_tolerances``.
 
+    ``components``: ``None`` (default, nothing extra runs) or the connectivity 4 or 8: adds the float64 ``[N, K]``
+    ``metrics()`` ``component_count_error``, ``component_recall``, ``component_precision`` and ``component_f1`` of the
+    connected components of each class (see ``components`` and ``derive.component_metrics``; independent of
+    ``contours`` and ``surface_dice``), the counts ``integers()["component_count"]`` / ``["component_hits"]``
+    (uint32 ``[N, K, 2]``) and ``component_connectivity``.
+
     Everything is launched asynchronously on the current stream; nothing is read back until
     ``totals_host()`` / ``metrics()`` / ``integers()`` is called on the result.
     ``timers``: optional dict filled with (start, end) CUDA-event pairs per kernel family.
@@ -626,12 +684,14 @@ def evaluate(y_true, y_pred, num_classes, *, contours=True, boundaries=False, ma
     class but drops it, so the item's confusion counts do not add up to H * W, which the totals kernel counts."""
     mode = _contour_mode(contours)
     taus = None if surface_dice is None else derive.surface_dice_tolerances(surface_dice)
+    conn = None if components is None else _connectivity(components)
     yt, yp = _check_pair(y_true, y_pred)
     first = mode == "first"
     # contour [0] is seeded by the label pass, and its boundary rows and certificate skip the walk on layered maps
     lp = label_pass(yt, yp, num_classes, counts=True, columns=True, seeds=first, boundaries=boundaries or first,
                     timers=timers, certify=first)
     sd = None if taus is None else _surface_dice_pass(yt, yp, num_classes, taus, timers=timers)
+    cc = None if conn is None else _components_pass(yt, yp, num_classes, conn, timers=timers)
     ct = None
     if mode is not None:
         ct = contour_pass(yt, yp, num_classes, lp.first_pos, max_pts=max_pts, timers=timers, check_overflow=False,
@@ -641,7 +701,7 @@ def evaluate(y_true, y_pred, num_classes, *, contours=True, boundaries=False, ma
             lp.bnd_true = lp.bnd_pred = None
     cls, bnd, tot = derive_on_device(lp, ct, yt.shape[0], timers)
     return SuiteResult(yt.shape[0], lp, ct, cls, bnd, tot, (yt, yp) if ct is not None else None,
-                       validate=bool(validate), contour_mode=mode, surface=sd)
+                       validate=bool(validate), contour_mode=mode, surface=sd, components=cc)
 
 
 def _cat_results(parts):
@@ -665,8 +725,12 @@ def _cat_results(parts):
     if parts[0].surface is not None:
         sds = [p.surface for p in parts]
         sd = SurfaceDiceOut(cat(sds, "n_surf"), cat(sds, "n_within"), sds[0].tolerances)
+    cc = None
+    if parts[0].components is not None:
+        ccs = [p.components for p in parts]
+        cc = ComponentsOut(cat(ccs, "n_comp"), cat(ccs, "n_hit"), ccs[0].connectivity)
     res = SuiteResult(n, lp, ct, cls, bnd, tot, validate=parts[0].validate, contour_mode=parts[0].contour_mode,
-                      surface=sd)
+                      surface=sd, components=cc)
     res._final = True
     return res
 
@@ -684,7 +748,7 @@ def _pinned(nbytes):
 
 
 def evaluate_host(y_true, y_pred, num_classes, *, contours=True, device=None, chunk_items=None,
-                  max_pts=None, pack=False, pack_threads=0, validate=True, surface_dice=None):
+                  max_pts=None, pack=False, pack_threads=0, validate=True, surface_dice=None, components=None):
     """The full suite on HOST label maps (numpy arrays or CPU torch tensors, ideally pinned).
 
     Items are streamed to the GPU in chunks through two staging buffers: the host->device copy of
@@ -782,7 +846,7 @@ def evaluate_host(y_true, y_pred, num_classes, *, contours=True, device=None, ch
             if use_pack:
                 expand(ci)
             parts.append(evaluate(bt[:e0 - s0], bp[:e0 - s0], num_classes, contours=contours, max_pts=max_pts,
-                                  validate=validate, surface_dice=surface_dice))
+                                  validate=validate, surface_dice=surface_dice, components=components))
             done = torch.cuda.Event()
             done.record(compute)
             freed[ci & 1] = done
