@@ -125,7 +125,8 @@ __global__ void __launch_bounds__(128) edt3_pass1_vec_kernel(const Edt3Params pr
 #pragma unroll
             for (int i = 0; i < 16; ++i) {
                 const uint32_t v = byte_of(cur, i);
-                const uint32_t nx = i < 15 ? byte_of(cur, i + 1) : (nxt.x & 0xffu);
+                // past the end of the line: a value no class takes (the padding byte 0xff is class 255)
+                const uint32_t nx = i < 15 ? byte_of(cur, i + 1) : (k + 1 < groups ? (nxt.x & 0xffu) : 0xffffffffu);
                 bool surf = false;
                 if (v == cls)
                     surf = border || prev != cls || nx != cls || byte_of(u, i) != cls || byte_of(d, i) != cls ||
