@@ -141,8 +141,10 @@ OCTM_API int octm_label_pass_path(int H, int W, int num_classes, const void* y_t
 /* What the suite's kernels assume about the stream of label maps -- a speed heuristic, never a difference in results:
  * 0 = follow the data (default: every certified label pass reports how many maps its certificate rejected; the next calls
  * assume a noisy stream once that was more than a fifth), 1 = assume clean (seeds from the column totals + a rescan of
- * rejected maps; contour stage: boundary-row pass first), 2 = assume noisy (seeds tracked per pixel; contour stage: the
- * rejected maps' contours are verified against the label pixels first so that the fast pass can measure them).
+ * rejected maps; confusion matrices from the boundary rows + a per-pixel histogram of the rejected items, when the call
+ * asks for the boundary rows; contour stage: boundary-row pass first), 2 = assume noisy (seeds tracked per pixel and the
+ * confusion histogram taken in the label pass; contour stage: the rejected maps' contours are verified against the label
+ * pixels first so that the fast pass can measure them).
  * Returns the previous policy (any other argument: just reports it). */
 OCTM_API int octm_label_pass_seed_policy(int policy);
 

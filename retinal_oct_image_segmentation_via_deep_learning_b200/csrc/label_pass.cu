@@ -24,6 +24,8 @@
 //     (ballot + popc) into a per-warp queue and drained 32 entries at a time, one entry per lane.
 //   * contour seeds: classes are tracked per warp; lanes that meet a new class record its first raster
 //     position with a shared-memory atomicMin.
+//   * without the histogram (CONF = 0, the suite's call on a mostly accepted stream) the confusion matrices come from the
+//     boundary rows afterwards (confusion_from_rows_kernel, confusion_fix_kernel for the items the certificate rejects).
 //   * per item and warp: column totals -> |thickness diff|, boundary error sums (REDUX warp sums), private
 //     histograms -> K x K counts; the strips of an item meet in the zero-initialised outputs through
 //     global reductions (a few dozen RED per warp and item), never at a CTA barrier.
@@ -43,6 +45,9 @@ constexpr int kStrip = 128;        // columns per consumer warp
 constexpr int kQueueCap = 64;      // queue entries (16 pixel pairs each) per warp
 constexpr uint32_t kPadWord = 0x08080808u;   // label 8: PRMT nibble 8 = "replicate sign of LUT byte 0" = 0x00
 constexpr uint32_t kSkipWord = 0xFFFFFFFFu;  // queue marker: this word holds no pixels
+// unsorted[item] bit 2, set by the label pass without the histogram when the item has a label >= K and cleared by
+// confusion_fix_kernel, which counts such items pixel by pixel; callers only ever see bits 0 and 1
+constexpr uint32_t kBadLabels = 4u;
 
 struct LabelPassParams {
     const uint8_t* yt;
@@ -221,6 +226,16 @@ __device__ __forceinline__ void record_first(uint32_t fresh, uint2 tA, uint2 pA,
     }
 }
 
+// some label among the 8 of one row of both maps (words t, p) is >= K; k_add = (128 - K) per byte
+template <int NP>
+__device__ __forceinline__ bool labels_from_k(uint2 t, uint2 p, uint32_t k_add) {
+    if (NP == 4) return ((t.x | t.y) | (p.x | p.y)) & 0xf8f8f8f8u;      // K = 8: a bit above the 3-bit class range
+    // bit 7 of a byte: the label is >= 128, or its low 7 bits plus 128 - K reach 128 (no carry leaves the byte)
+    const uint32_t m = (((t.x & 0x7f7f7f7fu) + k_add) | t.x) | (((t.y & 0x7f7f7f7fu) + k_add) | t.y) |
+                       (((p.x & 0x7f7f7f7fu) + k_add) | p.x) | (((p.y & 0x7f7f7f7fu) + k_add) | p.y);
+    return m & 0x80808080u;
+}
+
 __device__ __forceinline__ void hist_add(unsigned short* hist_lane, uint32_t code, uint32_t inc) {
     unsigned short* h = hist_lane + code * 32;
     *h = static_cast<unsigned short>(*h + inc);
@@ -276,7 +291,7 @@ struct LaneState {
 struct StageConsts {
     uint32_t srow2, srow4;        // 2 / 4 rows of a staged strip in shared memory (bytes)
     uint32_t W2, W4;              // 2 / 4 rows of the image (raster positions)
-    uint32_t map_bytes, one, all_classes;
+    uint32_t map_bytes, one, all_classes, k_add;
     int phase, lane;
     bool colv;
     unsigned short* hist_lane;
@@ -315,7 +330,7 @@ __device__ __forceinline__ void stage_rows(LaneState<NP>& ls, uint32_t at, uint3
             col_accumulate<NP>(ls.cs.nib[0], tA.x, pA.x, tB.x, pB.x, sc.one);
             col_accumulate<NP>(ls.cs.nib[1], tA.y, pA.y, tB.y, pB.y, sc.one);
         }
-        if (CONF || SEEDS) {
+        if (CONF || SEEDS || SORT) {
             uint4 j = make_uint4(tA.x * 8u + pA.x, tA.y * 8u + pA.y, tB.x * 8u + pB.x, tB.y * 8u + pB.y);
             const uint32_t b = prmt(j.x, 0, 0);
             // labels >= 8 (outside what the 6-bit joint code can hold) must never alias a valid code: OR of all 16
@@ -326,7 +341,7 @@ __device__ __forceinline__ void stage_rows(LaneState<NP>& ls, uint32_t at, uint3
             // uniform row pairs come in long runs of one joint code (a lane stays inside a layer for many rows): the
             // run length lives in a register and reaches the lane's private histogram column when the code changes
             const bool changed = uni && b != ls.last_b;
-            if (uni && !changed) ls.run += 16u;
+            if (CONF && uni && !changed) ls.run += 16u;
             const bool mixed_lane = FULL ? !uni : (va || vb);
             if (__any_sync(0xffffffffu, mixed_lane || changed)) {
                 if (SORT && (mixed_lane || changed)) {
@@ -357,6 +372,11 @@ __device__ __forceinline__ void stage_rows(LaneState<NP>& ls, uint32_t at, uint3
                 if (CONF && (FULL ? high != 0 : ((va && ((tA.x | tA.y | pA.x | pA.y) & 0xf8f8f8f8u)) ||
                                         (vb && ((tB.x | tB.y | pB.x | pB.y) & 0xf8f8f8f8u)))))
                     *sc.bad = 1;                    // this warp's counts of the item are withheld (epilogue)
+                // without the histogram the item's counts come from its boundary rows, which cannot see a label >= K:
+                // such an item is sent to the per-pixel histogram instead (a uniform lane's labels are checked when
+                // its run starts, so checking the lanes of this block covers every pixel)
+                if (!CONF && SORT && ((va && labels_from_k<NP>(tA, pA, sc.k_add)) || (vb && labels_from_k<NP>(tB, pB, sc.k_add))))
+                    atomicOr(sc.unsorted, kBadLabels);
                 if (changed) {
                     if (CONF && ls.last_b != 0xffffffffu) hist_add(sc.hist_lane, ls.last_b & 0x3fu, ls.run);
                     ls.last_b = b;
@@ -467,6 +487,7 @@ label_pass_fast(const LabelPassParams prm, const __grid_constant__ CUtensorMap t
     StageConsts sc;
     sc.srow2 = 2u * srow; sc.srow4 = 4u * srow; sc.W2 = 2u * W; sc.W4 = 4u * W;
     sc.map_bytes = map_bytes; sc.one = prm.one; sc.all_classes = ((1u << K) - 1u) * 0x101u;
+    sc.k_add = static_cast<uint32_t>(128 - K) * 0x01010101u;
     sc.phase = phase; sc.lane = lane; sc.colv = colv;
     sc.hist_lane = hist_lane; sc.queue = queue; sc.totals = totals; sc.first_tab = warp_first; sc.bad = warp_bad;
     sc.unsorted = warp_unsorted; sc.prev_rows = prev_rows;
@@ -1090,6 +1111,153 @@ __global__ void __launch_bounds__(256) first_pos_fix_kernel(const uint8_t* __res
     }
 }
 
+// Confusion matrices of the items whose two maps the certificate accepted, from their boundary rows b_k(x) = #{label < k}
+// alone.  In a column in class order the pixels of class < a form a prefix of length b_a, so
+//   C(a, b) = sum_x min(bt_a(x), bp_b(x)) = #{t < a, p < b}   (b_0 = 0, b_K = H)
+//   count(t = i, p = j) = C(i+1, j+1) - C(i, j+1) - C(i+1, j) + C(i, j).
+// A warp per item (persistent), a lane per 4 columns at a time (16-byte loads of the K-1 rows of each map); the 49 sums
+// C(a, b), a, b = 1..7, and the 2 x 7 row sums live in registers and meet in warp reductions.  Rows k >= K are taken as
+// b_k = H, which makes the K = 8 arithmetic serve every K.  Items with a rejected map or a label >= K (unsorted != 0) are
+// left to confusion_fix_kernel.
+constexpr int kRowsWarps = 8;
+__global__ void __launch_bounds__(kRowsWarps * 32) confusion_from_rows_kernel(const int* __restrict__ bnd_t, const int* __restrict__ bnd_p,
+                                                                              long long n_items, int H, int W, int K,
+                                                                              const uint32_t* __restrict__ unsorted,
+                                                                              unsigned long long* counts) {
+    const int lane = threadIdx.x & 31;
+    const long long stride = static_cast<long long>(gridDim.x) * kRowsWarps;
+    for (long long item = static_cast<long long>(blockIdx.x) * kRowsWarps + (threadIdx.x >> 5); item < n_items; item += stride) {
+        if (unsorted[item] != 0u) continue;                                   // warp-uniform
+        uint32_t C[7][7], St[7], Sp[7];
+#pragma unroll
+        for (int a = 0; a < 7; ++a) {
+            St[a] = Sp[a] = 0;
+#pragma unroll
+            for (int b = 0; b < 7; ++b) C[a][b] = 0;
+        }
+        const int4* rt = reinterpret_cast<const int4*>(bnd_t + item * (K - 1) * static_cast<long long>(W));
+        const int4* rp = reinterpret_cast<const int4*>(bnd_p + item * (K - 1) * static_cast<long long>(W));
+        const int W4 = W >> 2;
+        for (int q = lane; q < W4; q += 32) {
+            int4 t[7], p[7];
+#pragma unroll
+            for (int a = 0; a < 7; ++a) {
+                t[a] = a < K - 1 ? __ldg(rt + a * W4 + q) : make_int4(H, H, H, H);
+                p[a] = a < K - 1 ? __ldg(rp + a * W4 + q) : make_int4(H, H, H, H);
+            }
+#pragma unroll
+            for (int a = 0; a < 7; ++a) {
+                St[a] += static_cast<uint32_t>(t[a].x + t[a].y + t[a].z + t[a].w);
+                Sp[a] += static_cast<uint32_t>(p[a].x + p[a].y + p[a].z + p[a].w);
+#pragma unroll
+                for (int b = 0; b < 7; ++b)
+                    C[a][b] += static_cast<uint32_t>((min(t[a].x, p[b].x) + min(t[a].y, p[b].y)) +
+                                                     (min(t[a].z, p[b].z) + min(t[a].w, p[b].w)));
+            }
+        }
+#pragma unroll
+        for (int a = 0; a < 7; ++a) {
+            St[a] = __reduce_add_sync(0xffffffffu, St[a]);
+            Sp[a] = __reduce_add_sync(0xffffffffu, Sp[a]);
+#pragma unroll
+            for (int b = 0; b < 7; ++b) C[a][b] = __reduce_add_sync(0xffffffffu, C[a][b]);
+        }
+        // C(a, b) over a, b = 0..8 (index 8: b_8 = H; with K < 8 the rows from K on are H already)
+        const uint32_t HW = static_cast<uint32_t>(H) * static_cast<uint32_t>(W);
+        auto cab = [&](int a, int b) -> uint32_t {
+            if (a == 0 || b == 0) return 0u;
+            if (a == 8 && b == 8) return HW;
+            if (a == 8) return Sp[b - 1];
+            if (b == 8) return St[a - 1];
+            return C[a - 1][b - 1];
+        };
+        unsigned long long* out = counts + item * K * K;
+#pragma unroll
+        for (int i = 0; i < 8; ++i)
+#pragma unroll
+            for (int j = 0; j < 8; ++j) {
+                const uint32_t v = cab(i + 1, j + 1) - cab(i, j + 1) - cab(i + 1, j) + cab(i, j);
+                if (i < K && j < K && lane == ((i * 8 + j) & 31)) out[i * K + j] = v;
+            }
+    }
+}
+
+// Confusion matrices of the items confusion_from_rows_kernel leaves (a map the certificate rejected, or a label >= K):
+// the per-pixel histogram (K <= 8, W % 16 == 0, 16-byte aligned maps: the shapes of the strip kernel), with the strip
+// kernel's treatment of bad labels: a 128-column strip of the item that holds a label >= 8 contributes nothing (its warp
+// withholds its counts there), codes with a label in [K, 8) are dropped at the output.  Either way the item's counts fall
+// short of H * W.  One CTA per such item (grid-stride, one CTA-uniform skip per item as in first_pos_fix_kernel); a
+// thread takes every 256th 16-byte group of both maps, and a group of one joint code adds 16 at once.  Items with a label
+// >= K (the transient bit kBadLabels, cleared here) are read twice: once for the strips to leave out.
+__global__ void __launch_bounds__(256) confusion_fix_kernel(const uint8_t* __restrict__ yt, const uint8_t* __restrict__ yp,
+                                                            long long n_items, int H, int W, int K, uint32_t* unsorted,
+                                                            unsigned long long* counts) {
+    __shared__ uint32_t s_hist[8][64][16];      // u16 [warp][code t*8+p][lane]: at most H * W / 256 <= 2^15 per lane
+    __shared__ uint32_t s_sum[64];
+    __shared__ uint32_t s_bad_strips;           // bit s: strip s (columns 128 s ..) holds a label >= 8 (W <= 2048)
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    for (int i = tid; i < 8 * 64 * 16; i += 256) (&s_hist[0][0][0])[i] = 0;
+    __syncthreads();
+    unsigned short* hist_lane = reinterpret_cast<unsigned short*>(&s_hist[warp][0][0]) + lane;
+    const long long item_elems = static_cast<long long>(H) * W;
+    const int groups = static_cast<int>(item_elems >> 4), row_groups = W >> 4;     // H * W <= 2^23
+    for (long long item = blockIdx.x; item < n_items; item += gridDim.x) {
+        const uint32_t u = unsorted[item];
+        if (u == 0u) continue;                                                // CTA-uniform: counted from the rows
+        if (tid < 64) s_sum[tid] = 0;
+        if (tid == 0) s_bad_strips = 0;
+        const uint4* T = reinterpret_cast<const uint4*>(yt + item * item_elems);
+        const uint4* P = reinterpret_cast<const uint4*>(yp + item * item_elems);
+        __syncthreads();
+        uint32_t bad_strips = 0;
+        if (u & kBadLabels) {                                                 // CTA-uniform, rare
+            uint32_t mine = 0;
+            for (int g = tid; g < groups; g += 256) {
+                const uint4 a = __ldg(T + g), b = __ldg(P + g);
+                if ((((a.x | a.y) | (a.z | a.w)) | ((b.x | b.y) | (b.z | b.w))) & 0xf8f8f8f8u)
+                    mine |= 1u << ((g % row_groups) >> 3);
+            }
+            mine = __reduce_or_sync(0xffffffffu, mine);
+            if (lane == 0 && mine) atomicOr(&s_bad_strips, mine);
+            __syncthreads();
+            bad_strips = s_bad_strips;
+        }
+        for (int g = tid; g < groups; g += 256) {
+            if (bad_strips && ((bad_strips >> ((g % row_groups) >> 3)) & 1u)) continue;
+            const uint4 a = __ldg(T + g), b = __ldg(P + g);                   // labels < 8 from here on
+            const uint32_t j[4] = {a.x * 8u + b.x, a.y * 8u + b.y, a.z * 8u + b.z, a.w * 8u + b.w};
+            const uint32_t c = prmt(j[0], 0, 0);
+            if ((((j[0] ^ c) | (j[1] ^ c)) | ((j[2] ^ c) | (j[3] ^ c))) == 0u) {
+                hist_add(hist_lane, c & 0x3fu, 16);
+            } else {
+#pragma unroll
+                for (int k = 0; k < 4; ++k)
+#pragma unroll
+                    for (int i = 0; i < 4; ++i) hist_add(hist_lane, (j[k] >> (8 * i)) & 0x3fu, 1);
+            }
+        }
+        __syncthreads();
+        {
+            // code c = tid % 64 over the lanes of warps 2 q and 2 q + 1, q = tid / 64; the rotation spreads the banks
+            const int c = tid & 63, q = tid >> 6;
+            uint32_t sum = 0;
+#pragma unroll
+            for (int w = 0; w < 2; ++w)
+#pragma unroll
+                for (int i = 0; i < 16; ++i) {
+                    uint32_t& h = s_hist[2 * q + w][c][(c + i) & 15];
+                    sum += (h & 0xffffu) + (h >> 16);
+                    h = 0;
+                }
+            atomicAdd(&s_sum[c], sum);
+        }
+        __syncthreads();
+        for (int i = tid; i < K * K; i += 256) counts[item * K * K + i] = s_sum[(i / K) * 8 + i % K];
+        if (tid == 0) unsorted[item] = u & 3u;
+        __syncthreads();
+    }
+}
+
 // K3: sums over columns of (bt - bp)^2 and |bt - bp| for int32 boundary arrays [n][Kb][W].
 __global__ void __launch_bounds__(256) boundary_error_kernel(const int* __restrict__ bt, const int* __restrict__ bp,
                                                              long long n_rows, int W, long long* sum_sq,
@@ -1269,8 +1437,12 @@ static int launch_generic(const LabelPassParams& p, cudaStream_t stream) {
 // leaves "maps rejected / maps seen" in a host-mapped word (one tiny kernel, no synchronisation: the next call reads
 // whatever has arrived), and a call tracks per pixel when more than a fifth of the maps of the last report were
 // rejected.  Both ways give the same seeds (tests run both); octm_label_pass_seed_policy pins one.
+// The confusion matrices follow the same choice.  On a mostly accepted stream the strip kernel runs without its per-pixel
+// histogram, and the counts come from the boundary rows (confusion_from_rows_kernel) plus a per-pixel histogram of just
+// the rejected items (confusion_fix_kernel).  On a mostly rejected stream that would read the labels twice, so the strip
+// kernel keeps its histogram.
 // The report: host_report(kReportSeeds), [0] rejected maps, [1] maps.
-static std::atomic<int> g_seed_policy{0};      // 0 follow the data, 1 column totals + rescan, 2 per pixel
+static std::atomic<int> g_seed_policy{0};      // 0 follow the data, 1 column totals + rescans, 2 per pixel
 
 __global__ void __launch_bounds__(1024) seed_feedback_kernel(const uint32_t* __restrict__ unsorted, long long n, uint32_t* out) {
     __shared__ uint32_t s_sum[32];
@@ -1288,8 +1460,6 @@ __global__ void __launch_bounds__(1024) seed_feedback_kernel(const uint32_t* __r
     }
 }
 
-bool stream_mostly_rejected();
-static bool seeds_per_pixel() { return stream_mostly_rejected(); }
 bool stream_mostly_rejected() {
     const int policy = g_seed_policy.load();
     if (policy != 0) return policy == 2;
@@ -1306,6 +1476,19 @@ static int report_rejected(const LabelPassParams& p, cudaStream_t stream) {
     return check_launch("seed_feedback_kernel");
 }
 
+// counts of a certified strip-kernel pass that ran without its histogram: accepted items from their boundary rows,
+// the others pixel by pixel (every item's K x K counts are written by exactly one of the two kernels)
+static int confusion_from_rows(const LabelPassParams& p, cudaStream_t stream) {
+    const long long rgrid = resident_grid((p.n_items + kRowsWarps - 1) / kRowsWarps, confusion_from_rows_kernel, kRowsWarps * 32, 0, 2);
+    OCTM_TIMED("confusion_from_rows_kernel", stream) confusion_from_rows_kernel<<<static_cast<unsigned>(rgrid), kRowsWarps * 32, 0, stream>>>(
+        p.bnd_t, p.bnd_p, p.n_items, p.H, p.W, p.K, p.unsorted, p.counts);
+    if (int e = check_launch("confusion_from_rows_kernel")) return e;
+    const long long fgrid = resident_grid(p.n_items, confusion_fix_kernel, 256, 0, 4);
+    OCTM_TIMED("confusion_fix_kernel", stream) confusion_fix_kernel<<<static_cast<unsigned>(fgrid), 256, 0, stream>>>(
+        p.yt, p.yp, p.n_items, p.H, p.W, p.K, p.unsorted, p.counts);
+    return check_launch("confusion_fix_kernel");
+}
+
 int run_label_pass(const LabelPassParams& p, bool conf, bool cols, bool seeds, cudaStream_t stream) {
     if (p.n_items == 0) return OCTM_OK;
     if (fast_ok(p.H, p.W, p.K, p.yt, p.yp) && p.n_items * p.H < (1ll << 31) /* TMA row coordinate */ &&
@@ -1313,9 +1496,18 @@ int run_label_pass(const LabelPassParams& p, bool conf, bool cols, bool seeds, c
         (p.bnd_p == nullptr || reinterpret_cast<uintptr_t>(p.bnd_p) % 16 == 0)) {
         // the suite's call: certificate; seeds (if asked for) from the column totals, rescanned for rejected maps
         if (p.unsorted != nullptr) {
-            const int e = p.first_pos != nullptr && seeds_per_pixel() ? dispatch_np<true, true, true, true>(p, stream)
-                                                                      : dispatch_np<true, true, false, true>(p, stream);
-            if (e != OCTM_OK || p.first_pos == nullptr) return e;
+            const bool per_pixel = stream_mostly_rejected();
+            int e;
+            if (!per_pixel && p.bnd_t != nullptr) {
+                LabelPassParams q = p;
+                q.counts = nullptr;                  // written whole by the two kernels below
+                e = dispatch_np<false, true, false, true>(q, stream);
+                if (e == OCTM_OK) e = confusion_from_rows(p, stream);
+            } else {
+                e = p.first_pos != nullptr && per_pixel ? dispatch_np<true, true, true, true>(p, stream)
+                                                        : dispatch_np<true, true, false, true>(p, stream);
+            }
+            if (e != OCTM_OK) return e;
             return report_rejected(p, stream);
         }
         if (conf && cols && seeds) return dispatch_np<true, true, true, false>(p, stream);
