@@ -310,6 +310,27 @@ OCTM_API int octm_surface3d_u8(const uint8_t* y_true, const uint8_t* y_pred, int
                       int unit_begin, int unit_end, uint32_t* n_pts, uint32_t* max_sq, uint32_t* p95_sq,
                       double* sum_dist, void* workspace, size_t workspace_bytes, void* stream);
 
+/* The same surfaces, units and directions in physical units, plus normalized-surface-Dice counts.
+ *   spacing    double [3]: voxel spacing along D0, D1, D2 (finite, > 0, each square a normal double, the squared
+ *              diagonal of the volume finite).  With w_i = spacing[i]^2 the squared distance
+ *              to a source voxel at integer offset (a, b, c) is d2 = w0*a^2 + (w1*b^2 + w2*c^2), float64, in that order
+ *   tolerances double [num_tolerances], 0 <= num_tolerances <= 4, each finite and >= 0, in the units of spacing; a
+ *              query voxel is within tau when sqrt(d2) <= tau (float64)
+ *   n_pts      uint32 [K][2] as octm_surface3d_u8 (0 when either surface is empty)
+ *   max_sq     double [K][2], p95_sq double [K][2][2] (order statistics of d2 at ranks floor((m-1)*0.95) and the next),
+ *   sum_dist   double [K][2] (sum of sqrt(d2)); all bit-reproducible from run to run
+ *   n_surf     uint32 [K][2] surface voxels of y_true / y_pred, counted even when the other surface is empty
+ *   n_within   uint32 [K][2][num_tolerances] query voxels within each tolerance, per direction
+ *   n_surf and n_within may be null only when num_tolerances == 0.
+ * Unit (c, dir) writes only n_pts[c][1 - dir], n_surf[c][1 - dir] and its own [c][dir] entries.  Never uses the
+ * near-field path.  Limits: D0, D1 <= 2048, D2 <= 65534; workspace 16 B per voxel and a little more. */
+OCTM_API size_t octm_surface3d_spacing_workspace_bytes(int D0, int D1, int D2);
+OCTM_API int octm_surface3d_spacing_u8(const uint8_t* y_true, const uint8_t* y_pred, int D0, int D1, int D2,
+                      int num_classes, int unit_begin, int unit_end, const double* spacing,
+                      const double* tolerances, int num_tolerances, uint32_t* n_pts, double* max_sq,
+                      double* p95_sq, double* sum_dist, uint32_t* n_surf, uint32_t* n_within,
+                      void* workspace, size_t workspace_bytes, void* stream);
+
 /* ---------------------------------------------------------------------------------------------
  * Front end: model scores -> uint8 label map, argmax over the class dimension (what a user does between
  * a model's forward() and the metric functions; every model of the reference returns

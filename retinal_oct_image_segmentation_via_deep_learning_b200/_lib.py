@@ -59,6 +59,9 @@ SIGNATURES = {
     "octm_topology_violations_float": (_INT, [_P, _INT, _I64, _INT, _I64, _P, _P, _P]),
     "octm_surface3d_workspace_bytes": (_c.c_size_t, [_INT, _INT, _INT]),
     "octm_surface3d_u8": (_INT, [_P, _P, _INT, _INT, _INT, _INT, _INT, _INT, _P, _P, _P, _P, _P, _c.c_size_t, _P]),
+    "octm_surface3d_spacing_workspace_bytes": (_c.c_size_t, [_INT, _INT, _INT]),
+    "octm_surface3d_spacing_u8": (_INT, [_P, _P, _INT, _INT, _INT, _INT, _INT, _INT, _P, _P, _INT, _P, _P, _P, _P, _P, _P,
+                                         _P, _c.c_size_t, _P]),
     "octm_host_pack_nibbles": (_INT, [_P, _P, _c.c_size_t, _INT]),
     "octm_unpack_nibbles_u8": (_INT, [_P, _I64, _P, _P]),
     "octm_labels_from_boundaries": (_INT, [_P, _INT, _I64, _INT, _INT, _INT, _P, _P]),

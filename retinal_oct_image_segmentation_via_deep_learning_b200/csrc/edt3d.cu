@@ -21,7 +21,11 @@
 //                      global atomics for the rest).
 //   select             one CTA scans the histogram: count, max, order statistics, sum of count*sqrt(D2)
 //                      in a fixed order (deterministic).
+// octm_surface3d_spacing_u8 (end of the file) measures the same distances with a physical voxel spacing.
+#include <cmath>
 #include <cstdlib>
+#include <type_traits>
+#include <utility>
 
 #include "common.cuh"
 
@@ -163,19 +167,23 @@ __global__ void __launch_bounds__(128) edt3_pass1_vec_kernel(const Edt3Params pr
 }
 
 // ------------------------------------------------------------------------------------------ envelope
-// Lower envelope of the parabolas  x -> (x - j)^2 + w(j)  over the finite sites j of one line
+// Lower envelope of the parabolas  x -> a (x - j)^2 + w(j)  over the finite sites j of one line
 // (Meijster et al.).  s[k] = site of region k, t[k] = first x of region k.  Returns the top index q
-// (-1: the line has no finite site).
-template <class W>
-__device__ __forceinline__ int build_envelope(int n, W weight, uint16_t* s, uint16_t* t) {
+// (-1: the line has no finite site).  T = long long with a = 1: exact integers (voxel units); T = double: a is the
+// squared spacing of the line's axis and every value is computed as a * (x - j)^2 + w(j), the expression the passes
+// report.
+template <class W, class T = decltype(std::declval<W>()(0))>
+__device__ __forceinline__ int build_envelope(int n, W weight, uint16_t* s, uint16_t* t, T a = T(1)) {
     int q = -1;
-    long long wtop = 0, itop = 0, ttop = 0;       // weight, site and first x of the top region, kept in registers
+    T wtop = 0;                                   // weight, site and first x of the top region, kept in registers
+    long long itop = 0, ttop = 0;
+    auto f = [a](long long x, long long i, T wi) -> T { return a * static_cast<T>((x - i) * (x - i)) + wi; };
     for (int u = 0; u < n; ++u) {
-        const long long wu = weight(u);
+        const T wu = weight(u);
         if (wu < 0) continue;                                   // infinite site
         while (q >= 0) {
-            const long long fi = (ttop - itop) * (ttop - itop) + wtop;
-            const long long fu = (ttop - u) * (ttop - u) + wu;
+            const T fi = f(ttop, itop, wtop);
+            const T fu = f(ttop, u, wu);
             if (fi <= fu) break;
             --q;                                                // u is lower over the whole top region: pop it
             if (q >= 0) {
@@ -190,10 +198,22 @@ __device__ __forceinline__ int build_envelope(int n, W weight, uint16_t* s, uint
             t[0] = 0;
             itop = u; ttop = 0; wtop = wu;
         } else {
-            // Meijster: Sep(i, u) = (u^2 - i^2 + w(u) - w(i)) div (2 (u - i)); u takes over from x = Sep + 1
-            const long long num = static_cast<long long>(u) * u - itop * itop + wu - wtop;
-            const long long den = 2 * (u - itop);
-            const long long sep = num >= 0 ? num / den : -((-num + den - 1) / den);       // floor division
+            long long sep;
+            if constexpr (std::is_integral<T>::value) {
+                // Meijster: Sep(i, u) = (u^2 - i^2 + w(u) - w(i)) div (2 (u - i)); u takes over from x = Sep + 1
+                const long long num = static_cast<long long>(u) * u - itop * itop + wu - wtop;
+                const long long den = 2 * (u - itop);
+                sep = num >= 0 ? num / den : -((-num + den - 1) / den);       // floor division
+            } else {
+                // the rounded crossing of the two parabolas, then moved to the last x at which the top site's value is
+                // still <= u's as f evaluates them (at ttop it is: the loop above stopped there), so that every region
+                // holds the site of least reported value
+                const double xc = ((wu - wtop) / a + static_cast<double>(static_cast<long long>(u) * u - itop * itop)) /
+                                  (2.0 * static_cast<double>(u - itop));
+                sep = xc >= n ? n - 1 : (xc <= ttop ? ttop : static_cast<long long>(floor(xc)));
+                while (sep + 1 < n && f(sep + 1, itop, wtop) <= f(sep + 1, u, wu)) ++sep;
+                while (sep > ttop && f(sep, itop, wtop) > f(sep, u, wu)) --sep;
+            }
             const long long w = sep + 1;
             if (w < n) {
                 ++q;
@@ -570,6 +590,277 @@ __global__ void __launch_bounds__(1024) edt3_select_kernel(const Sel3Params prm)
     }
 }
 
+// ================================================================================================ physical spacing
+// octm_surface3d_spacing_u8: the same surfaces and directions, distances in the units of a voxel spacing (s0, s1, s2).
+// With w_i = s_i^2 the squared distance to a source voxel at offset (a, b, c) is  d2 = w0 a^2 + (w1 b^2 + w2 c^2),
+// evaluated in float64 in exactly that order: pass 2 forms w1 b^2 + w2 g^2, pass 3 adds w0 a^2.  Pass 1 (g, integer
+// voxels along D2) does not depend on the weights and is the kernel above.  There is no integer histogram: pass 3
+// stores the query voxels' d2 (their bit patterns: order-preserving for non-negative doubles) in one segment per CTA,
+// the order statistics come from an 8-pass radix select over those bits, the sum of sqrt(d2) from per-CTA sums over a
+// fixed set of lines added in a fixed order.  Everything is bit-reproducible.  The near-field path is not used (its
+// byte planes hold integer squared distances).
+constexpr int kW3Threads = 128;          // pass-3 CTA: one D0 line per thread, CTA b owns lines [128 b, 128 b + 128)
+constexpr int kMaxTol = 4;
+enum { kAccCount, kAccMax, kAccSurf, kAccWithin, kAccWords = kAccWithin + kMaxTol };
+
+struct Edt3wParams {
+    const uint8_t* qry;            // volume whose class surface holds the query voxels
+    int D0, D1, D2, cls;
+    const uint16_t* g;             // pass 1: [D0][D1][D2] distance along D2 in voxels
+    double* h2;                    // [D0][D1][D2] w1 b^2 + w2 c^2 to the nearest source voxel of the i0 plane, -1: none
+    double w0, w1, w2;
+    double tau[kMaxTol];
+    int ntau;
+    unsigned long long* vals;      // [blocks][kW3Threads * D0] d2 bits of the query voxels of each pass-3 CTA
+    uint32_t* seg_n;               // [blocks] values of each CTA
+    double* seg_sum;               // [blocks] sum of sqrt(d2) of each CTA
+    unsigned long long* acc;       // [kAccWords]: count, max d2 bits, query surface voxels, within each tolerance
+};
+
+__global__ void __launch_bounds__(128) edt3w_pass2_kernel(const Edt3wParams prm) {
+    const int D0 = prm.D0, D1 = prm.D1, D2 = prm.D2;
+    const double w1 = prm.w1, w2 = prm.w2;
+    const long long lines = static_cast<long long>(D0) * D2;
+    uint16_t s[kMaxLine], t[kMaxLine];
+    for (long long line = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x; line < lines;
+         line += static_cast<long long>(gridDim.x) * blockDim.x) {
+        const int i0 = static_cast<int>(line / D2), i2 = static_cast<int>(line % D2);
+        const uint16_t* g = prm.g + static_cast<long long>(i0) * D1 * D2 + i2;       // element j at g[j * D2]
+        double* h = prm.h2 + static_cast<long long>(i0) * D1 * D2 + i2;
+        auto weight = [&](int j) -> double {
+            const uint32_t v = g[static_cast<long long>(j) * D2];
+            return v == kInf16 ? -1.0 : w2 * static_cast<double>(v * v);
+        };
+        int q = build_envelope(D1, weight, s, t, w1);
+        if (q < 0) {
+            for (int x = 0; x < D1; ++x) h[static_cast<long long>(x) * D2] = -1.0;
+            continue;
+        }
+        long long i = s[q];
+        double wi = weight(static_cast<int>(i));
+        int tq = t[q];
+        for (int x = D1 - 1; x >= 0; --x) {
+            h[static_cast<long long>(x) * D2] = w1 * static_cast<double>((x - i) * (x - i)) + wi;
+            if (x == tq && q > 0) {
+                --q;
+                i = s[q];
+                tq = t[q];
+                wi = weight(static_cast<int>(i));
+            }
+        }
+    }
+}
+
+__global__ void __launch_bounds__(kW3Threads) edt3w_pass3_kernel(const Edt3wParams prm) {
+    __shared__ uint32_t s_n;
+    __shared__ unsigned long long s_acc[kAccWords];
+    __shared__ double s_sum[kW3Threads / 32];
+    const int D0 = prm.D0, D1 = prm.D1, D2 = prm.D2, cls = prm.cls, tid = threadIdx.x;
+    const long long plane = static_cast<long long>(D1) * D2;
+    if (tid < kAccWords) s_acc[tid] = 0;
+    if (tid == 0) s_n = 0;
+    __syncthreads();
+    unsigned long long* vals = prm.vals + static_cast<long long>(blockIdx.x) * kW3Threads * D0;
+    const long long line = static_cast<long long>(blockIdx.x) * kW3Threads + tid;
+    double sum = 0.0;
+    unsigned long long mx = 0;
+    uint32_t n = 0, nsurf = 0, within[kMaxTol] = {0, 0, 0, 0};
+    if (line < plane) {
+        uint16_t s[kMaxLine], t[kMaxLine];
+        const int i1 = static_cast<int>(line / D2), i2 = static_cast<int>(line % D2);
+        const double* h = prm.h2 + line;                                            // element j at h[j * plane]
+        auto weight = [&](int j) -> double { return h[static_cast<long long>(j) * plane]; };
+        const double w0 = prm.w0;
+        int q = build_envelope(D0, weight, s, t, w0);                               // -1: no source surface at all
+        long long i = q >= 0 ? s[q] : 0;
+        double wi = q >= 0 ? weight(static_cast<int>(i)) : 0.0;
+        int tq = q >= 0 ? t[q] : 0;
+        for (int x = D0 - 1; x >= 0; --x) {
+            if (surface_at(prm.qry, D0, D1, D2, x, i1, i2, cls)) {
+                ++nsurf;                                                            // counted without a source too
+                if (q >= 0) {
+                    const double d2 = w0 * static_cast<double>((x - i) * (x - i)) + wi;
+                    const double d = sqrt(d2);
+                    sum = __dadd_rn(sum, d);
+#pragma unroll
+                    for (int j = 0; j < kMaxTol; ++j) within[j] += j < prm.ntau && d <= prm.tau[j] ? 1u : 0u;
+                    const unsigned long long bits = static_cast<unsigned long long>(__double_as_longlong(d2));
+                    mx = max(mx, bits);
+                    vals[atomicAdd(&s_n, 1u)] = bits;
+                    ++n;
+                }
+            }
+            if (x == tq && q > 0) {
+                --q;
+                i = s[q];
+                tq = t[q];
+                wi = weight(static_cast<int>(i));
+            }
+        }
+    }
+    // CTA totals: the float sum in a fixed order (lanes tree, then warps in order), integers by atomics
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        sum = __dadd_rn(sum, __shfl_xor_sync(0xffffffffu, sum, o));
+        mx = max(mx, __shfl_xor_sync(0xffffffffu, mx, o));
+    }
+    n = __reduce_add_sync(0xffffffffu, n);
+    nsurf = __reduce_add_sync(0xffffffffu, nsurf);
+#pragma unroll
+    for (int j = 0; j < kMaxTol; ++j) within[j] = __reduce_add_sync(0xffffffffu, within[j]);
+    if ((tid & 31) == 0) {
+        s_sum[tid >> 5] = sum;
+        atomicAdd(&s_acc[kAccCount], static_cast<unsigned long long>(n));
+        atomicMax(&s_acc[kAccMax], mx);
+        atomicAdd(&s_acc[kAccSurf], static_cast<unsigned long long>(nsurf));
+        for (int j = 0; j < kMaxTol; ++j) atomicAdd(&s_acc[kAccWithin + j], static_cast<unsigned long long>(within[j]));
+    }
+    __syncthreads();
+    if (tid == 0) {
+        double cta = 0.0;
+        for (int w = 0; w < kW3Threads / 32; ++w) cta = __dadd_rn(cta, s_sum[w]);
+        prm.seg_sum[blockIdx.x] = cta;
+        prm.seg_n[blockIdx.x] = s_n;
+    }
+    if (tid < kAccWords && s_acc[tid] != 0) {
+        if (tid == kAccMax) atomicMax(&prm.acc[tid], s_acc[tid]);
+        else atomicAdd(&prm.acc[tid], s_acc[tid]);
+    }
+}
+
+struct Sel3wParams {
+    const unsigned long long* vals;
+    const uint32_t* seg_n;
+    const double* seg_sum;
+    const unsigned long long* acc;
+    unsigned long long* hist;      // [8 passes][2 ranks][256]: digit counts of the values that share the rank's prefix
+    long long seg_len;             // kW3Threads * D0
+    int nseg, pass, ntau;
+    uint32_t* n_pts;               // [1]
+    double* max_sq;                // [1]
+    double* p95_sq;                // [2]
+    double* sum_dist;              // [1]
+    uint32_t* n_surf;              // [1] or null
+    uint32_t* n_within;            // [ntau]
+};
+
+// the two ranks numpy's linear 95th percentile interpolates between among m > 0 values (as edt3_select_kernel)
+__device__ __forceinline__ void p95_ranks(unsigned long long m, unsigned long long& lo, unsigned long long& hi) {
+    lo = static_cast<unsigned long long>(floor(__dmul_rn(static_cast<double>(m - 1), 0.95)));
+    hi = lo + 1 < m ? lo + 1 : lo;
+}
+
+// One warp: the top 8 * passes bits of the value of rank k, from the digit counts of the first `passes` passes (h: this
+// rank's counts of pass 0, 512 apart per pass).  Every lane returns the same prefix.
+__device__ unsigned long long radix_prefix(const unsigned long long* h, int passes, unsigned long long k) {
+    const int lane = threadIdx.x & 31;
+    unsigned long long prefix = 0, rank = k;
+    for (int p = 0; p < passes; ++p, h += 512) {
+        unsigned long long c[8], tot = 0;
+#pragma unroll
+        for (int j = 0; j < 8; ++j) { c[j] = h[lane * 8 + j]; tot += c[j]; }
+        unsigned long long inc = tot;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const unsigned long long v = __shfl_up_sync(0xffffffffu, inc, o);
+            if (lane >= o) inc += v;
+        }
+        const unsigned long long exc = inc - tot;
+        const bool mine = exc <= rank && rank < inc;
+        const int owner = __ffs(__ballot_sync(0xffffffffu, mine)) - 1;
+        int d = 0;
+        unsigned long long r = rank - exc;
+        if (mine) {
+            for (int j = 0; j < 8; ++j) {
+                if (r < c[j]) { d = lane * 8 + j; break; }
+                r -= c[j];
+            }
+        }
+        prefix = (prefix << 8) | static_cast<unsigned long long>(__shfl_sync(0xffffffffu, d, owner));
+        rank = __shfl_sync(0xffffffffu, r, owner);
+    }
+    return prefix;
+}
+
+// radix-select pass p: digit p (bits 63 - 8p .. 56 - 8p) of the values whose top 8p bits are the prefix of either rank
+__global__ void __launch_bounds__(256) edt3w_radix_kernel(const Sel3wParams prm) {
+    __shared__ unsigned long long s_hist[512];
+    __shared__ unsigned long long s_prefix[2];
+    const unsigned long long m = prm.acc[kAccCount];
+    if (m == 0) return;
+    const int p = prm.pass, tid = threadIdx.x;
+    for (int i = tid; i < 512; i += blockDim.x) s_hist[i] = 0;
+    if (tid < 32) {
+        unsigned long long lo, hi;
+        p95_ranks(m, lo, hi);
+        const unsigned long long pl = radix_prefix(prm.hist, p, lo), ph = radix_prefix(prm.hist + 256, p, hi);
+        if (tid == 0) { s_prefix[0] = pl; s_prefix[1] = ph; }
+    }
+    __syncthreads();
+    const int shift = 56 - 8 * p;
+    const unsigned long long pl = s_prefix[0], ph = s_prefix[1];
+    for (int seg = blockIdx.x; seg < prm.nseg; seg += gridDim.x) {
+        const uint32_t n = prm.seg_n[seg];
+        const unsigned long long* v = prm.vals + seg * prm.seg_len;
+        // most values share their top digits: the lanes of a warp that hit the same counter add to it once
+        // (the loop bound is uniform over the CTA, so every warp is converged at the match)
+        for (uint32_t base = 0; base < n; base += blockDim.x) {
+            const uint32_t e = base + tid;
+            uint32_t klo = 0xffffffffu, khi = 0xffffffffu;
+            if (e < n) {
+                const unsigned long long x = v[e];
+                const unsigned long long top = p == 0 ? 0ull : x >> (shift + 8);
+                const uint32_t d = static_cast<uint32_t>(x >> shift) & 0xffu;
+                if (top == pl) klo = d;
+                if (top == ph) khi = 256 + d;
+            }
+            const uint32_t mlo = __match_any_sync(0xffffffffu, klo), mhi = __match_any_sync(0xffffffffu, khi);
+            if (klo != 0xffffffffu && (mlo & lanemask_lt()) == 0) atomicAdd(&s_hist[klo], static_cast<unsigned long long>(__popc(mlo)));
+            if (khi != 0xffffffffu && (mhi & lanemask_lt()) == 0) atomicAdd(&s_hist[khi], static_cast<unsigned long long>(__popc(mhi)));
+        }
+    }
+    __syncthreads();
+    for (int i = tid; i < 512; i += blockDim.x)
+        if (s_hist[i]) atomicAdd(&prm.hist[p * 512 + i], s_hist[i]);
+}
+
+__global__ void __launch_bounds__(1024) edt3w_finish_kernel(const Sel3wParams prm) {
+    __shared__ double s_dsum[32];
+    __shared__ unsigned long long s_sel[2];
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const unsigned long long m = prm.acc[kAccCount];
+    // fixed-order float64 sum of the per-CTA sums: contiguous chunks per thread, lanes tree, warps in order
+    const int chunk = (prm.nseg + 1023) / 1024;
+    const int b = min(prm.nseg, tid * chunk), e = min(prm.nseg, b + chunk);
+    double ds = 0.0;
+    for (int v = b; v < e; ++v) ds = __dadd_rn(ds, prm.seg_sum[v]);
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) ds = __dadd_rn(ds, __shfl_xor_sync(0xffffffffu, ds, o));
+    if (lane == 0) s_dsum[warp] = ds;
+    if (warp == 0) {
+        unsigned long long lo = 0, hi = 0, vl = 0, vh = 0;
+        if (m > 0) {
+            p95_ranks(m, lo, hi);
+            vl = radix_prefix(prm.hist, 8, lo);
+            vh = radix_prefix(prm.hist + 256, 8, hi);
+        }
+        if (lane == 0) { s_sel[0] = vl; s_sel[1] = vh; }
+    }
+    __syncthreads();
+    if (tid == 0) {
+        double sum = 0.0;
+        for (int w = 0; w < 32; ++w) sum = __dadd_rn(sum, s_dsum[w]);
+        auto clamp32 = [](unsigned long long v) { return static_cast<uint32_t>(v > 0xffffffffull ? 0xffffffffull : v); };
+        prm.n_pts[0] = clamp32(m);
+        prm.max_sq[0] = __longlong_as_double(static_cast<long long>(prm.acc[kAccMax]));
+        prm.p95_sq[0] = __longlong_as_double(static_cast<long long>(s_sel[0]));
+        prm.p95_sq[1] = __longlong_as_double(static_cast<long long>(s_sel[1]));
+        prm.sum_dist[0] = sum;
+        if (prm.n_surf) prm.n_surf[0] = clamp32(prm.acc[kAccSurf]);
+        for (int j = 0; j < prm.ntau; ++j) prm.n_within[j] = clamp32(prm.acc[kAccWithin + j]);
+    }
+}
+
 }  // namespace octm
 
 static uint32_t edt3_nbins(int D0, int D1, int D2) {
@@ -675,6 +966,123 @@ extern "C" int octm_surface3d_u8(const uint8_t* y_true, const uint8_t* y_pred, i
         octm::Sel3Params sp{hist, nbins, n_pts + cls * 2 + (1 - dir), max_sq + unit, p95_sq + 2 * unit, sum_dist + unit};
         OCTM_TIMED("edt3_select_kernel", st) octm::edt3_select_kernel<<<1, 1024, 0, st>>>(sp);
         if (int e = octm::check_launch("edt3_select_kernel")) return e;
+    }
+    return OCTM_OK;
+}
+
+// physical-spacing workspace: g and then the pass-3 value segments (g is dead once pass 2 has run), h2 (float64), the
+// per-CTA counts and sums of pass 3, the unit's totals and radix-select digit counts
+namespace {
+struct Edt3wLayout {
+    size_t vals, h2, seg_n, seg_sum, acc, total;
+    long long nseg;
+};
+Edt3wLayout edt3w_layout(int D0, int D1, int D2) {
+    auto up = [](size_t v) { return (v + 255) & ~static_cast<size_t>(255); };
+    Edt3wLayout L{};
+    const size_t vox = static_cast<size_t>(D0) * D1 * D2;
+    L.nseg = (static_cast<long long>(D1) * D2 + octm::kW3Threads - 1) / octm::kW3Threads;
+    L.vals = 0;
+    L.h2 = L.vals + up(static_cast<size_t>(L.nseg) * octm::kW3Threads * D0 * 8);
+    L.seg_n = L.h2 + up(vox * 8);
+    L.seg_sum = L.seg_n + up(static_cast<size_t>(L.nseg) * 4);
+    L.acc = L.seg_sum + up(static_cast<size_t>(L.nseg) * 8);
+    L.total = L.acc + up((octm::kAccWords + 8 * 512) * 8);
+    return L;
+}
+}  // namespace
+
+extern "C" size_t octm_surface3d_spacing_workspace_bytes(int D0, int D1, int D2) {
+    if (D0 < 1 || D1 < 1 || D2 < 1) return 0;
+    return edt3w_layout(D0, D1, D2).total;
+}
+
+extern "C" int octm_surface3d_spacing_u8(const uint8_t* y_true, const uint8_t* y_pred, int D0, int D1, int D2,
+                                         int num_classes, int unit_begin, int unit_end, const double* spacing,
+                                         const double* tolerances, int num_tolerances, uint32_t* n_pts, double* max_sq,
+                                         double* p95_sq, double* sum_dist, uint32_t* n_surf, uint32_t* n_within,
+                                         void* workspace, size_t workspace_bytes, void* stream) {
+    if (D0 < 1 || D1 < 1 || D2 < 1) return octm::fail(OCTM_ERR_INVALID, "bad volume shape");
+    if (num_classes < 1 || num_classes > 256) return octm::fail(OCTM_ERR_INVALID, "num_classes outside [1, 256]");
+    if (unit_begin < 0 || unit_end > 2 * num_classes || unit_begin > unit_end) return octm::fail(OCTM_ERR_INVALID, "bad unit range");
+    if (D0 > octm::kMaxLine || D1 > octm::kMaxLine || D2 > 65534)
+        return octm::fail(OCTM_ERR_UNSUPPORTED, "volume sides: D0, D1 <= %d and D2 <= 65534", octm::kMaxLine);
+    if (!y_true || !y_pred || !n_pts || !max_sq || !p95_sq || !sum_dist || !spacing) return octm::fail(OCTM_ERR_INVALID, "null pointer");
+    for (int a = 0; a < 3; ++a)
+        if (!std::isfinite(spacing[a]) || !(spacing[a] > 0.0))
+            return octm::fail(OCTM_ERR_INVALID, "spacing[%d] = %g: must be finite and > 0", a, spacing[a]);
+    // the kernels work with w = spacing^2: it must be a normal double (no overflow to inf, no underflow to 0 or
+    // subnormals), and so must the largest squared distance the volume can hold
+    for (int a = 0; a < 3; ++a)
+        if (!std::isnormal(spacing[a] * spacing[a]))
+            return octm::fail(OCTM_ERR_INVALID, "spacing[%d] = %g: its square is not a normal double", a, spacing[a]);
+    const double diag2 = spacing[0] * spacing[0] * (1.0 * (D0 - 1) * (D0 - 1)) + spacing[1] * spacing[1] * (1.0 * (D1 - 1) * (D1 - 1)) +
+                         spacing[2] * spacing[2] * (1.0 * (D2 - 1) * (D2 - 1));
+    if (!std::isfinite(diag2))
+        return octm::fail(OCTM_ERR_INVALID, "spacing: the squared diagonal of the volume overflows a double");
+    if (num_tolerances < 0 || num_tolerances > octm::kMaxTol)
+        return octm::fail(OCTM_ERR_INVALID, "num_tolerances %d outside [0, %d]", num_tolerances, octm::kMaxTol);
+    if (num_tolerances > 0 && (!tolerances || !n_surf || !n_within))
+        return octm::fail(OCTM_ERR_INVALID, "null pointer: tolerances, n_surf and n_within are needed with tolerances");
+    for (int j = 0; j < num_tolerances; ++j)
+        if (!std::isfinite(tolerances[j]) || !(tolerances[j] >= 0.0))
+            return octm::fail(OCTM_ERR_INVALID, "tolerances[%d] = %g: must be finite and >= 0", j, tolerances[j]);
+    const Edt3wLayout L = edt3w_layout(D0, D1, D2);
+    if (workspace == nullptr || workspace_bytes < L.total)
+        return octm::fail(OCTM_ERR_WORKSPACE, "workspace too small: need %zu B", L.total);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    uint8_t* ws = static_cast<uint8_t*>(workspace);
+    uint16_t* g = reinterpret_cast<uint16_t*>(ws + L.vals);
+    unsigned long long* vals = reinterpret_cast<unsigned long long*>(ws + L.vals);
+    double* h2 = reinterpret_cast<double*>(ws + L.h2);
+    uint32_t* seg_n = reinterpret_cast<uint32_t*>(ws + L.seg_n);
+    double* seg_sum = reinterpret_cast<double*>(ws + L.seg_sum);
+    unsigned long long* acc = reinterpret_cast<unsigned long long*>(ws + L.acc);
+    unsigned long long* hist = acc + octm::kAccWords;
+    const int sms = octm::sm_count();
+    auto blocks = [&](long long threads, long long per_sm) {
+        long long b = (threads + 127) / 128;
+        const long long cap = static_cast<long long>(sms) * per_sm;
+        return static_cast<unsigned>(b < cap ? b : cap);
+    };
+    octm::Edt3wParams wp{};
+    wp.D0 = D0; wp.D1 = D1; wp.D2 = D2;
+    wp.g = g; wp.h2 = h2;
+    wp.w0 = spacing[0] * spacing[0];
+    wp.w1 = spacing[1] * spacing[1];
+    wp.w2 = spacing[2] * spacing[2];
+    for (int j = 0; j < num_tolerances; ++j) wp.tau[j] = tolerances[j];
+    wp.ntau = num_tolerances;
+    wp.vals = vals; wp.seg_n = seg_n; wp.seg_sum = seg_sum; wp.acc = acc;
+    for (int unit = unit_begin; unit < unit_end; ++unit) {
+        const int cls = unit >> 1, dir = unit & 1;
+        // direction 0: queries = y_pred surface, sources = y_true surface; 1 swapped (as octm_surface3d_u8)
+        const uint8_t* src = dir == 0 ? y_true : y_pred;
+        octm::Edt3Params p{src, nullptr, D0, D1, D2, cls, g, nullptr, nullptr, 0, nullptr};
+        wp.qry = dir == 0 ? y_pred : y_true;
+        wp.cls = cls;
+        if (cudaMemsetAsync(acc, 0, (octm::kAccWords + 8 * 512) * 8, st) != cudaSuccess)
+            return octm::fail(OCTM_ERR_LAUNCH, "memset(acc) failed");
+        if (D2 % 16 == 0 && reinterpret_cast<uintptr_t>(src) % 16 == 0)
+            OCTM_TIMED("edt3_pass1_vec_kernel", st) octm::edt3_pass1_vec_kernel<<<blocks(1ll * D0 * D1, 16), 128, 0, st>>>(p);
+        else
+            OCTM_TIMED("edt3_pass1_kernel", st) octm::edt3_pass1_kernel<<<blocks(1ll * D0 * D1, 16), 128, 0, st>>>(p);
+        if (int e = octm::check_launch("edt3_pass1_kernel")) return e;
+        OCTM_TIMED("edt3w_pass2_kernel", st) octm::edt3w_pass2_kernel<<<blocks(1ll * D0 * D2, 16), 128, 0, st>>>(wp);
+        if (int e = octm::check_launch("edt3w_pass2_kernel")) return e;
+        OCTM_TIMED("edt3w_pass3_kernel", st) octm::edt3w_pass3_kernel<<<static_cast<unsigned>(L.nseg), octm::kW3Threads, 0, st>>>(wp);
+        if (int e = octm::check_launch("edt3w_pass3_kernel")) return e;
+        // n_pts and n_surf keep the layout [K][2] = (y_true, y_pred): direction 0 queries y_pred's surface
+        octm::Sel3wParams sp{vals, seg_n, seg_sum, acc, hist, 1ll * octm::kW3Threads * D0, static_cast<int>(L.nseg), 0,
+                             num_tolerances, n_pts + cls * 2 + (1 - dir), max_sq + unit, p95_sq + 2 * unit, sum_dist + unit,
+                             n_surf ? n_surf + cls * 2 + (1 - dir) : nullptr,
+                             n_within ? n_within + unit * num_tolerances : nullptr};
+        for (sp.pass = 0; sp.pass < 8; ++sp.pass) {
+            OCTM_TIMED("edt3w_radix_kernel", st) octm::edt3w_radix_kernel<<<blocks(L.nseg * 128, 2), 256, 0, st>>>(sp);
+            if (int e = octm::check_launch("edt3w_radix_kernel")) return e;
+        }
+        OCTM_TIMED("edt3w_finish_kernel", st) octm::edt3w_finish_kernel<<<1, 1024, 0, st>>>(sp);
+        if (int e = octm::check_launch("edt3w_finish_kernel")) return e;
     }
     return OCTM_OK;
 }

@@ -79,6 +79,23 @@ def read_mhd(path):
     return arr.reshape(shape).astype(dtype.newbyteorder("="), copy=False), header
 
 
+def mhd_spacing(header):
+    """Voxel spacing of a ``read_mhd`` header in the order of the array's axes (``[slices, rows, cols]`` for a volume),
+    ready for ``suite.surface_distance_3d(spacing=...)``: the header lists ``ElementSpacing`` fastest axis first (x, y,
+    z), so the order is reversed.  KeyError without ``ElementSpacing``, ValueError when it does not have ``NDims``
+    numbers."""
+    if "ElementSpacing" not in header:
+        raise KeyError("the MetaImage header has no ElementSpacing")
+    try:
+        sp = [float(v) for v in header["ElementSpacing"].split()]
+    except ValueError:
+        raise ValueError(f"ElementSpacing {header['ElementSpacing']!r} is not a list of numbers") from None
+    ndims = int(header.get("NDims", len(sp)))
+    if len(sp) != ndims:
+        raise ValueError(f"ElementSpacing has {len(sp)} entries, NDims = {ndims}")
+    return tuple(reversed(sp))
+
+
 def write_mhd(path, array, spacing=None, compressed=False):
     """Write ``array`` (C order ``[slices, rows, cols]``) as ``path`` (.mhd) + a sibling .raw / .zraw file."""
     array = np.ascontiguousarray(array)

@@ -84,9 +84,11 @@ def contour_metrics(n_pts, max_sq, p95_sq, sum_dist, lattice=4.0):
     indexed by direction (0: pred vertices -> true contour = ``d1``; 1: true -> pred = ``d2``).
     Entries whose masks have no contour (the reference raises IndexError) come back as NaN.
     ``lattice``: squared length unit of the integer distances -- 4.0 for the doubled lattice of the 2-D
-    contours (distance = sqrt(D2 / 4)), 1.0 for the voxel lattice of the 3-D surfaces."""
+    contours (distance = sqrt(D2 / 4)), 1.0 for the voxel lattice of the 3-D surfaces.  Floating ``max_sq`` /
+    ``p95_sq`` (physical squared distances of the 3-D surfaces with a spacing) are taken as they are."""
     n_pts = np.asarray(n_pts).astype(np.int64)
-    max_sq = np.asarray(max_sq).astype(np.int64)
+    max_sq = np.asarray(max_sq)
+    max_sq = max_sq.astype(np.float64) if np.issubdtype(max_sq.dtype, np.floating) else max_sq.astype(np.int64)
     p95 = np.asarray(p95_sq).astype(np.float64)
     valid = (n_pts[..., 0] > 0) & (n_pts[..., 1] > 0)
     m = np.stack([n_pts[..., 1], n_pts[..., 0]], axis=-1)         # query count per direction

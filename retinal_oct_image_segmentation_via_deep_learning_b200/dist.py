@@ -233,27 +233,28 @@ def component_totals(res, world, device=None, group=None):
     return out
 
 
-def surface_distance_3d_sharded(vol_true, vol_pred, num_classes, rank, world, group=None):
+def surface_distance_3d_sharded(vol_true, vol_pred, num_classes, rank, world, group=None, spacing=None,
+                                tolerances=None):
     """BASELINE config 5 on several GPUs: the volume pair is replicated (it is small), the ``2 * K``
     independent (class, direction) distance transforms are split into contiguous unit ranges per rank,
     and the per-unit integers / sums are combined by ONE small all-reduce (every unit is written by exactly
     one rank, the others contribute zeros, so the sum is exact).  Returns the same dict as
-    ``suite.surface_distance_3d`` with identical contents on every rank."""
+    ``suite.surface_distance_3d`` (``spacing`` and ``tolerances`` passed through) with identical contents on every
+    rank."""
     import torch
     from . import suite
     ub, ue = shard_range(2 * num_classes, rank, world)
-    ints = suite.surface_distance_3d(vol_true, vol_pred, num_classes, units=(ub, ue))
+    ints = suite.surface_distance_3d(vol_true, vol_pred, num_classes, units=(ub, ue), spacing=spacing,
+                                     tolerances=tolerances)
     if world > 1:
         import torch.distributed as dist
-        packed = torch.cat([ints["n_pts"].to(torch.float64).reshape(-1), ints["max_sq"].to(torch.float64).reshape(-1),
-                            ints["p95_sq"].to(torch.float64).reshape(-1), ints["sum_dist"].reshape(-1)])
+        # every output in float64, in the dict's order: n_pts, max_sq, p95_sq, sum_dist[, n_surf, n_within]
+        packed = torch.cat([v.to(torch.float64).reshape(-1) for v in ints.values()])
         dist.all_reduce(packed, op=dist.ReduceOp.SUM, group=group)
-        k = num_classes
         o = 0
-        for key, shape, dt in (("n_pts", (k, 2), torch.int32), ("max_sq", (k, 2), torch.int32),
-                               ("p95_sq", (k, 2, 2), torch.int32), ("sum_dist", (k, 2), torch.float64)):
-            m = int(np.prod(shape))
-            v = packed[o:o + m].reshape(shape)
-            ints[key] = v.to(torch.int64).to(dt) if dt != torch.float64 else v.clone()
+        for key, v in list(ints.items()):
+            m = v.numel()
+            s = packed[o:o + m].reshape(v.shape)
+            ints[key] = s.clone() if v.dtype == torch.float64 else s.to(torch.int64).to(v.dtype)
             o += m
     return ints

@@ -920,14 +920,43 @@ def auc_scores(y_true, scores, *, single_class_value=float("nan")):
     return out
 
 
-def surface_distance_3d(vol_true, vol_pred, num_classes, *, units=None):
+SURFACE3D_MAX_TOL = 4           # tolerances per call of octm_surface3d_spacing_u8
+
+
+def surface3d_spacing_args(spacing, tolerances):
+    """``(spacing, tolerances)`` of ``surface_distance_3d`` -> (3 floats, tuple of 0 to 4 floats); ValueError unless the
+    spacing is 3 finite numbers > 0 whose squares are normal doubles and the tolerances 1 to 4 finite numbers >= 0
+    (``None``: none)."""
+    sp = (1.0, 1.0, 1.0) if spacing is None else tuple(np.asarray(spacing, dtype=np.float64).reshape(-1).tolist())
+    if len(sp) != 3 or not all(np.isfinite(s) and s > 0 for s in sp):
+        raise ValueError(f"spacing must be 3 finite numbers > 0, got {spacing!r}")
+    # the kernels work with the squares: each must be a normal double (no overflow to inf, no underflow)
+    if not all(np.isfinite(s * s) and s * s >= np.finfo(np.float64).tiny for s in sp):
+        raise ValueError(f"spacing {spacing!r}: the square of every entry must be a normal double")
+    if tolerances is None:
+        return sp, ()
+    taus = tuple(np.asarray(tolerances, dtype=np.float64).reshape(-1).tolist())
+    if not 1 <= len(taus) <= SURFACE3D_MAX_TOL:
+        raise ValueError(f"1 to {SURFACE3D_MAX_TOL} tolerances, got {len(taus)}")
+    if not all(np.isfinite(t) and t >= 0 for t in taus):
+        raise ValueError(f"tolerances must be finite and >= 0, got {tolerances!r}")
+    return sp, taus
+
+
+def surface_distance_3d(vol_true, vol_pred, num_classes, *, units=None, spacing=None, tolerances=None):
     """3-D surface-distance integers per class of two label volumes ``[D0, D1, D2]`` (BASELINE config 5).
 
     Surfaces = region voxels with a 6-neighbour outside the region; exact squared Euclidean distances by
     a separable distance transform.  ``units=(begin, end)`` restricts the work to a range of the
     ``2 * num_classes`` (class, direction) units (multi-GPU sharding; the other entries stay zero and
     the per-rank outputs add up).  Returns a dict of CUDA tensors ``n_pts [K, 2]``, ``max_sq [K, 2]``,
-    ``p95_sq [K, 2, 2]``, ``sum_dist [K, 2]``; ``surface_metrics_3d`` turns them into hd / hd95 / assd."""
+    ``p95_sq [K, 2, 2]``, ``sum_dist [K, 2]``; ``surface_metrics_3d`` turns them into hd / hd95 / assd.
+
+    ``spacing=(s0, s1, s2)``: voxel spacing along the three axes (e.g. ``datasets.mhd_spacing``); distances are then
+    physical, ``max_sq`` and ``p95_sq`` float64 squared distances ``w0 a^2 + (w1 b^2 + w2 c^2)`` with ``w = s^2``.
+    ``tolerances``: 1 to 4 distances in the units of the spacing (default spacing 1, 1, 1) for the normalized surface
+    Dice; adds ``n_surf [K, 2]`` (surface voxels of y_true, y_pred) and ``n_within [K, 2, T]`` (per direction, query
+    voxels with ``sqrt(d2) <= tau``).  With neither, the integer voxel-unit kernels run."""
     for name, t in (("vol_true", vol_true), ("vol_pred", vol_pred)):
         if not isinstance(t, torch.Tensor) or not t.is_cuda or t.dtype not in (torch.uint8, torch.bool) or t.dim() != 3:
             raise TypeError(f"{name} must be a CUDA uint8 tensor [D0, D1, D2]")
@@ -939,6 +968,8 @@ def surface_distance_3d(vol_true, vol_pred, num_classes, *, units=None):
     k = int(num_classes)
     ub, ue = (0, 2 * k) if units is None else (int(units[0]), int(units[1]))
     dev = vt.device
+    if spacing is not None or tolerances is not None:
+        return _surface_distance_3d_spacing(vt, vp, k, ub, ue, *surface3d_spacing_args(spacing, tolerances))
     out = {"n_pts": torch.zeros((k, 2), dtype=torch.int32, device=dev),
            "max_sq": torch.zeros((k, 2), dtype=torch.int32, device=dev),
            "p95_sq": torch.zeros((k, 2, 2), dtype=torch.int32, device=dev),
@@ -951,12 +982,40 @@ def surface_distance_3d(vol_true, vol_pred, num_classes, *, units=None):
     return out
 
 
+def _surface_distance_3d_spacing(vt, vp, k, ub, ue, spacing, taus):
+    d0, d1, d2 = vt.shape
+    dev = vt.device
+    out = {"n_pts": torch.zeros((k, 2), dtype=torch.int32, device=dev),
+           "max_sq": torch.zeros((k, 2), dtype=torch.float64, device=dev),
+           "p95_sq": torch.zeros((k, 2, 2), dtype=torch.float64, device=dev),
+           "sum_dist": torch.zeros((k, 2), dtype=torch.float64, device=dev)}
+    if taus:
+        out["n_surf"] = torch.zeros((k, 2), dtype=torch.int32, device=dev)
+        out["n_within"] = torch.zeros((k, 2, len(taus)), dtype=torch.int32, device=dev)
+    sp = (ctypes.c_double * 3)(*spacing)
+    tol = (ctypes.c_double * max(1, len(taus)))(*taus)
+    with torch.cuda.device(dev):
+        nbytes = int(_lib.load().octm_surface3d_spacing_workspace_bytes(d0, d1, d2))
+        ws = _vertex_scratch(dev, (nbytes + 3) // 4 + 64)
+        _lib.call("octm_surface3d_spacing_u8", _ptr(vt), _ptr(vp), d0, d1, d2, k, ub, ue, ctypes.addressof(sp),
+                  ctypes.addressof(tol), len(taus), _ptr(out["n_pts"]), _ptr(out["max_sq"]), _ptr(out["p95_sq"]),
+                  _ptr(out["sum_dist"]), _ptr(out["n_surf"]) if taus else None,
+                  _ptr(out["n_within"]) if taus else None, _ptr(ws), ws.numel() * 4, _stream())
+    return out
+
+
 def surface_metrics_3d(ints):
     """hausdorff_distance / hausdorff_distance_95 / assd per class from ``surface_distance_3d`` outputs
-    (after any cross-rank sum), with the reference's 2-D definitions carried over to voxel surfaces."""
+    (after any cross-rank sum), with the reference's 2-D definitions carried over to voxel surfaces; in the units of the
+    spacing when one was given.  With tolerances also ``surface_dice [K, T]`` (``derive.surface_dice``)."""
     g = lambda key: ints[key].cpu().numpy() if isinstance(ints[key], torch.Tensor) else np.asarray(ints[key])   # noqa: E731
-    return derive.contour_metrics(g("n_pts").view(np.uint32), g("max_sq").view(np.uint32), g("p95_sq").view(np.uint32),
-                                  g("sum_dist"), lattice=1.0)
+    mx, p95 = g("max_sq"), g("p95_sq")
+    if not np.issubdtype(mx.dtype, np.floating):              # voxel units: uint32 squared distances in int32 tensors
+        mx, p95 = mx.view(np.uint32), p95.view(np.uint32)
+    out = derive.contour_metrics(g("n_pts").view(np.uint32), mx, p95, g("sum_dist"), lattice=1.0)
+    if "n_surf" in ints:
+        out["surface_dice"] = derive.surface_dice(g("n_surf").view(np.uint32), g("n_within").view(np.uint32))
+    return out
 
 
 def validate_labels(labels, num_classes):
