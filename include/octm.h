@@ -224,6 +224,24 @@ OCTM_API int octm_contour2d_distance(const uint32_t* verts, const uint32_t* n_pt
                             void* stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * Contour distances with a physical pixel spacing.  spacing is a HOST array {sy, sx}: the pixel size along rows (H,
+ * axial) and along columns (W, lateral), in any unit.  Same vertex lists (octm_contour2d_trace_u8 or
+ * octm_contour2d_all_vertices_u8), units and directions as octm_contour2d_distance; with wy = sy * sy, wx = sx * sx a
+ * vertex pair at lattice offset (a, b) is q = fl(fl(wy * a^2) + fl(wx * b^2)) in float64, in that order, and
+ *   d2       double [n][K][2][max_pts]  per query vertex, the minimum of q over the source set.  Required; with
+ *                                       keep_d2 == 0 it is scratch (short lists are kept in shared memory instead)
+ *   max_sq   double [n][K][2]           the largest d2
+ *   p95_sq   double [n][K][2][2]        the d2 of ranks floor((m - 1) * 0.95) and the next one (the same at the end)
+ *   sum_dist double [n][K][2]           sum of sqrt(d2 / 4.0), in a fixed order
+ * Distance = sqrt(d2 / 4.0) in the units of the spacing; at {1, 1} d2 equals the integer D2 and every statistic the
+ * pixel one (sum_dist up to its summation order).  Bit-reproducible run to run.  Every argument is checked before any
+ * CUDA call: both spacings finite and > 0, their squares normal doubles, q of the image diagonal finite. */
+OCTM_API int octm_contour2d_distance_spacing(const uint32_t* verts, const uint32_t* n_pts, int64_t n_items,
+                                    int num_classes, int max_pts, int H, int W, const double* spacing /* HOST [2] */,
+                                    double* max_sq, double* p95_sq, double* sum_dist, double* d2, int keep_d2,
+                                    void* stream);
+
+/* ---------------------------------------------------------------------------------------------
  * All-contour distances (build-defined, no reference counterpart): hausdorff / hd95 / assd over EVERY contour of
  * each class mask instead of contour [0] only -- the whole boundary, as MONAI, medpy and surface-distance measure it.
  * Per (item i, class c, map m) the vertex set is
@@ -269,6 +287,17 @@ OCTM_API int octm_surface_dice_u8(const uint8_t* y_true, const uint8_t* y_pred, 
                                   int num_classes, const uint32_t* thresholds_sq /* HOST array, ascending */,
                                   int n_thresholds, uint32_t* n_surf /* [n][K][2] */,
                                   uint32_t* n_within /* [n][K][2][n_thresholds] */, void* stream);
+/* The same counts with a pixel spacing {sy, sx} (HOST array, as octm_contour2d_distance_spacing) and 1 to
+ * OCTM_SURFACE_DICE_MAX_TOL tolerances (HOST array, any order, in the units of the spacing): a vertex is within tau when
+ * sqrt(q / 4.0) <= tau for q = fl(fl(wy * a^2) + fl(wx * b^2)) of its nearest source vertex.  The library turns each tau
+ * into the exact column reach of every lattice row offset; the reach is limited to 16 lattice rows and 16 lattice columns,
+ * i.e. tau < min(sqrt(fl(wy * 289) / 4.0), sqrt(fl(wx * 289) / 4.0)) (just below 8.5 at {1, 1}); a larger tau returns
+ * OCTM_ERR_INVALID with the largest one allowed in octm_last_error(). */
+OCTM_API int octm_surface_dice_spacing_u8(const uint8_t* y_true, const uint8_t* y_pred, int64_t n_items, int H, int W,
+                                          int num_classes, const double* spacing /* HOST [2] */,
+                                          const double* tolerances /* HOST [n_tolerances] */, int n_tolerances,
+                                          uint32_t* n_surf /* [n][K][2] */,
+                                          uint32_t* n_within /* [n][K][2][n_tolerances] */, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
  * Connected components per class (build-defined, no reference counterpart; scipy.ndimage.label, skimage.measure.label).
@@ -409,6 +438,15 @@ OCTM_API int octm_derive_metrics(const uint64_t* counts, const int64_t* thick_ab
                         const uint32_t* p95_sq, const double* sum_dist, const uint32_t* contour_flags,
                         int64_t n_items, int H, int W, int num_classes, double* class_metrics,
                         double* boundary_metrics, double* totals, void* stream);
+/* octm_derive_metrics with a pixel spacing {sy, sx} (HOST array): max_sq / p95_sq are the float64 squared distances of
+ * octm_contour2d_distance_spacing, and the thickness and boundary errors scale with the row spacing:
+ * thickness (sum / W) * sy, boundary MSE (sum / W) * wy (RMSE its square root), MAD (sum / W) * sy.  The totals are the
+ * same integer sums as without a spacing (a dataset-level mean is scaled by its reader). */
+OCTM_API int octm_derive_metrics_spacing(const uint64_t* counts, const int64_t* thick_absdiff, const int64_t* bnd_sq,
+                        const int64_t* bnd_abs, const uint32_t* n_pts, const double* max_sq,
+                        const double* p95_sq, const double* sum_dist, const uint32_t* contour_flags,
+                        int64_t n_items, int H, int W, int num_classes, const double* spacing /* HOST [2] */,
+                        double* class_metrics, double* boundary_metrics, double* totals, void* stream);
 
 #ifdef __cplusplus
 }

@@ -48,9 +48,11 @@ SIGNATURES = {
     "octm_first_pos_u8": (_INT, [_P, _I64, _I64, _INT, _P, _P]),
     "octm_contour2d_trace_u8": (_INT, [_P, _P, _I64, _INT, _INT, _INT, _P, _P, _P, _INT, _P, _P, _P, _P]),
     "octm_contour2d_distance": (_INT, [_P, _P, _I64, _INT, _INT, _INT, _INT, _P, _P, _P, _P, _INT, _P]),
+    "octm_contour2d_distance_spacing": (_INT, [_P, _P, _I64, _INT, _INT, _INT, _INT, _P, _P, _P, _P, _P, _INT, _P]),
     "octm_contour2d_all_vertices_u8": (_INT, [_P, _P, _I64, _INT, _INT, _INT, _INT, _P, _P, _P, _P]),
     "octm_contour2d_all_u8": (_INT, [_P, _P, _I64, _INT, _INT, _INT, _INT, _P, _P, _P, _P, _P, _P, _c.c_size_t, _P]),
     "octm_surface_dice_u8": (_INT, [_P, _P, _I64, _INT, _INT, _INT, _P, _INT, _P, _P, _P]),
+    "octm_surface_dice_spacing_u8": (_INT, [_P, _P, _I64, _INT, _INT, _INT, _P, _P, _INT, _P, _P, _P]),
     "octm_components_u8": (_INT, [_P, _P, _I64, _INT, _INT, _INT, _INT, _P, _P, _P]),
     "octm_argmax_labels": (_INT, [_P, _INT, _I64, _INT, _I64, _INT, _P, _P]),
     "octm_auc_workspace_bytes": (_c.c_size_t, [_I64, _I64, _INT]),
@@ -68,6 +70,8 @@ SIGNATURES = {
     "octm_totals_len": (_INT, [_INT]),
     "octm_totals_sum_len": (_INT, [_INT]),
     "octm_derive_metrics": (_INT, [_P, _P, _P, _P, _P, _P, _P, _P, _P, _I64, _INT, _INT, _INT, _P, _P, _P, _P]),
+    "octm_derive_metrics_spacing": (_INT, [_P, _P, _P, _P, _P, _P, _P, _P, _P, _I64, _INT, _INT, _INT, _P, _P, _P, _P,
+                                           _P]),
 }
 
 _lib = None

@@ -10,6 +10,9 @@
 //   Metrics/Contour_based_metrics.py:22,39,56,68-71   (numpy linear percentile for hd95)
 // Multiplications that feed an addition use __dmul_rn/__dadd_rn so nvcc cannot contract them
 // into an FMA (numpy rounds after each operation).
+#include <cmath>
+#include <type_traits>
+
 #include "common.cuh"
 
 namespace octm {
@@ -22,17 +25,19 @@ struct DeriveParams {
     const long long* bsq;               // [n][K-1] or null
     const long long* babs;              // [n][K-1] or null
     const uint32_t* n_pts;              // [n][K][2] or null (no contour metrics)
-    const uint32_t* max_sq;             // [n][K][2]
-    const uint32_t* p95_sq;             // [n][K][2][2]
+    const void* max_sq;                 // [n][K][2]     uint32 (pixel units) or float64 (with a spacing)
+    const void* p95_sq;                 // [n][K][2][2]
     const double* sum_dist;             // [n][K][2]
     long long n_items;
     int H, W, K;
     double* cls;                        // [n][K][OCTM_NUM_CLASS_METRICS]
     double* bnd;                        // [n][K-1][3] or null
     double* n_bad;                      // totals slot "n_bad_label_items" (zeroed before the launch) or null
+    double sy, wy;                      // with a spacing: the row (axial) spacing and its square
 };
 
-__device__ __forceinline__ double percentile95(uint32_t lo_sq, uint32_t hi_sq, uint32_t m) {
+template <class SQ>
+__device__ __forceinline__ double percentile95(SQ lo_sq, SQ hi_sq, uint32_t m) {
     const double pos = __dmul_rn(static_cast<double>(m - 1), 0.95);     // numpy: (n - 1) * quantile
     const double gamma = pos - floor(pos);
     const double a = sqrt(static_cast<double>(lo_sq) / 4.0), b = sqrt(static_cast<double>(hi_sq) / 4.0);
@@ -41,7 +46,13 @@ __device__ __forceinline__ double percentile95(uint32_t lo_sq, uint32_t hi_sq, u
     return __dadd_rn(a, __dmul_rn(d, gamma));
 }
 
+// SPACING: float64 squared contour distances (octm_contour2d_distance_spacing) and the thickness and boundary errors
+// scaled by the row spacing: thickness (sum / W) * sy, boundary MSE (sum / W) * wy, MAD (sum / W) * sy.
+template <bool SPACING>
 __global__ void __launch_bounds__(128) derive_kernel(const DeriveParams p) {
+    using SQ = typename std::conditional<SPACING, double, uint32_t>::type;
+    const SQ* max_sq = static_cast<const SQ*>(p.max_sq);
+    const SQ* p95_sq = static_cast<const SQ*>(p.p95_sq);
     const long long gid = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
     const int K = p.K;
     if (gid >= p.n_items * K) return;
@@ -77,15 +88,17 @@ __global__ void __launch_bounds__(128) derive_kernel(const DeriveParams p) {
     o[OCTM_M_RMSE] = sqrt(err);
     o[OCTM_M_MAD] = err;
     o[OCTM_M_VASCULARITY] = fabs(static_cast<double>(st) / n - static_cast<double>(sp) / n);
-    o[OCTM_M_THICKNESS_DIFF] = p.thick ? static_cast<double>(p.thick[gid]) / static_cast<double>(p.W) : nan("");
+    double thick = p.thick ? static_cast<double>(p.thick[gid]) / static_cast<double>(p.W) : nan("");
+    if (SPACING) thick = __dmul_rn(thick, p.sy);
+    o[OCTM_M_THICKNESS_DIFF] = thick;
     double hd = nan(""), hd95 = nan(""), assd = nan("");
     if (p.n_pts != nullptr) {
         const uint32_t nt = p.n_pts[gid * 2 + 0], np = p.n_pts[gid * 2 + 1];
         if (nt > 0 && np > 0) {
             const uint32_t m0 = np, m1 = nt;       // query counts: direction 0 = pred vertices, 1 = true vertices
-            hd = sqrt(static_cast<double>(max(p.max_sq[gid * 2], p.max_sq[gid * 2 + 1])) / 4.0);
-            hd95 = fmax(percentile95(p.p95_sq[gid * 4 + 0], p.p95_sq[gid * 4 + 1], m0),
-                        percentile95(p.p95_sq[gid * 4 + 2], p.p95_sq[gid * 4 + 3], m1));
+            hd = sqrt(static_cast<double>(max(max_sq[gid * 2], max_sq[gid * 2 + 1])) / 4.0);
+            hd95 = fmax(percentile95(p95_sq[gid * 4 + 0], p95_sq[gid * 4 + 1], m0),
+                        percentile95(p95_sq[gid * 4 + 2], p95_sq[gid * 4 + 3], m1));
             assd = __dadd_rn(p.sum_dist[gid * 2] / static_cast<double>(m0), p.sum_dist[gid * 2 + 1] / static_cast<double>(m1)) / 2.0;
         }
     }
@@ -94,10 +107,15 @@ __global__ void __launch_bounds__(128) derive_kernel(const DeriveParams p) {
     o[OCTM_M_ASSD] = assd;
     if (p.bnd != nullptr && p.bsq != nullptr && c < K - 1) {
         const long long b = item * (K - 1) + c;
-        const double mse = static_cast<double>(p.bsq[b]) / static_cast<double>(p.W);
+        double mse = static_cast<double>(p.bsq[b]) / static_cast<double>(p.W);
+        double mad = static_cast<double>(p.babs[b]) / static_cast<double>(p.W);
+        if (SPACING) {
+            mse = __dmul_rn(mse, p.wy);
+            mad = __dmul_rn(mad, p.sy);
+        }
         p.bnd[b * 3 + 0] = mse;
         p.bnd[b * 3 + 1] = sqrt(mse);
-        p.bnd[b * 3 + 2] = static_cast<double>(p.babs[b]) / static_cast<double>(p.W);
+        p.bnd[b * 3 + 2] = mad;
     }
 }
 
@@ -193,11 +211,11 @@ extern "C" int octm_totals_sum_len(int num_classes) {
     return 1 + K * K + K + 2 * (K - 1) + 4 * K + 2;
 }
 
-extern "C" int octm_derive_metrics(const uint64_t* counts, const int64_t* thick_absdiff, const int64_t* bnd_sq,
-                                   const int64_t* bnd_abs, const uint32_t* n_pts, const uint32_t* max_sq,
-                                   const uint32_t* p95_sq, const double* sum_dist, const uint32_t* contour_flags,
-                                   int64_t n_items, int H, int W, int num_classes, double* class_metrics,
-                                   double* boundary_metrics, double* totals, void* stream) {
+static int derive_metrics(const uint64_t* counts, const int64_t* thick_absdiff, const int64_t* bnd_sq, const int64_t* bnd_abs,
+                          const uint32_t* n_pts, const void* max_sq, const void* p95_sq, const double* sum_dist,
+                          const uint32_t* contour_flags, int64_t n_items, int H, int W, int num_classes,
+                          const double* spacing, double* class_metrics, double* boundary_metrics, double* totals,
+                          void* stream) {
     if (n_items < 0 || num_classes < 2 || num_classes > OCTM_MAX_CLASSES || W < 1 || H < 1)
         return octm::fail(OCTM_ERR_INVALID, "bad shape");
     if (n_items > 0 && (!counts || !class_metrics)) return octm::fail(OCTM_ERR_INVALID, "counts and class_metrics are required");
@@ -207,12 +225,15 @@ extern "C" int octm_derive_metrics(const uint64_t* counts, const int64_t* thick_
     octm::DeriveParams p{reinterpret_cast<const unsigned long long*>(counts), reinterpret_cast<const long long*>(thick_absdiff),
                          reinterpret_cast<const long long*>(bnd_sq), reinterpret_cast<const long long*>(bnd_abs), n_pts, max_sq,
                          p95_sq, sum_dist, n_items, H, W, num_classes, class_metrics, boundary_metrics,
-                         totals ? totals + (octm_totals_sum_len(num_classes) - 1) : nullptr};
+                         totals ? totals + (octm_totals_sum_len(num_classes) - 1) : nullptr,
+                         spacing ? spacing[0] : 1.0, spacing ? spacing[0] * spacing[0] : 1.0};
     if (totals != nullptr && cudaMemsetAsync(p.n_bad, 0, sizeof(double), s) != cudaSuccess)
         return octm::fail(OCTM_ERR_LAUNCH, "memset(totals) failed");
     const long long threads = n_items * num_classes;
     if (n_items > 0) {
-        OCTM_TIMED("derive_kernel", s) octm::derive_kernel<<<static_cast<unsigned>((threads + 127) / 128), 128, 0, s>>>(p);
+        const unsigned grid = static_cast<unsigned>((threads + 127) / 128);
+        if (spacing) OCTM_TIMED("derive_kernel", s) octm::derive_kernel<true><<<grid, 128, 0, s>>>(p);
+        else OCTM_TIMED("derive_kernel", s) octm::derive_kernel<false><<<grid, 128, 0, s>>>(p);
         if (int e = octm::check_launch("derive_kernel")) return e;
     }
     if (totals != nullptr) {       // also for an empty batch: n_items 0, sums 0, maxima -1, flags 0
@@ -221,4 +242,26 @@ extern "C" int octm_derive_metrics(const uint64_t* counts, const int64_t* thick_
         if (int e = octm::check_launch("totals_kernel")) return e;
     }
     return OCTM_OK;
+}
+
+extern "C" int octm_derive_metrics(const uint64_t* counts, const int64_t* thick_absdiff, const int64_t* bnd_sq,
+                                   const int64_t* bnd_abs, const uint32_t* n_pts, const uint32_t* max_sq,
+                                   const uint32_t* p95_sq, const double* sum_dist, const uint32_t* contour_flags,
+                                   int64_t n_items, int H, int W, int num_classes, double* class_metrics,
+                                   double* boundary_metrics, double* totals, void* stream) {
+    return derive_metrics(counts, thick_absdiff, bnd_sq, bnd_abs, n_pts, max_sq, p95_sq, sum_dist, contour_flags, n_items,
+                          H, W, num_classes, nullptr, class_metrics, boundary_metrics, totals, stream);
+}
+
+extern "C" int octm_derive_metrics_spacing(const uint64_t* counts, const int64_t* thick_absdiff, const int64_t* bnd_sq,
+                                           const int64_t* bnd_abs, const uint32_t* n_pts, const double* max_sq,
+                                           const double* p95_sq, const double* sum_dist, const uint32_t* contour_flags,
+                                           int64_t n_items, int H, int W, int num_classes, const double* spacing,
+                                           double* class_metrics, double* boundary_metrics, double* totals, void* stream) {
+    if (spacing == nullptr) return octm::fail(OCTM_ERR_INVALID, "null pointer: spacing");
+    for (int a = 0; a < 2; ++a)
+        if (!std::isfinite(spacing[a]) || !(spacing[a] > 0.0) || !std::isnormal(spacing[a] * spacing[a]))
+            return octm::fail(OCTM_ERR_INVALID, "spacing[%d] = %g: must be finite and > 0 with a normal square", a, spacing[a]);
+    return derive_metrics(counts, thick_absdiff, bnd_sq, bnd_abs, n_pts, max_sq, p95_sq, sum_dist, contour_flags, n_items,
+                          H, W, num_classes, spacing, class_metrics, boundary_metrics, totals, stream);
 }

@@ -18,6 +18,11 @@
 // vertical-crack query meets a horizontal-crack row at dx = 2d + 1, d in [-(r + 1) / 2, (r - 1) / 2] (d = x' - x in
 // image columns).  T <= 256 (tau <= 8 px) gives R <= 16 lattice rows and |d| <= 8 columns.
 //
+// With a pixel spacing (octm_surface_dice_spacing_u8) "within tau" is sqrt(q / 4.0) <= tau for
+// q = fl(fl(wy dy^2) + fl(wx dx^2)), wy = sy^2, wx = sx^2; q grows with |dy| and with |dx|, so r(dy) = the largest |dx|
+// within tau is found exactly by a short scan on the host.  The windows are then the same: rows with r(dy) >= 0, columns
+// |dx| <= r(dy), both limited to 16 lattice offsets.  The host turns every r into the shift codes below.
+//
 //   surface_dice_kernel  one CTA of kSdWarps warps per (item, class group); an iteration handles kSdWarps image rows.
 //                        A lane owns 16 columns and, per class and map, one crack word (crack_masks.cuh: 16 horizontal |
 //                        16 vertical crack bits).  Shared memory holds a ring of these words for both maps: the
@@ -27,6 +32,9 @@
 //                        threshold with two shifted ORs of a power-of-two run mask, ORs the hits of the query bits,
 //                        and finally popc + warp sum + one shared atomic per (class, direction, threshold).  A warp
 //                        whose query words of a class are all zero skips the class (the common case on layers).
+#include <algorithm>
+#include <cmath>
+
 #include "crack_masks.cuh"
 
 namespace octm {
@@ -42,8 +50,8 @@ struct SurfaceDiceParams {
     int H, W, K;
     int group, n_groups;  // classes per CTA, class groups per item
     int n_thr;
-    uint32_t thr[OCTM_SURFACE_DICE_MAX_TOL];   // ascending
-    int reach;            // R = floor(sqrt(thr[n_thr - 1])) lattice rows
+    uint32_t code[2][kSdMaxReach + 1][OCTM_SURFACE_DICE_MAX_TOL];   // range_code of (query row type, |dy|, threshold)
+    int reach;            // R: the largest |dy| with a source column within reach of some threshold
     int halo;             // ceil(R / 2) image rows
     int slots;            // ring rows: kSdWarps + 2 * halo
     int nw;               // crack words per row: 32 per 512-column segment
@@ -51,20 +59,21 @@ struct SurfaceDiceParams {
     uint32_t* n_within;   // [n][K][2][n_thr]
 };
 
-__device__ __forceinline__ int isqrt_small(int v) {      // floor(sqrt(v)), 0 <= v <= 256
-    int r = static_cast<int>(sqrtf(static_cast<float>(v)));
+// floor(sqrt(v)), 0 <= v <= 256
+static int isqrt_small(int v) {
+    int r = static_cast<int>(std::sqrt(static_cast<float>(v)));
     while (r * r > v) --r;
     while ((r + 1) * (r + 1) <= v) ++r;
     return r;
 }
 
-// Shift code of (query row type qt, |dy|, threshold j): the dilation by columns [lo, hi] of a source row is
+// Shift code of (query row type qt, |dy| = a, column reach r): the source columns of lattice row offset a within reach
+// are |dx| <= r (r < 0: none).  The dilation by columns [lo, hi] of a source row is
 // (x_p >> (16 + lo)) | (x_p >> (16 + hi - p + 1)), x_p the run-of-p mask of the 48-bit window, p = 2^psel the largest
 // power of two <= hi - lo + 1.  Code = sh1 | sh2 << 8 | psel << 16 | 1 << 24; 0 = no source column within reach.
-__device__ uint32_t range_code(int qt, int a, uint32_t T) {
-    const int a2 = a * a;
-    if (static_cast<uint32_t>(a2) > T) return 0u;
-    const int r = isqrt_small(static_cast<int>(T) - a2);
+// Built on the host: r comes from the integer threshold (r = isqrt(T - a^2)) or from a pixel spacing.
+static uint32_t range_code(int qt, int a, int r) {
+    if (r < 0) return 0u;
     int lo, hi;
     if ((a & 1) == 0) {                 // same row type: dx = 2d
         lo = -(r >> 1);
@@ -75,13 +84,13 @@ __device__ uint32_t range_code(int qt, int a, uint32_t T) {
         hi = qt == 0 ? (r + 1) >> 1 : (r - 1) >> 1;
     }
     const int len = hi - lo + 1;
-    const int psel = 31 - __clz(len);
+    const int psel = 31 - __builtin_clz(static_cast<unsigned>(len));
     return static_cast<uint32_t>(16 + lo) | static_cast<uint32_t>(16 + hi - (1 << psel) + 1) << 8 |
            static_cast<uint32_t>(psel) << 16 | 1u << 24;
 }
 
 template <bool VEC>
-__global__ void __launch_bounds__(kSdWarps * 32) surface_dice_kernel(const SurfaceDiceParams p) {
+__global__ void __launch_bounds__(kSdWarps * 32) surface_dice_kernel(const __grid_constant__ SurfaceDiceParams p) {
     extern __shared__ uint32_t ring[];   // [slots][2 maps][group][nw + 2]: one zero pad word at each end of a row
     __shared__ uint32_t s_code[2][kSdMaxReach + 1][OCTM_SURFACE_DICE_MAX_TOL];
     __shared__ uint32_t s_within[OCTM_MAX_CLASSES][2][OCTM_SURFACE_DICE_MAX_TOL];
@@ -90,12 +99,8 @@ __global__ void __launch_bounds__(kSdWarps * 32) surface_dice_kernel(const Surfa
     const int H = p.H, W = p.W, K = p.K, G = p.group, n_thr = p.n_thr, R = p.reach;
     const int stride = p.nw + 2;
     const int nseg = (W + kSdSeg - 1) / kSdSeg;
-    for (int e = tid; e < 2 * (kSdMaxReach + 1) * OCTM_SURFACE_DICE_MAX_TOL; e += blockDim.x) {
-        const int j = e % OCTM_SURFACE_DICE_MAX_TOL, a = (e / OCTM_SURFACE_DICE_MAX_TOL) % (kSdMaxReach + 1);
-        const int qt = e / (OCTM_SURFACE_DICE_MAX_TOL * (kSdMaxReach + 1));
-        const uint32_t T = j == 0 ? p.thr[0] : j == 1 ? p.thr[1] : j == 2 ? p.thr[2] : p.thr[3];   // no local copy of p
-        s_code[qt][a][j] = j < n_thr ? range_code(qt, a, T) : 0u;
-    }
+    for (int e = tid; e < 2 * (kSdMaxReach + 1) * OCTM_SURFACE_DICE_MAX_TOL; e += blockDim.x)
+        (&s_code[0][0][0])[e] = (&p.code[0][0][0])[e];
     for (int e = tid; e < p.slots * 2 * G * stride; e += blockDim.x) ring[e] = 0u;    // the pad words stay zero
     for (int e = tid; e < OCTM_MAX_CLASSES * 2 * OCTM_SURFACE_DICE_MAX_TOL; e += blockDim.x) (&s_within[0][0][0])[e] = 0u;
     if (tid < OCTM_MAX_CLASSES * 2) (&s_surf[0][0])[tid] = 0u;
@@ -206,25 +211,20 @@ __global__ void __launch_bounds__(kSdWarps * 32) surface_dice_kernel(const Surfa
 }  // namespace octm
 
 // ----------------------------------------------------------------------------------- C ABI
-extern "C" int octm_surface_dice_u8(const uint8_t* y_true, const uint8_t* y_pred, int64_t n_items, int H, int W,
-                                    int num_classes, const uint32_t* thresholds_sq, int n_thresholds, uint32_t* n_surf,
-                                    uint32_t* n_within, void* stream) {
-    if (int e = octm::check_shape(n_items, H, W, num_classes, 8)) return e;    // no vertex bound: 8 passes that check
-    if (thresholds_sq == nullptr) return octm::fail(OCTM_ERR_INVALID, "null pointer: thresholds_sq");
-    if (n_thresholds < 1 || n_thresholds > OCTM_SURFACE_DICE_MAX_TOL)
-        return octm::fail(OCTM_ERR_INVALID, "n_thresholds %d outside [1, %d]", n_thresholds, OCTM_SURFACE_DICE_MAX_TOL);
-    octm::SurfaceDiceParams p{};
-    for (int j = 0; j < n_thresholds; ++j) {
-        const uint32_t t = thresholds_sq[j];
-        if (t > OCTM_SURFACE_DICE_MAX_SQ)
-            return octm::fail(OCTM_ERR_INVALID, "thresholds_sq[%d] = %u > %d", j, t, OCTM_SURFACE_DICE_MAX_SQ);
-        if (j > 0 && t < thresholds_sq[j - 1]) return octm::fail(OCTM_ERR_INVALID, "thresholds_sq not ascending");
-        p.thr[j] = t;
-    }
+// Both entry points: reach[j][a] = the largest lattice column offset |dx| within threshold j at lattice row offset a
+// (-1: none), a = 0 .. kSdMaxReach.  Everything but the table is the same.
+static int launch_surface_dice(const uint8_t* y_true, const uint8_t* y_pred, int64_t n_items, int H, int W,
+                               int num_classes, const int (*reach_col)[octm::kSdMaxReach + 1], int n_thresholds,
+                               uint32_t* n_surf, uint32_t* n_within, void* stream) {
     if (n_items == 0) return OCTM_OK;
     if (!y_true || !y_pred || !n_surf || !n_within) return octm::fail(OCTM_ERR_INVALID, "null pointer");
+    octm::SurfaceDiceParams p{};
     int reach = 0;
-    while ((reach + 1) * (reach + 1) <= static_cast<int>(p.thr[n_thresholds - 1])) ++reach;
+    for (int j = 0; j < n_thresholds; ++j)
+        for (int a = 0; a <= octm::kSdMaxReach; ++a) {
+            if (reach_col[j][a] >= 0 && a > reach) reach = a;
+            for (int qt = 0; qt < 2; ++qt) p.code[qt][a][j] = octm::range_code(qt, a, reach_col[j][a]);
+        }
     const int halo = (reach + 1) / 2, slots = octm::kSdWarps + 2 * halo;
     const int nw = (W + octm::kSdSeg - 1) / octm::kSdSeg * 32;
     const size_t per_class = static_cast<size_t>(slots) * 2 * (nw + 2) * sizeof(uint32_t);
@@ -258,4 +258,63 @@ extern "C" int octm_surface_dice_u8(const uint8_t* y_true, const uint8_t* y_pred
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     OCTM_TIMED("surface_dice_kernel", s) kern<<<grid, octm::kSdWarps * 32, smem, s>>>(p);
     return octm::check_launch("surface_dice_kernel");
+}
+
+extern "C" int octm_surface_dice_u8(const uint8_t* y_true, const uint8_t* y_pred, int64_t n_items, int H, int W,
+                                    int num_classes, const uint32_t* thresholds_sq, int n_thresholds, uint32_t* n_surf,
+                                    uint32_t* n_within, void* stream) {
+    if (int e = octm::check_shape(n_items, H, W, num_classes, 8)) return e;    // no vertex bound: 8 passes that check
+    if (thresholds_sq == nullptr) return octm::fail(OCTM_ERR_INVALID, "null pointer: thresholds_sq");
+    if (n_thresholds < 1 || n_thresholds > OCTM_SURFACE_DICE_MAX_TOL)
+        return octm::fail(OCTM_ERR_INVALID, "n_thresholds %d outside [1, %d]", n_thresholds, OCTM_SURFACE_DICE_MAX_TOL);
+    int reach_col[OCTM_SURFACE_DICE_MAX_TOL][octm::kSdMaxReach + 1];
+    for (int j = 0; j < n_thresholds; ++j) {
+        const uint32_t t = thresholds_sq[j];
+        if (t > OCTM_SURFACE_DICE_MAX_SQ)
+            return octm::fail(OCTM_ERR_INVALID, "thresholds_sq[%d] = %u > %d", j, t, OCTM_SURFACE_DICE_MAX_SQ);
+        if (j > 0 && t < thresholds_sq[j - 1]) return octm::fail(OCTM_ERR_INVALID, "thresholds_sq not ascending");
+        for (int a = 0; a <= octm::kSdMaxReach; ++a)       // dy^2 + dx^2 <= T  <=>  |dx| <= isqrt(T - dy^2)
+            reach_col[j][a] = static_cast<uint32_t>(a * a) > t ? -1 : octm::isqrt_small(static_cast<int>(t) - a * a);
+    }
+    return launch_surface_dice(y_true, y_pred, n_items, H, W, num_classes, reach_col, n_thresholds, n_surf, n_within, stream);
+}
+
+extern "C" int octm_surface_dice_spacing_u8(const uint8_t* y_true, const uint8_t* y_pred, int64_t n_items, int H, int W,
+                                            int num_classes, const double* spacing, const double* tolerances,
+                                            int n_tolerances, uint32_t* n_surf, uint32_t* n_within, void* stream) {
+    if (int e = octm::check_shape(n_items, H, W, num_classes, 8)) return e;
+    if (spacing == nullptr || tolerances == nullptr) return octm::fail(OCTM_ERR_INVALID, "null pointer: spacing / tolerances");
+    for (int a = 0; a < 2; ++a)
+        if (!std::isfinite(spacing[a]) || !(spacing[a] > 0.0))
+            return octm::fail(OCTM_ERR_INVALID, "spacing[%d] = %g: must be finite and > 0", a, spacing[a]);
+    const double wy = spacing[0] * spacing[0], wx = spacing[1] * spacing[1];
+    for (int a = 0; a < 2; ++a)
+        if (!std::isnormal(a == 0 ? wy : wx))
+            return octm::fail(OCTM_ERR_INVALID, "spacing[%d] = %g: its square is not a normal double", a, spacing[a]);
+    if (n_tolerances < 1 || n_tolerances > OCTM_SURFACE_DICE_MAX_TOL)
+        return octm::fail(OCTM_ERR_INVALID, "n_tolerances %d outside [1, %d]", n_tolerances, OCTM_SURFACE_DICE_MAX_TOL);
+    // q(a, b) = fl(fl(wy a^2) + fl(wx b^2)) is within tau when sqrt(q / 4.0) <= tau: monotone in |a| and in |b|
+    auto within = [&](int a, int b, double tau) {
+        const double q = wy * static_cast<double>(a * a) + wx * static_cast<double>(b * b);
+        return std::sqrt(q / 4.0) <= tau;
+    };
+    constexpr int kOut = octm::kSdMaxReach + 1;                // the first lattice offset beyond the kernel's window
+    const double limit = std::min(std::sqrt(wy * (kOut * kOut) / 4.0), std::sqrt(wx * (kOut * kOut) / 4.0));
+    int reach_col[OCTM_SURFACE_DICE_MAX_TOL][octm::kSdMaxReach + 1];
+    for (int j = 0; j < n_tolerances; ++j) {
+        const double tau = tolerances[j];
+        if (!std::isfinite(tau) || !(tau >= 0.0))
+            return octm::fail(OCTM_ERR_INVALID, "tolerances[%d] = %g: must be finite and >= 0", j, tau);
+        if (!(tau < limit))
+            return octm::fail(OCTM_ERR_INVALID,
+                              "tolerances[%d] = %.17g reaches beyond %d lattice rows or columns at spacing (%g, %g): the "
+                              "largest tolerance allowed is %.17g", j, tau, octm::kSdMaxReach, spacing[0], spacing[1],
+                              std::nextafter(limit, 0.0));
+        for (int a = 0; a <= octm::kSdMaxReach; ++a) {
+            int r = -1;
+            while (r < octm::kSdMaxReach && within(a, r + 1, tau)) ++r;
+            reach_col[j][a] = r;
+        }
+    }
+    return launch_surface_dice(y_true, y_pred, n_items, H, W, num_classes, reach_col, n_tolerances, n_surf, n_within, stream);
 }

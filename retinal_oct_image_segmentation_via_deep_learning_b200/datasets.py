@@ -246,11 +246,32 @@ def read_labels(path, key=None):
     return np.ascontiguousarray(arr)
 
 
-def evaluate_files(true_path, pred_path, num_classes, **kwargs):
+def header_spacing_2d(true_path):
+    """The B-scan pixel spacing ``(rows, cols)`` of a MetaImage label file: the last two axes of ``mhd_spacing``.
+    ValueError for other formats and for a header without ``ElementSpacing``."""
+    if os.path.splitext(true_path)[1].lower() != ".mhd":
+        raise ValueError(f"{true_path}: spacing='header' needs a MetaImage (.mhd) file with ElementSpacing")
+    _, header = read_mhd(true_path)
+    try:
+        sp = mhd_spacing(header)
+    except KeyError:
+        raise ValueError(f"{true_path}: the MetaImage header has no ElementSpacing") from None
+    if len(sp) < 2:
+        raise ValueError(f"{true_path}: ElementSpacing has {len(sp)} entry, a B-scan needs rows and columns")
+    return sp[-2:]
+
+
+def evaluate_files(true_path, pred_path, num_classes, *, spacing=None, **kwargs):
     """Score one predicted label volume against its ground truth, both on disk: reads the two files and runs
-    ``suite.evaluate_host`` (chunked, copy/compute overlapped).  Keyword arguments go to ``evaluate_host``."""
+    ``suite.evaluate_host`` (chunked, copy/compute overlapped).  Keyword arguments go to ``evaluate_host``.
+    ``spacing``: None (pixel units), ``(rows, cols)``, or ``"header"``: the ground truth's MetaImage ``ElementSpacing``
+    (``header_spacing_2d``; ValueError for formats without one)."""
     from . import suite
+    if isinstance(spacing, str):
+        if spacing != "header":
+            raise ValueError(f"spacing must be None, (rows, cols) or 'header', got {spacing!r}")
+        spacing = header_spacing_2d(true_path)
     yt, yp = read_labels(true_path), read_labels(pred_path)
     if yt.shape != yp.shape:
         raise ValueError(f"shape mismatch: {yt.shape} vs {yp.shape}")
-    return suite.evaluate_host(yt, yp, num_classes, **kwargs)
+    return suite.evaluate_host(yt, yp, num_classes, spacing=spacing, **kwargs)

@@ -56,17 +56,23 @@ def count_metrics(tp, fp, fn, tn, n):
         }
 
 
-def thickness_difference(thick_absdiff, width):
-    """Biomarker_based_metrics.py:18-21 -- mean over the W columns of |thickness_t - thickness_p|."""
-    return np.asarray(thick_absdiff, dtype=np.int64).astype(np.float64) / width
+def thickness_difference(thick_absdiff, width, spacing=None):
+    """Biomarker_based_metrics.py:18-21 -- mean over the W columns of |thickness_t - thickness_p|; with a pixel
+    ``spacing=(sy, sx)`` in the units of the row spacing: ``(sum / W) * sy``."""
+    out = np.asarray(thick_absdiff, dtype=np.int64).astype(np.float64) / width
+    return out if spacing is None else out * np.float64(spacing[0])
 
 
-def boundary_errors(sum_sq, sum_abs, width):
+def boundary_errors(sum_sq, sum_abs, width, spacing=None):
     """MSE / RMSE / MAD of boundary-position rows (PixelError_based_metrics.py:14-17, 32-35;
-    Contour_based_metrics.py:68-71 applied to integer boundary arrays of W columns)."""
+    Contour_based_metrics.py:68-71 applied to integer boundary arrays of W columns).  With a pixel ``spacing=(sy, sx)``
+    the positions are in the units of the row spacing: MSE ``(sum / W) * sy**2``, MAD ``(sum / W) * sy``."""
     mse = np.asarray(sum_sq, dtype=np.int64).astype(np.float64) / width
-    return {"boundary_mse": mse, "boundary_rmse": np.sqrt(mse),
-            "boundary_mad": np.asarray(sum_abs, dtype=np.int64).astype(np.float64) / width}
+    mad = np.asarray(sum_abs, dtype=np.int64).astype(np.float64) / width
+    if spacing is not None:
+        sy = np.float64(spacing[0])
+        mse, mad = mse * (sy * sy), mad * sy
+    return {"boundary_mse": mse, "boundary_rmse": np.sqrt(mse), "boundary_mad": mad}
 
 
 def _lerp(a, b, t):
@@ -141,6 +147,57 @@ def surface_dice_tolerances(tolerances):
             raise ValueError(f"surface_dice tolerance {t!r} is not a number") from None
         if not 0.0 <= v <= SURFACE_DICE_MAX_TAU:          # False for NaN
             raise ValueError(f"surface_dice tolerance {v} outside [0, {SURFACE_DICE_MAX_TAU}] pixels")
+        out.append(v)
+    return tuple(out)
+
+
+SURFACE_DICE_MAX_REACH = 16      # lattice rows and lattice columns the surface Dice kernel reaches
+
+
+def spacing_2d(spacing):
+    """A B-scan pixel spacing ``(sy, sx)`` (rows = axial, columns = lateral; e.g. ``datasets.mhd_spacing(hdr)[-2:]``) ->
+    tuple of 2 floats, or None for None.  ValueError unless both are finite and > 0 with squares that are normal doubles
+    (the kernels work with ``wy = sy * sy`` and ``wx = sx * sx``)."""
+    if spacing is None:
+        return None
+    try:
+        sp = tuple(float(v) for v in np.asarray(spacing, dtype=np.float64).reshape(-1))
+    except (TypeError, ValueError):
+        raise ValueError(f"spacing must be 2 numbers (rows, columns), got {spacing!r}") from None
+    if len(sp) != 2 or not all(np.isfinite(v) and v > 0 for v in sp):
+        raise ValueError(f"spacing must be 2 finite numbers > 0 (rows, columns), got {spacing!r}")
+    if not all(np.isfinite(v * v) and v * v >= np.finfo(np.float64).tiny for v in sp):
+        raise ValueError(f"spacing {spacing!r}: the square of each entry must be a normal double")
+    return sp
+
+
+def surface_dice_spacing_limit(spacing):
+    """The largest tolerance ``surface_dice`` accepts at pixel spacing ``(sy, sx)``: the kernel reaches 16 lattice rows and
+    16 lattice columns, so tau must stay below ``sqrt(fl(w * 17**2) / 4.0)`` for ``w = sy**2`` and ``w = sx**2``."""
+    sy, sx = spacing_2d(spacing)
+    out = SURFACE_DICE_MAX_REACH + 1
+    limit = min(np.sqrt(sy * sy * (out * out) / 4.0), np.sqrt(sx * sx * (out * out) / 4.0))
+    return float(np.nextafter(limit, 0.0))
+
+
+def surface_dice_spacing_tolerances(tolerances, spacing):
+    """``surface_dice_tolerances`` with a pixel spacing: 1 to 4 finite tolerances ``>= 0`` in the units of the spacing, each
+    at most ``surface_dice_spacing_limit(spacing)`` (ValueError naming that limit otherwise)."""
+    taus = (tolerances,) if np.ndim(tolerances) == 0 else tuple(tolerances)
+    if not 1 <= len(taus) <= SURFACE_DICE_MAX_TOL:
+        raise ValueError(f"surface_dice takes 1 to {SURFACE_DICE_MAX_TOL} tolerances, got {len(taus)}")
+    limit = surface_dice_spacing_limit(spacing)
+    out = []
+    for t in taus:
+        try:
+            v = float(t)
+        except (TypeError, ValueError):
+            raise ValueError(f"surface_dice tolerance {t!r} is not a number") from None
+        if not 0.0 <= v < np.inf:
+            raise ValueError(f"surface_dice tolerance {v} must be finite and >= 0")
+        if v > limit:
+            raise ValueError(f"surface_dice tolerance {v} reaches beyond {SURFACE_DICE_MAX_REACH} lattice rows or columns "
+                             f"at spacing {tuple(spacing)}: the largest tolerance allowed is {limit!r}")
         out.append(v)
     return tuple(out)
 

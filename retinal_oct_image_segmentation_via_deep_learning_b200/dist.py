@@ -61,7 +61,10 @@ def _check_exact(vec, k):
         raise OverflowError("an integer partial exceeds 2**53 and would not be exact in the float64 all-reduce")
 
 
-def unpack(vec, num_classes, width):
+def unpack(vec, num_classes, width, spacing=None):
+    """The summed totals vector -> dataset-level numbers.  With the pixel ``spacing=(sy, sx)`` of the result the
+    thickness and boundary means are in the units of the row spacing, as the per-item ones: thickness and MAD times
+    ``sy``, MSE times ``sy**2``."""
     k = num_classes
     o = 0
 
@@ -84,8 +87,13 @@ def unpack(vec, num_classes, width):
     denom = max(n_items, 1) * width
     out["thickness_difference"] = thick.astype(np.float64) / denom       # mean over all columns of all items
     out["boundary_mse"] = bsq.astype(np.float64) / denom
-    out["boundary_rmse"] = np.sqrt(out["boundary_mse"])
     out["boundary_mad"] = bab.astype(np.float64) / denom
+    if spacing is not None:
+        sy = np.float64(spacing[0])
+        out["thickness_difference"] = out["thickness_difference"] * sy
+        out["boundary_mse"] = out["boundary_mse"] * (sy * sy)
+        out["boundary_mad"] = out["boundary_mad"] * sy
+    out["boundary_rmse"] = np.sqrt(out["boundary_mse"])
     with np.errstate(invalid="ignore", divide="ignore"):
         out["hausdorff_distance_mean"] = s_hd / nvalid
         out["hausdorff_distance_95_mean"] = s_hd95 / nvalid
@@ -149,7 +157,7 @@ def _finish(res, world, group, want_max, local, reduced):
     if res._totals_host is None:
         res._totals_host, res._final, res._inputs = vec_local, True, None
     _check_exact(vec_local, k)
-    out = unpack(vec[:nb], k, w)
+    out = unpack(vec[:nb], k, w, getattr(res, "spacing", None))      # results without the attribute are in pixels
     if want_max:
         out["hausdorff_distance_max"] = np.where(vec[nb:nb + k] < 0, np.nan, vec[nb:nb + k])
     return out

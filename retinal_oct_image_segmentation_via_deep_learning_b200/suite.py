@@ -235,13 +235,14 @@ class ContourOut:
     """Exact integers (and the float64 distance sums) of the contour kernels, device tensors."""
     n_pts: torch.Tensor        # [N, K, 2]   uint32 bits
     flags: torch.Tensor        # [N, K]
-    max_sq: torch.Tensor       # [N, K, 2]
+    max_sq: torch.Tensor       # [N, K, 2]      uint32 bits; float64 squared distances with a spacing
     p95_sq: torch.Tensor       # [N, K, 2, 2]
     sum_dist: torch.Tensor     # [N, K, 2]   float64
     verts: torch.Tensor | None = None     # [N, K, 2, max_pts] when requested
     sq: torch.Tensor | None = None        # [N, K, 2, max_pts] when requested
     max_pts: int = 0
     mode: str = "first"                   # "first": contour [0] only; "all": every contour of each class
+    spacing: tuple | None = None          # (sy, sx) pixel spacing of the distances, None: pixel units
 
 
 _SCRATCH = {}      # (device, stream) -> grow-only int32 scratch for contour vertices (pure workspace, never returned)
@@ -275,16 +276,28 @@ def _vertex_scratch(dev, numel):
     return buf[:numel]
 
 
-def _contour_outputs(n, k, dev):
-    """Empty ``n_pts``, ``flags``, ``max_sq``, ``p95_sq``, ``sum_dist`` of ``n`` items (the ``ContourOut`` order)."""
+def _contour_outputs(n, k, dev, spacing=None):
+    """Empty ``n_pts``, ``flags``, ``max_sq``, ``p95_sq``, ``sum_dist`` of ``n`` items (the ``ContourOut`` order); the
+    squared distances are float64 with a spacing."""
     i32 = dict(dtype=torch.int32, device=dev)
-    return (torch.empty((n, k, 2), **i32), torch.empty((n, k), **i32), torch.empty((n, k, 2), **i32),
-            torch.empty((n, k, 2, 2), **i32), torch.empty((n, k, 2), dtype=torch.float64, device=dev))
+    sq = dict(dtype=torch.int32 if spacing is None else torch.float64, device=dev)
+    return (torch.empty((n, k, 2), **i32), torch.empty((n, k), **i32), torch.empty((n, k, 2), **sq),
+            torch.empty((n, k, 2, 2), **sq), torch.empty((n, k, 2), dtype=torch.float64, device=dev))
 
 
-def _contour_chunk(yt, yp, k, max_pts, mode, want_verts, want_sq, timers=None, first_pos=None, bnd=None, unsorted=None):
+def _vertex_bytes(spacing):
+    """Scratch bytes per vertex slot of the contour stage: the packed vertex and its squared distance (int32, or float64
+    with a spacing)."""
+    return 4 + (4 if spacing is None else 8)
+
+
+def _contour_chunk(yt, yp, k, max_pts, mode, want_verts, want_sq, timers=None, first_pos=None, bnd=None, unsorted=None,
+                   spacing=None):
     """One chunk of ``contour_pass``.  Metrics alone take the one-call entry point of ``mode`` on the shared scratch;
-    requested vertices or squared distances take the vertex emitter of ``mode``, then ``octm_contour2d_distance``."""
+    requested vertices or squared distances take the vertex emitter of ``mode``, then ``octm_contour2d_distance``.
+    A spacing always takes the vertex emitter, then ``octm_contour2d_distance_spacing``."""
+    if spacing is not None:
+        return _contour_chunk_spacing(yt, yp, k, max_pts, mode, want_verts, want_sq, timers, first_pos, bnd, spacing)
     n, h, w = yt.shape
     dev = yt.device
     n_pts, flags, max_sq, p95, sums = _contour_outputs(n, k, dev)
@@ -318,8 +331,42 @@ def _contour_chunk(yt, yp, k, max_pts, mode, want_verts, want_sq, timers=None, f
                       mode)
 
 
+def _contour_chunk_spacing(yt, yp, k, max_pts, mode, want_verts, want_sq, timers, first_pos, bnd, spacing):
+    """The vertex emitter of ``mode`` (the same vertices as without a spacing), then the float64 nearest-vertex search
+    ``octm_contour2d_distance_spacing``.  Without requested outputs the vertices and distances live in the shared
+    scratch.  Contour [0] is always walked, not verified from the boundary rows ``bnd``: the walk emits the same
+    vertices in the same order in the overflow retry, so ``sum_dist``, a float64 sum in vertex order, does not depend
+    on ``max_pts``."""
+    n, h, w = yt.shape
+    dev = yt.device
+    n_pts, flags, max_sq, p95, sums = _contour_outputs(n, k, dev, spacing)
+    bt = bp = None
+    slots = n * k * 2 * max_pts
+    if want_verts or want_sq:
+        verts = torch.empty((n, k, 2, max_pts), dtype=torch.int32, device=dev)
+        sq = torch.empty((n, k, 2, max_pts), dtype=torch.float64, device=dev)
+    else:
+        scratch = _vertex_scratch(dev, slots * 3)            # int32 words: vertices, then float64 distances
+        verts = scratch[:slots].view(n, k, 2, max_pts)
+        sq = scratch[slots:].view(torch.float64).view(n, k, 2, max_pts)
+    with _Timed(timers, "contour_trace"):
+        if mode == "first":
+            _lib.call("octm_contour2d_trace_u8", _ptr(yt), _ptr(yp), n, h, w, k, _ptr(first_pos), _ptr(bt), _ptr(bp),
+                      max_pts, _ptr(verts), _ptr(n_pts), _ptr(flags), _stream())
+        else:
+            _lib.call("octm_contour2d_all_vertices_u8", _ptr(yt), _ptr(yp), n, h, w, k, max_pts, _ptr(verts),
+                      _ptr(n_pts), _ptr(flags), _stream())
+    sp = (ctypes.c_double * 2)(*spacing)
+    with _Timed(timers, "contour_distance"):
+        _lib.call("octm_contour2d_distance_spacing", _ptr(verts), _ptr(n_pts), n, k, max_pts, h, w, ctypes.addressof(sp),
+                  _ptr(max_sq), _ptr(p95), _ptr(sums), _ptr(sq), 1 if want_sq else 0, _stream())
+    return ContourOut(n_pts, flags, max_sq, p95, sums, verts if want_verts else None, sq if want_sq else None, max_pts,
+                      mode, spacing)
+
+
 def contour_pass(y_true, y_pred, num_classes, first_pos=None, *, max_pts=None, return_vertices=False,
-                 return_sq=False, timers=None, check_overflow=True, boundaries=None, unsorted=None, mode="first"):
+                 return_sq=False, timers=None, check_overflow=True, boundaries=None, unsorted=None, mode="first",
+                 spacing=None):
     """Contour ``[0]`` of every class mask of both maps, then hausdorff / hd95 / assd integers.
 
     ``mode="all"`` measures EVERY contour of each class instead (build-defined, no reference counterpart): the vertex
@@ -333,10 +380,16 @@ def contour_pass(y_true, y_pred, num_classes, first_pos=None, *, max_pts=None, r
     ``unsorted``: optional layering certificate ``[N]`` of ``label_pass(certify=True)``; with it (and the boundary
     rows) certified items are verified and measured from the boundary rows alone.
 
+    ``spacing=(sy, sx)``: pixel size along rows (axial) and columns (lateral), in any unit.  The same vertices are then
+    measured by ``octm_contour2d_distance_spacing``: a vertex pair at lattice offset (a, b) is
+    ``q = fl(fl(sy**2 * a**2) + fl(sx**2 * b**2))`` and its distance ``sqrt(q / 4.0)`` in the units of the spacing;
+    ``max_sq``, ``p95_sq`` (and ``sq``) are float64 ``q`` values.  Neither the layered fast path nor the counters run.
+
     Items are processed in chunks so the vertex workspace stays under ~1 GiB; items whose contour is
     longer than ``max_pts`` are re-run on their own with a larger bound."""
     if mode not in CONTOUR_MODES:
         raise ValueError(f"mode must be one of {CONTOUR_MODES}, got {mode!r}")
+    spacing = derive.spacing_2d(spacing)
     yt, yp = _check_pair(y_true, y_pred)
     n, h, w = yt.shape
     k = int(num_classes)
@@ -345,6 +398,8 @@ def contour_pass(y_true, y_pred, num_classes, first_pos=None, *, max_pts=None, r
     max_pts = (int(max_pts) + 3) & ~3
     if h < 2 or w < 2:
         raise ValueError("Input array must be at least 2x2.")     # skimage's message for find_contours
+    if spacing is not None and not np.isfinite(spacing[0] ** 2 * (2.0 * h) ** 2 + spacing[1] ** 2 * (2.0 * w) ** 2):
+        raise ValueError(f"spacing {spacing}: the squared diagonal of a {h} x {w} image overflows a double")
     dev = yt.device
     if mode == "all":
         first_pos = boundaries = unsorted = None
@@ -357,8 +412,8 @@ def contour_pass(y_true, y_pred, num_classes, first_pos=None, *, max_pts=None, r
                 first_pos[:, m, :] = tmp
         keep = return_vertices or return_sq
         if n == 0:
-            return ContourOut(*_contour_outputs(0, k, dev), None, None, max_pts, mode)
-        per_item = k * 2 * max_pts * 4 * 2          # vertices + squared-distance scratch
+            return ContourOut(*_contour_outputs(0, k, dev, spacing), None, None, max_pts, mode, spacing)
+        per_item = k * 2 * max_pts * _vertex_bytes(spacing)          # vertices + squared-distance scratch
         chunk = n if keep else max(1, min(n, CONTOUR_CHUNK_BYTES // per_item))
         parts = []
         for s in range(0, n, chunk):
@@ -366,13 +421,13 @@ def contour_pass(y_true, y_pred, num_classes, first_pos=None, *, max_pts=None, r
             parts.append(_contour_chunk(yt[s:e], yp[s:e], k, max_pts, mode, return_vertices, return_sq, timers,
                                         None if first_pos is None else first_pos[s:e],
                                         None if boundaries is None else (boundaries[0][s:e], boundaries[1][s:e]),
-                                        None if unsorted is None else unsorted[s:e]))
+                                        None if unsorted is None else unsorted[s:e], spacing))
         if len(parts) == 1:
             out = parts[0]
         else:
             cat = lambda f: torch.cat([getattr(p, f) for p in parts])      # noqa: E731
             out = ContourOut(cat("n_pts"), cat("flags"), cat("max_sq"), cat("p95_sq"), cat("sum_dist"), None, None,
-                             max_pts, mode)
+                             max_pts, mode, spacing)
         if check_overflow:
             _retry_overflow(out, yt, yp, k, first_pos, keep)
     return out
@@ -404,12 +459,13 @@ def _retry_overflow(out, yt, yp, k, first_pos, keep=False):
             if big >= MAX_MAX_PTS:
                 raise _lib.OctmError(f"a contour has more than {MAX_MAX_PTS} vertices: pass a larger max_pts")
             big = min(big * 8, MAX_MAX_PTS)
-        chunk = max(1, CONTOUR_CHUNK_BYTES // (k * 2 * big * 4 * 2))
+        chunk = max(1, CONTOUR_CHUNK_BYTES // (k * 2 * big * _vertex_bytes(out.spacing)))
         still = []
         for s0 in range(0, idx.numel(), chunk):
             sub = idx[s0:s0 + chunk]
             redo = _contour_chunk(yt[sub].contiguous(), yp[sub].contiguous(), k, big, out.mode, False, False,
-                                  first_pos=None if first_pos is None else first_pos[sub].contiguous())
+                                  first_pos=None if first_pos is None else first_pos[sub].contiguous(),
+                                  spacing=out.spacing)
             for f in ("n_pts", "flags", "max_sq", "p95_sq", "sum_dist"):
                 getattr(out, f)[sub] = getattr(redo, f)
             if out.mode == "first":
@@ -418,17 +474,27 @@ def _retry_overflow(out, yt, yp, k, first_pos, keep=False):
     return True
 
 
-def derive_on_device(lp, ct, n, timers=None):
-    """Float64 per-class metrics + this batch's dataset totals, computed by ``octm_derive_metrics``."""
+def derive_on_device(lp, ct, n, timers=None, spacing=None):
+    """Float64 per-class metrics + this batch's dataset totals, computed by ``octm_derive_metrics`` (with a pixel
+    spacing ``(sy, sx)``: ``octm_derive_metrics_spacing``, float64 squared distances and scaled thickness and boundary
+    errors)."""
     k, dev = lp.num_classes, lp.counts.device
     cls = torch.empty((n, k, len(_lib.CLASS_METRICS)), dtype=torch.float64, device=dev)
     bnd = torch.empty((n, k - 1, 3), dtype=torch.float64, device=dev) if lp.bnd_sq is not None else None
     tot = torch.empty((_lib.load().octm_totals_len(k),), dtype=torch.float64, device=dev)
+    contour = ((_ptr(ct.n_pts), _ptr(ct.max_sq), _ptr(ct.p95_sq), _ptr(ct.sum_dist), _ptr(ct.flags)) if ct
+               else (None,) * 5)
     with torch.cuda.device(dev), _Timed(timers, "derive"):
-        _lib.call("octm_derive_metrics", _ptr(lp.counts), _ptr(lp.thick_absdiff), _ptr(lp.bnd_sq), _ptr(lp.bnd_abs),
-                  _ptr(ct.n_pts) if ct else None, _ptr(ct.max_sq) if ct else None, _ptr(ct.p95_sq) if ct else None,
-                  _ptr(ct.sum_dist) if ct else None, _ptr(ct.flags) if ct else None, n, lp.height, lp.width, k,
-                  _ptr(cls), _ptr(bnd), _ptr(tot), _stream())
+        if spacing is None:
+            _lib.call("octm_derive_metrics", _ptr(lp.counts), _ptr(lp.thick_absdiff), _ptr(lp.bnd_sq), _ptr(lp.bnd_abs),
+                      *contour, n, lp.height, lp.width, k, _ptr(cls), _ptr(bnd), _ptr(tot), _stream())
+        else:
+            if ct is not None and ct.spacing != tuple(spacing):
+                raise ValueError(f"contour distances at spacing {ct.spacing}, epilogue at {tuple(spacing)}")
+            sp = (ctypes.c_double * 2)(*spacing)
+            _lib.call("octm_derive_metrics_spacing", _ptr(lp.counts), _ptr(lp.thick_absdiff), _ptr(lp.bnd_sq),
+                      _ptr(lp.bnd_abs), *contour, n, lp.height, lp.width, k, ctypes.addressof(sp), _ptr(cls), _ptr(bnd),
+                      _ptr(tot), _stream())
     return cls, bnd, tot
 
 
@@ -437,10 +503,10 @@ class SurfaceDiceOut:
     """Exact counts of the surface Dice pass (device tensors, uint32 stored as int32 bits)."""
     n_surf: torch.Tensor       # [N, K, 2]      (|V_t|, |V_p|): all-contour vertices of y_true / y_pred
     n_within: torch.Tensor     # [N, K, 2, T]   vertices within tolerance j of the other boundary; direction 0: pred -> true
-    tolerances: tuple          # T tolerances in pixels, in the caller's order
+    tolerances: tuple          # T tolerances in pixels (in the units of the spacing with one), in the caller's order
 
 
-def surface_dice(y_true, y_pred, num_classes, tolerances=(1.0,), *, timers=None):
+def surface_dice(y_true, y_pred, num_classes, tolerances=(1.0,), *, timers=None, spacing=None):
     """Normalized surface Dice counts of every class at 1 to 4 tolerances ``0 <= tau <= 8`` pixels (build-defined,
     no reference counterpart; MONAI ``compute_surface_dice``, surface-distance ``compute_surface_dice_at_tolerance``).
 
@@ -448,7 +514,15 @@ def surface_dice(y_true, y_pred, num_classes, tolerances=(1.0,), *, timers=None)
     as within ``tau`` when the nearest vertex of the other map lies at ``sqrt(D2 / 4.0) <= tau``, the expression every
     contour distance of the suite is reported through.  One read of each label map (``octm_surface_dice_u8``).
     Tolerances may come in any order; the counts come back in that order.  ``derive.surface_dice`` turns them into
-    float64 NSD values."""
+    float64 NSD values.
+
+    ``spacing=(sy, sx)``: pixel size along rows and columns; the tolerances are then in its units and a vertex is within
+    ``tau`` when ``sqrt(q / 4.0) <= tau`` for the ``q`` of ``contour_pass(spacing=...)`` (``octm_surface_dice_spacing_u8``).
+    The kernel reaches 16 lattice rows and 16 lattice columns: a larger tolerance raises ValueError naming
+    ``derive.surface_dice_spacing_limit(spacing)``."""
+    spacing = derive.spacing_2d(spacing)
+    if spacing is not None:
+        return _surface_dice_spacing(y_true, y_pred, num_classes, tolerances, timers, spacing)
     taus = derive.surface_dice_tolerances(tolerances)
     thr = [derive.surface_dice_threshold(t) for t in taus]
     order = sorted(range(len(taus)), key=lambda j: thr[j])
@@ -464,6 +538,22 @@ def surface_dice(y_true, y_pred, num_classes, tolerances=(1.0,), *, timers=None)
                   _ptr(n_within), _stream())
     if order != sorted(order):
         n_within = n_within[..., [order.index(j) for j in range(len(taus))]]
+    return SurfaceDiceOut(n_surf, n_within, taus)
+
+
+def _surface_dice_spacing(y_true, y_pred, num_classes, tolerances, timers, spacing):
+    taus = derive.surface_dice_spacing_tolerances(tolerances, spacing)
+    yt, yp = _check_pair(y_true, y_pred)
+    n, h, w = yt.shape
+    k = int(num_classes)
+    dev = yt.device
+    n_surf = torch.empty((n, k, 2), dtype=torch.int32, device=dev)
+    n_within = torch.empty((n, k, 2, len(taus)), dtype=torch.int32, device=dev)
+    sp = (ctypes.c_double * 2)(*spacing)
+    tol = (ctypes.c_double * len(taus))(*taus)
+    with torch.cuda.device(dev), _Timed(timers, "surface_dice"):
+        _lib.call("octm_surface_dice_spacing_u8", _ptr(yt), _ptr(yp), n, h, w, k, ctypes.addressof(sp),
+                  ctypes.addressof(tol), len(taus), _ptr(n_surf), _ptr(n_within), _stream())
     return SurfaceDiceOut(n_surf, n_within, taus)
 
 
@@ -529,6 +619,7 @@ class SuiteResult:
     contour_mode: str | None = "first"     # "first" / "all" (contour_pass modes), None without contour metrics
     surface: SurfaceDiceOut | None = None  # evaluate(surface_dice=...) only
     components: ComponentsOut | None = None  # evaluate(components=...) only
+    spacing: tuple | None = None           # (sy, sx) pixel spacing of the distances, None: pixel units
 
     @property
     def surface_dice_tolerances(self):
@@ -551,7 +642,8 @@ class SuiteResult:
             return False
         yt, yp = self._inputs
         _retry_overflow(self.contours, yt, yp, self.labels.num_classes, self.labels.first_pos)
-        self.class_metrics, self.boundary_metrics, self.totals = derive_on_device(self.labels, self.contours, self.num_items)
+        self.class_metrics, self.boundary_metrics, self.totals = derive_on_device(self.labels, self.contours, self.num_items,
+                                                                                   spacing=self.spacing)
         return True
 
     def totals_host(self):
@@ -592,8 +684,9 @@ class SuiteResult:
         if ct is not None:
             d["contour_n_pts"] = ct.n_pts.cpu().numpy().view(np.uint32)
             d["contour_flags"] = ct.flags.cpu().numpy().view(np.uint32)
-            d["contour_max_sq"] = ct.max_sq.cpu().numpy().view(np.uint32)
-            d["contour_p95_sq"] = ct.p95_sq.cpu().numpy().view(np.uint32)
+            sq = (lambda t: t.cpu().numpy().view(np.uint32)) if ct.spacing is None else (lambda t: t.cpu().numpy())   # noqa: E731
+            d["contour_max_sq"] = sq(ct.max_sq)
+            d["contour_p95_sq"] = sq(ct.p95_sq)
             d["contour_sum_dist"] = ct.sum_dist.cpu().numpy()
         if self.surface is not None:
             d["surface_dice_n_surf"] = self.surface.n_surf.cpu().numpy().view(np.uint32)
@@ -637,8 +730,9 @@ class SuiteResult:
         if "confusion" in ints:
             m.update(derive.count_metrics(*derive.class_counts(ints["confusion"])))
         if "thickness_absdiff" in ints:
-            m["thickness_difference"] = derive.thickness_difference(ints["thickness_absdiff"], self.labels.width)
-            m.update(derive.boundary_errors(ints["boundary_sq"], ints["boundary_abs"], self.labels.width))
+            m["thickness_difference"] = derive.thickness_difference(ints["thickness_absdiff"], self.labels.width,
+                                                                    self.spacing)
+            m.update(derive.boundary_errors(ints["boundary_sq"], ints["boundary_abs"], self.labels.width, self.spacing))
         if "contour_n_pts" in ints:
             m.update(derive.contour_metrics(ints["contour_n_pts"], ints["contour_max_sq"],
                                             ints["contour_p95_sq"], ints["contour_sum_dist"]))
@@ -658,7 +752,7 @@ def _contour_mode(contours):
 
 
 def evaluate(y_true, y_pred, num_classes, *, contours=True, boundaries=False, max_pts=None, timers=None,
-             validate=True, surface_dice=None, components=None):
+             validate=True, surface_dice=None, components=None, spacing=None):
     """The full suite on a batch of label maps: fused label pass, contour kernels, float64 epilogue.
 
     ``contours``: ``True`` / ``"first"`` = hausdorff / hd95 / assd on contour ``[0]`` of each class mask, as the
@@ -676,6 +770,12 @@ def evaluate(y_true, y_pred, num_classes, *, contours=True, boundaries=False, ma
     ``contours`` and ``surface_dice``), the counts ``integers()["component_count"]`` / ``["component_hits"]``
     (uint32 ``[N, K, 2]``) and ``component_connectivity``.
 
+    ``spacing``: ``None`` (default, pixel units) or ``(sy, sx)``, the pixel size along rows (axial) and columns (lateral)
+    in any unit, e.g. ``datasets.mhd_spacing(header)[-2:]``.  Hausdorff, HD95, ASSD and the surface Dice tolerances are
+    then in its units (see ``contour_pass`` and ``surface_dice``), ``thickness_difference`` and ``boundary_mad`` scale
+    with ``sy`` and ``boundary_mse`` with ``sy**2``; ``integers()["contour_max_sq"]`` / ``["contour_p95_sq"]`` become
+    float64 squared distances.  Confusion-matrix, region and component metrics do not change.
+
     Everything is launched asynchronously on the current stream; nothing is read back until
     ``totals_host()`` / ``metrics()`` / ``integers()`` is called on the result.
     ``timers``: optional dict filled with (start, end) CUDA-event pairs per kernel family.
@@ -683,25 +783,31 @@ def evaluate(y_true, y_pred, num_classes, *, contours=True, boundaries=False, ma
     the results are read.  The check costs nothing extra: the label pass never aliases such a pixel into another
     class but drops it, so the item's confusion counts do not add up to H * W, which the totals kernel counts."""
     mode = _contour_mode(contours)
-    taus = None if surface_dice is None else derive.surface_dice_tolerances(surface_dice)
+    spacing = derive.spacing_2d(spacing)
+    if surface_dice is None:
+        taus = None
+    elif spacing is None:
+        taus = derive.surface_dice_tolerances(surface_dice)
+    else:
+        taus = derive.surface_dice_spacing_tolerances(surface_dice, spacing)
     conn = None if components is None else _connectivity(components)
     yt, yp = _check_pair(y_true, y_pred)
     first = mode == "first"
     # contour [0] is seeded by the label pass, and its boundary rows and certificate skip the walk on layered maps
     lp = label_pass(yt, yp, num_classes, counts=True, columns=True, seeds=first, boundaries=boundaries or first,
                     timers=timers, certify=first)
-    sd = None if taus is None else _surface_dice_pass(yt, yp, num_classes, taus, timers=timers)
+    sd = None if taus is None else _surface_dice_pass(yt, yp, num_classes, taus, timers=timers, spacing=spacing)
     cc = None if conn is None else _components_pass(yt, yp, num_classes, conn, timers=timers)
     ct = None
     if mode is not None:
         ct = contour_pass(yt, yp, num_classes, lp.first_pos, max_pts=max_pts, timers=timers, check_overflow=False,
                           boundaries=(lp.bnd_true, lp.bnd_pred) if first else None,
-                          unsorted=lp.unsorted if first else None, mode=mode)
+                          unsorted=lp.unsorted if first else None, mode=mode, spacing=spacing)
         if first and not boundaries:
             lp.bnd_true = lp.bnd_pred = None
-    cls, bnd, tot = derive_on_device(lp, ct, yt.shape[0], timers)
+    cls, bnd, tot = derive_on_device(lp, ct, yt.shape[0], timers, spacing)
     return SuiteResult(yt.shape[0], lp, ct, cls, bnd, tot, (yt, yp) if ct is not None else None,
-                       validate=bool(validate), contour_mode=mode, surface=sd, components=cc)
+                       validate=bool(validate), contour_mode=mode, surface=sd, components=cc, spacing=spacing)
 
 
 def _cat_results(parts):
@@ -718,9 +824,10 @@ def _cat_results(parts):
     if parts[0].contours is not None:
         cts = [p.contours for p in parts]
         ct = ContourOut(*[cat(cts, f) for f in ("n_pts", "flags", "max_sq", "p95_sq", "sum_dist")], None, None,
-                        cts[0].max_pts, cts[0].mode)
+                        cts[0].max_pts, cts[0].mode, cts[0].spacing)
     n = sum(p.num_items for p in parts)
-    cls, bnd, tot = derive_on_device(lp, ct, n)            # per-item values again + totals of the whole batch
+    spacing = parts[0].spacing
+    cls, bnd, tot = derive_on_device(lp, ct, n, spacing=spacing)    # per-item values again + totals of the whole batch
     sd = None
     if parts[0].surface is not None:
         sds = [p.surface for p in parts]
@@ -730,7 +837,7 @@ def _cat_results(parts):
         ccs = [p.components for p in parts]
         cc = ComponentsOut(cat(ccs, "n_comp"), cat(ccs, "n_hit"), ccs[0].connectivity)
     res = SuiteResult(n, lp, ct, cls, bnd, tot, validate=parts[0].validate, contour_mode=parts[0].contour_mode,
-                      surface=sd, components=cc)
+                      surface=sd, components=cc, spacing=spacing)
     res._final = True
     return res
 
@@ -748,7 +855,8 @@ def _pinned(nbytes):
 
 
 def evaluate_host(y_true, y_pred, num_classes, *, contours=True, device=None, chunk_items=None,
-                  max_pts=None, pack=False, pack_threads=0, validate=True, surface_dice=None, components=None):
+                  max_pts=None, pack=False, pack_threads=0, validate=True, surface_dice=None, components=None,
+                  spacing=None):
     """The full suite on HOST label maps (numpy arrays or CPU torch tensors, ideally pinned).
 
     Items are streamed to the GPU in chunks through two staging buffers: the host->device copy of
@@ -758,7 +866,8 @@ def evaluate_host(y_true, y_pred, num_classes, *, contours=True, device=None, ch
     being copied, and a streaming kernel expands it in HBM.  Off by default: on the 16-core B200 boxes the
     packer sustains ~80 GB/s of input, which only ties with the plain copy (measured 92-100 k vs 98-100 k
     B-scans/s); it pays on hosts with more memory bandwidth per PCIe lane.  Results stay on the device
-    until ``metrics()`` / ``integers()`` reads them back."""
+    until ``metrics()`` / ``integers()`` reads them back.  ``spacing`` as for ``evaluate``."""
+    spacing = derive.spacing_2d(spacing)
     if not torch.cuda.is_available():
         raise RuntimeError("a CUDA device is required: this package has no CPU fallback")
     dev = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
@@ -846,7 +955,8 @@ def evaluate_host(y_true, y_pred, num_classes, *, contours=True, device=None, ch
             if use_pack:
                 expand(ci)
             parts.append(evaluate(bt[:e0 - s0], bp[:e0 - s0], num_classes, contours=contours, max_pts=max_pts,
-                                  validate=validate, surface_dice=surface_dice, components=components))
+                                  validate=validate, surface_dice=surface_dice, components=components,
+                                  spacing=spacing))
             done = torch.cuda.Event()
             done.record(compute)
             freed[ci & 1] = done
@@ -883,10 +993,10 @@ def labels_from_scores(scores, *, channels_last=False, out=None):
     return out
 
 
-def evaluate_scores(y_true, scores, num_classes=None, *, channels_last=False, **kw):
+def evaluate_scores(y_true, scores, num_classes=None, *, channels_last=False, spacing=None, **kw):
     """``evaluate(y_true, argmax(scores), ...)`` with the argmax done by ``labels_from_scores``."""
     k = scores.shape[-1 if channels_last else 1] if num_classes is None else int(num_classes)
-    return evaluate(y_true, labels_from_scores(scores, channels_last=channels_last), k, **kw)
+    return evaluate(y_true, labels_from_scores(scores, channels_last=channels_last), k, spacing=spacing, **kw)
 
 
 def auc_scores(y_true, scores, *, single_class_value=float("nan")):
