@@ -322,6 +322,27 @@ OCTM_API int octm_labels_from_boundaries(const void* boundaries, int dtype, int6
                                 int H, int W, uint8_t* labels, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * Layer thickness per en-face sector of OCT volumes (build-defined, no reference counterpart; the ETDRS grid of clinical
+ * OCT reports).  Reads the boundary rows b_k(x) = #{y : L[y][x] < k} of octm_label_pass_u8 (b_0 = 0, b_K = H): they are
+ * counts, so for ANY label map with values < K the thickness of the classes first .. last in A-scan x is
+ * b_{last+1}(x) - b_first(x).  Items [v * items_per_volume, (v + 1) * items_per_volume) form volume v.
+ *   bnd_true, bnd_pred  int32 [n][K-1][W]   boundary rows of y_true / y_pred (undefined for maps with a label >= K)
+ *   region   uint8 [n][W]                   region of every A-scan: 0 .. n_regions - 1; any other value (255) = none
+ *   groups   HOST int32 [n_groups][2]       (first, last) class of each group, 0 <= first <= last <= K - 1
+ *   sums     int64 [n / items_per_volume][n_groups][n_regions][5]   per (volume, group, region), over its A-scans:
+ *                                           count, sum t, sum p, sum |t - p|, sum (t - p)^2, with t / p the group
+ *                                           thickness of y_true / y_pred in pixels.  Fully overwritten; exact integers
+ *                                           (the order of the device atomics does not matter: bit-reproducible)
+ *   thick    int32 [n][2][n_groups][W]      t ([i][0]) and p ([i][1]) of every A-scan, whatever its region; or NULL
+ * Every argument is checked before any CUDA call: shapes, 2 <= K <= 16, n % items_per_volume == 0, 1 <= n_regions <= 16,
+ * 1 <= n_groups <= 16 and the group bounds, items_per_volume * W * H^2 < 2^53 (every sum exact in int64 and in a float64
+ * all-reduce), at most 65535 volumes; device pointers other than thick may be NULL only when n_items == 0. */
+OCTM_API int octm_sector_thickness_i32(const int32_t* bnd_true, const int32_t* bnd_pred, int64_t n_items,
+                                       int num_classes, int H, int W, int items_per_volume, const uint8_t* region,
+                                       int n_regions, const int32_t* groups /* HOST [n_groups][2] */, int n_groups,
+                                       int64_t* sums, int32_t* thick, void* stream);
+
+/* ---------------------------------------------------------------------------------------------
  * 3-D surface-distance metrics (BASELINE config 5; the reference's contour metrics are 2-D only, this is
  * their build-defined 3-D counterpart): per class, distances between the SURFACES of the class regions of
  * two label volumes [D0][D1][D2] by an exact separable squared Euclidean distance transform (Meijster).

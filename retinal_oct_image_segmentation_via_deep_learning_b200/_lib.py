@@ -67,6 +67,7 @@ SIGNATURES = {
     "octm_host_pack_nibbles": (_INT, [_P, _P, _c.c_size_t, _INT]),
     "octm_unpack_nibbles_u8": (_INT, [_P, _I64, _P, _P]),
     "octm_labels_from_boundaries": (_INT, [_P, _INT, _I64, _INT, _INT, _INT, _P, _P]),
+    "octm_sector_thickness_i32": (_INT, [_P, _P, _I64, _INT, _INT, _INT, _INT, _P, _INT, _P, _INT, _P, _P, _P]),
     "octm_totals_len": (_INT, [_INT]),
     "octm_totals_sum_len": (_INT, [_INT]),
     "octm_derive_metrics": (_INT, [_P, _P, _P, _P, _P, _P, _P, _P, _P, _I64, _INT, _INT, _INT, _P, _P, _P, _P]),

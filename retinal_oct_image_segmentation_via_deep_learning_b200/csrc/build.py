@@ -16,7 +16,7 @@ from concurrent.futures import ThreadPoolExecutor
 HERE = os.path.dirname(os.path.abspath(__file__))
 PKG = os.path.dirname(HERE)
 LIB = os.path.join(PKG, "liboctm.so")
-SOURCES = ["common.cu", "label_pass.cu", "contour.cu", "contour_all.cu", "contour_spacing.cu", "surface_dice.cu", "components.cu", "derive.cu", "argmax.cu", "auc.cu", "boundary.cu", "edt3d.cu", "hostpack.cu", "rasterise.cu"]
+SOURCES = ["common.cu", "label_pass.cu", "contour.cu", "contour_all.cu", "contour_spacing.cu", "surface_dice.cu", "components.cu", "derive.cu", "argmax.cu", "auc.cu", "boundary.cu", "edt3d.cu", "hostpack.cu", "rasterise.cu", "sector_thickness.cu"]
 HEADERS = ["common.cuh", "crack_masks.cuh", "trace_core.h", os.path.join("..", "..", "include", "octm.h")]
 NVCC_FLAGS = ["-std=c++17", "-O3", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "--fmad=false",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden"]

@@ -241,3 +241,156 @@ def component_metrics(n_comp, n_hit):
     f1 = np.where((nt == 0) & (npred == 0), np.nan, f1)
     return {"component_count_error": np.abs(nt - npred).astype(np.float64), "component_recall": rec,
             "component_precision": prec, "component_f1": f1}
+
+
+# ETDRS grid: region codes of ``etdrs_regions`` in this order.  The names are en-face index directions (b: B-scan index,
+# x: column), not anatomy: which one is superior, inferior, nasal or temporal depends on the eye and on the device's
+# B-scan order (INTEGRATION.md).
+ETDRS_SECTORS = ("center", "inner_b-", "inner_x+", "inner_b+", "inner_x-", "outer_b-", "outer_x+", "outer_b+", "outer_x-")
+ETDRS_RADII = (0.5, 1.5, 3.0)        # mm: 1, 3 and 6 mm diameters
+NO_REGION = 255
+SECTOR_STATS = ("n_ascans", "sum_true", "sum_pred", "sum_absdiff", "sum_sqdiff")     # last axis of the kernel's sums
+
+
+def spacing_3d(spacing):
+    """A volume spacing ``(sb, sy, sx)`` (B-scans, rows = axial, columns = lateral; ``datasets.mhd_spacing(hdr)``) ->
+    tuple of 3 floats; ValueError unless all are finite and > 0."""
+    try:
+        sp = tuple(float(v) for v in np.asarray(spacing, dtype=np.float64).reshape(-1))
+    except (TypeError, ValueError):
+        raise ValueError(f"spacing must be 3 numbers (B-scans, rows, columns), got {spacing!r}") from None
+    if len(sp) != 3 or not all(np.isfinite(v) and v > 0 for v in sp):
+        raise ValueError(f"spacing must be 3 finite numbers > 0 (B-scans, rows, columns), got {spacing!r}")
+    return sp
+
+
+def etdrs_radii(radii):
+    """``(R0, R1, R2)`` -> tuple of 3 floats; ValueError unless finite with ``0 < R0 <= R1 <= R2``."""
+    try:
+        r = tuple(float(v) for v in np.asarray(radii, dtype=np.float64).reshape(-1))
+    except (TypeError, ValueError):
+        raise ValueError(f"radii must be 3 numbers, got {radii!r}") from None
+    if len(r) != 3 or not all(np.isfinite(v) for v in r) or not 0 < r[0] <= r[1] <= r[2]:
+        raise ValueError(f"radii must be 3 finite numbers with 0 < R0 <= R1 <= R2, got {radii!r}")
+    return r
+
+
+def etdrs_regions(n_bscans, width, spacing, center, radii=ETDRS_RADII):
+    """uint8 ``[n_bscans, width]`` ETDRS region of every A-scan (b, x) of one volume.
+
+    With ``spacing = (sb, sy, sx)`` and ``center = (cb, cx)`` (fractional B-scan and column indices) the en-face position
+    is ``pb = (b - cb) * sb``, ``px = (x - cx) * sx`` and ``r2 = pb * pb + px * px`` in float64.  With
+    ``radii = (R0, R1, R2)``: region 0 (center) if ``r2 <= R0 * R0``, the inner ring if ``r2 <= R1 * R1``, the outer ring
+    if ``r2 <= R2 * R2``, ``NO_REGION`` (255) otherwise.  A ring's quadrant is on the b side when ``|pb| > |px|`` and
+    on the x side otherwise (diagonal ties go to x); regions 1-4 are inner b-, x+, b+, x-, regions 5-8 outer ones in the
+    same order (``ETDRS_SECTORS``)."""
+    sb, _, sx = spacing_3d(spacing)
+    r0, r1, r2_ = etdrs_radii(radii)
+    cb, cx = (float(v) for v in np.asarray(center, dtype=np.float64).reshape(2))
+    if not (np.isfinite(cb) and np.isfinite(cx)):
+        raise ValueError(f"center must be finite, got {center!r}")
+    pb = (np.arange(int(n_bscans), dtype=np.float64) - cb)[:, None] * sb
+    px = (np.arange(int(width), dtype=np.float64) - cx)[None, :] * sx
+    r2 = pb * pb + px * px
+    bside = np.abs(pb) > np.abs(px)
+    quad = np.where(bside, np.where(pb < 0, 0, 2), np.where(px > 0, 1, 3))
+    out = np.full(r2.shape, NO_REGION, dtype=np.uint8)
+    out[r2 <= r2_ * r2_] = 5 + quad[r2 <= r2_ * r2_]
+    out[r2 <= r1 * r1] = 1 + quad[r2 <= r1 * r1]
+    out[r2 <= r0 * r0] = 0
+    return out
+
+
+def sector_thickness(sums, spacing):
+    """Per-volume sector thickness from the exact sums of ``octm_sector_thickness_i32``: ``sums [V, G, R, 5]``
+    (``SECTOR_STATS``) and the volume ``spacing = (sb, sy, sx)`` -> dict of float64 ``[V, G, R]`` arrays, NaN where a
+    region holds no A-scan, plus ``n_ascans`` (int64).  In the units of the spacing, with n A-scans:
+
+    - ``thickness_true`` = (sum t / n) * sy, ``thickness_pred`` = (sum p / n) * sy;
+    - ``thickness_bias`` = ((sum p - sum t) / n) * sy;
+    - ``thickness_mae`` = (sum |t - p| / n) * sy;
+    - ``thickness_rmse`` = sqrt(sum (t - p)^2 / n) * sy;
+    - ``volume_true`` = sum t * ((sb * sy) * sx), ``volume_pred`` likewise.
+    """
+    sb, sy, sx = spacing_3d(spacing)
+    s = np.asarray(sums).astype(np.int64)
+    n = s[..., 0]
+    nf = np.where(n > 0, n, 1).astype(np.float64)
+    nan = np.full(n.shape, np.nan)
+    vox = (sb * sy) * sx
+
+    def per(v):
+        return np.where(n > 0, v, nan)
+    return {"thickness_true": per(s[..., 1] / nf * sy), "thickness_pred": per(s[..., 2] / nf * sy),
+            "thickness_bias": per((s[..., 2] - s[..., 1]) / nf * sy), "thickness_mae": per(s[..., 3] / nf * sy),
+            "thickness_rmse": per(np.sqrt(s[..., 4] / nf) * sy),
+            "volume_true": per(s[..., 1] * vox), "volume_pred": per(s[..., 2] * vox), "n_ascans": n}
+
+
+SECTOR_SUMMARY = ("abs_bias", "bias", "mae", "rmse", "thickness_true", "thickness_pred")
+
+
+def sector_thickness_summary(per_volume):
+    """Dataset-level sector thickness from ``sector_thickness`` output: per (group, sector) the mean over the volumes
+    whose region holds at least one A-scan, summed in volume order, of |bias|, bias, MAE, RMSE, true and predicted
+    thickness (``SECTOR_SUMMARY`` order), float64 ``[G, R]`` each (NaN where no volume covers the region), and
+    ``n_volumes`` (int64 ``[G, R]``), the number of volumes covering it."""
+    src = {"abs_bias": np.abs(per_volume["thickness_bias"]), "bias": per_volume["thickness_bias"],
+           "mae": per_volume["thickness_mae"], "rmse": per_volume["thickness_rmse"],
+           "thickness_true": per_volume["thickness_true"], "thickness_pred": per_volume["thickness_pred"]}
+    covered = np.asarray(per_volume["n_ascans"]) > 0
+    cnt = covered.sum(axis=0).astype(np.int64)
+    out = {}
+    for name in SECTOR_SUMMARY:
+        v = np.asarray(src[name], dtype=np.float64)
+        acc = np.zeros(v.shape[1:])
+        for i in range(v.shape[0]):
+            acc = acc + np.where(covered[i], v[i], 0.0)
+        with np.errstate(invalid="ignore", divide="ignore"):
+            out[name] = np.where(cnt > 0, acc / np.maximum(cnt, 1), np.nan)
+    out["n_volumes"] = cnt
+    return out
+
+
+SECTOR_MAX_GROUPS = 16
+
+
+def sector_groups(classes, num_classes):
+    """``classes`` of ``suite.sector_thickness`` -> tuple of ``(first, last)`` class pairs: None gives one group per class;
+    otherwise 1 to 16 entries, each a class or a ``(first, last)`` pair with ``0 <= first <= last <= num_classes - 1``."""
+    k = int(num_classes)
+    if classes is None:
+        entries = list(range(k))
+    else:
+        entries = list(classes)
+    if not 1 <= len(entries) <= SECTOR_MAX_GROUPS:
+        raise ValueError(f"classes: 1 to {SECTOR_MAX_GROUPS} groups, got {len(entries)}")
+    out = []
+    for e in entries:
+        pair = (e, e) if np.ndim(e) == 0 else tuple(e)
+        if len(pair) != 2 or not all(isinstance(v, (int, np.integer)) and not isinstance(v, bool) for v in pair):
+            raise ValueError(f"classes: each entry must be a class or a (first, last) pair of ints, got {e!r}")
+        f, last = int(pair[0]), int(pair[1])
+        if not 0 <= f <= last <= k - 1:
+            raise ValueError(f"classes: group {e!r} needs 0 <= first <= last <= {k - 1}")
+        out.append((f, last))
+    return tuple(out)
+
+
+def sector_centers(center, n_volumes, n_bscans, width):
+    """``center`` of ``suite.sector_thickness`` -> float64 ``[V, 2]`` (B-scan, column) fractional indices: None gives the
+    geometric centre ``((B - 1) / 2, (W - 1) / 2)`` of every volume, one pair is used for every volume, and a ``[V, 2]``
+    array gives one per volume.  ValueError for another shape or a value that is not finite."""
+    if center is None:
+        return np.tile(np.array([(n_bscans - 1) / 2.0, (width - 1) / 2.0]), (n_volumes, 1))
+    try:
+        c = np.asarray(center, dtype=np.float64)
+    except (TypeError, ValueError):
+        raise ValueError(f"center must be a (b, x) pair or a [V, 2] array, got {center!r}") from None
+    if c.shape == (2,):
+        c = np.tile(c, (n_volumes, 1))
+    if c.shape != (n_volumes, 2):
+        raise ValueError(f"center must be a (b, x) pair or a [{n_volumes}, 2] array, got shape {c.shape}")
+    if not np.all(np.isfinite(c)):
+        raise ValueError("center must be finite")
+    return c

@@ -266,3 +266,42 @@ def surface_distance_3d_sharded(vol_true, vol_pred, num_classes, rank, world, gr
             ints[key] = s.clone() if v.dtype == torch.float64 else s.to(torch.int64).to(v.dtype)
             o += m
     return ints
+
+
+def sector_thickness_totals(out, world, first_volume, n_volumes, group=None):
+    """Sector thickness over all ranks' volumes from one ``suite.sector_thickness`` result per rank, each rank holding the
+    volumes ``[first_volume, first_volume + V)`` of ``n_volumes`` (e.g. ``shard_range(n_volumes, rank, world)``).
+
+    Each rank writes its exact integer sums at its offset of a zero float64 ``[n_volumes, G, 9, 5]`` vector, plus its
+    count of items with a label >= num_classes and a flag for a volume range outside ``[0, n_volumes)``, and ONE SUM
+    all-reduce combines them: every entry is written by exactly one rank and is below 2**53, so the reduced sums are
+    exact.  Every rank then derives the same ``metrics`` (``derive.sector_thickness``, ``[n_volumes, G, 9]``) and
+    ``summary`` (``derive.sector_thickness_summary``) from the reduced ``sums``: bit-identical to one process scoring
+    every volume, for any world size; a rank may hold no volume.  A label >= num_classes or a bad volume range on any rank
+    raises ValueError on every rank, after the collective, so that no rank is left waiting in it.  ``n_volumes`` and the
+    groups must be the same on every rank (they fix the length of the reduced vector)."""
+    import torch
+    sums = out.sums.cpu().numpy()
+    v, g, r, s = sums.shape
+    first_volume, n_volumes = int(first_volume), int(n_volumes)
+    unit = g * r * s
+    vec = np.zeros(max(n_volumes, 0) * unit + 2)
+    if 0 <= first_volume <= first_volume + v <= n_volumes:
+        vec[first_volume * unit:(first_volume + v) * unit] = sums.reshape(-1)
+    else:
+        vec[-2] = 1                                   # decided after the collective, on every rank
+    vec[-1] = out.bad_label_items()
+    dev = out.sums.device
+    use_dev = dev.type == "cuda" and torch.distributed.is_initialized() and \
+        torch.distributed.get_backend(group) == "nccl"
+    vec = all_reduce_sum(vec, world, device=dev if use_dev else None, group=group)
+    if int(round(vec[-2])):
+        raise ValueError(f"{int(round(vec[-2]))} rank(s) hold volumes outside [0, {n_volumes}) (this rank: "
+                         f"[{first_volume}, {first_volume + v}))")
+    bad = int(round(vec[-1]))
+    if bad:
+        raise ValueError(f"{bad} item(s) hold a label >= num_classes {out.num_classes}")
+    total = np.rint(vec[:-2]).astype(np.int64).reshape(n_volumes, g, r, s)
+    metrics = derive.sector_thickness(total, out.spacing)
+    return {"sums": total, "metrics": metrics, "summary": derive.sector_thickness_summary(metrics),
+            "groups": out.groups, "spacing": out.spacing}

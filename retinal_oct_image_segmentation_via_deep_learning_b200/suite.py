@@ -1137,3 +1137,95 @@ def validate_labels(labels, num_classes):
     mx = int(out.item())
     if mx >= num_classes:
         raise ValueError(f"label {mx} >= num_classes {num_classes}")
+
+
+@dataclass
+class SectorThicknessOut:
+    """Exact sums of ``sector_thickness`` (device tensors) and what they were taken with."""
+    sums: torch.Tensor          # [V, G, 9, 5] int64: count, sum t, sum p, sum |t - p|, sum (t - p)^2 per (volume, group, sector)
+    maps: torch.Tensor | None   # [V, B, 2, G, W] int32 group thickness of y_true ([.., 0, ..]) / y_pred per A-scan
+    groups: tuple               # G (first, last) class pairs
+    spacing: tuple              # (sb, sy, sx)
+    num_classes: int
+    counts: torch.Tensor = field(repr=False)       # [V * B, K, K] confusion matrices of the label pass
+    pixels: int = field(repr=False, default=0)     # H * W
+
+    def bad_label_items(self):
+        """Items holding a label >= num_classes: their confusion counts do not add up to H * W (the label pass drops such
+        pixels, and their boundary rows are undefined)."""
+        n, k = self.counts.shape[0], self.counts.shape[-1]
+        cm = self.counts.cpu().numpy().view(np.uint64).reshape(n, k * k)      # n may be 0: an empty batch
+        return int((cm.sum(axis=1) != self.pixels).sum())
+
+    def _check(self):
+        bad = self.bad_label_items()
+        if bad:
+            raise ValueError(f"{bad} item(s) hold a label >= num_classes {self.num_classes}")
+
+    def integers(self):
+        """Host copies: ``sums`` int64 ``[V, G, 9, 5]`` and, with ``maps=True``, ``maps`` int32 ``[V, B, 2, G, W]``.
+        Raises ValueError when an item holds a label >= num_classes."""
+        self._check()
+        d = {"sums": self.sums.cpu().numpy()}
+        if self.maps is not None:
+            d["maps"] = self.maps.cpu().numpy()
+        return d
+
+    def metrics(self):
+        """``derive.sector_thickness``: float64 ``[V, G, 9]`` per-volume thickness, bias, MAE, RMSE and volumes in the
+        units of the spacing (sectors in ``derive.ETDRS_SECTORS`` order); ``derive.sector_thickness_summary`` of it gives
+        the dataset-level means."""
+        return derive.sector_thickness(self.integers()["sums"], self.spacing)
+
+
+def sector_thickness(y_true, y_pred, num_classes, spacing, *, center=None, radii=derive.ETDRS_RADII, classes=None,
+                     maps=False, timers=None):
+    """Layer thickness per ETDRS sector of OCT volumes (build-defined, no reference counterpart).
+
+    ``y_true`` / ``y_pred``: CUDA uint8 / bool ``[V, B, H, W]`` (V volumes of B B-scans) or ``[B, H, W]``.
+    ``spacing = (sb, sy, sx)``: B-scan distance, row (axial) and column (lateral) size, e.g. ``datasets.mhd_spacing``;
+    the grid is physical, so it is required.  ``center``: None (the geometric centre of every volume), one ``(cb, cx)``
+    pair or a ``[V, 2]`` array of fractional (B-scan, column) indices.  ``radii``: the three ring radii in the units of
+    the spacing (1, 3 and 6 mm diameters by default).  ``classes``: None (one group per class) or up to 16 classes or
+    ``(first, last)`` class runs, e.g. ``[(1, 7)]`` for the total retina of a layer map.
+
+    The thickness of a group in A-scan x is the number of its pixels in that column, ``b_{last+1}(x) - b_first(x)`` of
+    the label pass's boundary rows.  One label pass (``counts``, ``columns``, ``boundaries``), then
+    ``octm_sector_thickness_i32`` sums per (volume, group, sector) the A-scan count, sum t, sum p, sum |t - p| and
+    sum (t - p)^2 exactly; the region maps (``derive.etdrs_regions``) are built on the host and copied to the device.
+    ``maps=True`` also keeps every A-scan's t and p, the en-face thickness maps.  Reading the result raises ValueError
+    when an item holds a label >= num_classes."""
+    spacing = derive.spacing_3d(spacing)
+    radii = derive.etdrs_radii(radii)
+    k = int(num_classes)
+    groups = derive.sector_groups(classes, k)
+    for name, t in (("y_true", y_true), ("y_pred", y_pred)):
+        if not isinstance(t, torch.Tensor) or not t.is_cuda:
+            raise TypeError(f"{name} must be a CUDA torch tensor")
+    if y_true.shape != y_pred.shape:
+        raise ValueError(f"shape mismatch: {tuple(y_true.shape)} vs {tuple(y_pred.shape)}")
+    if y_true.dim() == 3:
+        y_true, y_pred = y_true[None], y_pred[None]
+    if y_true.dim() != 4:
+        raise ValueError("expected [V, B, H, W] or [B, H, W] label volumes")
+    v, b, h, w = y_true.shape
+    centers = derive.sector_centers(center, v, b, w)
+    lp = label_pass(y_true.reshape(v * b, h, w), y_pred.reshape(v * b, h, w), k, counts=True, columns=True,
+                    boundaries=True, timers=timers)
+    dev = lp.counts.device
+    uniq, inv = np.unique(centers, axis=0, return_inverse=True)
+    reg = np.stack([derive.etdrs_regions(b, w, spacing, c, radii) for c in uniq]) if v else np.zeros((0, b, w), np.uint8)
+    with torch.cuda.device(dev):
+        if len(uniq) == 1:          # one map for every volume: copy it once, repeat it on the device
+            region = torch.from_numpy(reg).to(dev).expand(v, b, w).contiguous()
+        else:
+            region = torch.from_numpy(np.ascontiguousarray(reg[inv.reshape(-1)])).to(dev)
+        g = len(groups)
+        nr = len(derive.ETDRS_SECTORS)
+        sums = torch.empty((v, g, nr, 5), dtype=torch.int64, device=dev)
+        thick = torch.empty((v, b, 2, g, w), dtype=torch.int32, device=dev) if maps else None
+        grp = (ctypes.c_int32 * (2 * g))(*[c for pair in groups for c in pair])
+        with _Timed(timers, "sector_thickness"):
+            _lib.call("octm_sector_thickness_i32", _ptr(lp.bnd_true), _ptr(lp.bnd_pred), v * b, k, h, w, b, _ptr(region),
+                      nr, grp, g, _ptr(sums), _ptr(thick), _stream())
+    return SectorThicknessOut(sums, thick, groups, spacing, k, lp.counts, h * w)
