@@ -15,7 +15,7 @@
  *   - label maps are uint8 [n_items][H][W], C-contiguous, values < K (2 <= K <= 16); a value >= K
  *     is undefined behaviour for the fast kernels (checked only by octm_validate_labels_u8).
  *   - return value: OCTM_OK or a negative OCTM_ERR_*; octm_last_error() gives the thread-local
- *     message of the last failure.
+ *     message of the last failure.  The one positive status is OCTM_PACK_WIDE_LABEL of the host packer.
  *   - outputs are fully overwritten (no pre-zeroing needed) unless stated otherwise.
  */
 #ifndef OCTM_H_
@@ -412,7 +412,11 @@ OCTM_API int octm_auc_u8(const uint8_t* y_true, const void* scores, int dtype, i
  *   octm_host_pack_nibbles   HOST function: dst[i] = src[2i] | src[2i+1] << 4 for n_labels labels
  *                            (dst holds (n_labels + 1) / 2 bytes), on `threads` host threads (<= 0: all cores).
  *                            A data-format conversion only; no metric arithmetic runs on the host.
+ *                            Returns OCTM_PACK_WIDE_LABEL (not an error) when some src byte is >= 16: such a
+ *                            label has no 4-bit code, dst does not encode src, and the caller must send src as
+ *                            it is (a transfer encoding must never change a result).
  *   octm_unpack_nibbles_u8   device kernel: the inverse, packed (device) -> labels uint8 [n_labels] (device). */
+#define OCTM_PACK_WIDE_LABEL 1    /* octm_host_pack_nibbles: a label >= 16 was seen, dst is not usable */
 OCTM_API int octm_host_pack_nibbles(const uint8_t* src, uint8_t* dst, size_t n_labels, int threads);
 OCTM_API int octm_unpack_nibbles_u8(const uint8_t* packed, int64_t n_labels, uint8_t* labels, void* stream);
 

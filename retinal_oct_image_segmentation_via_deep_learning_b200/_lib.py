@@ -13,6 +13,7 @@ _PKG = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_PKG, "liboctm.so")
 
 OK = 0
+PACK_WIDE_LABEL = 1       # octm_host_pack_nibbles: a label >= 16 has no 4-bit code, the packed bytes are unusable
 NO_SEED = 0xFFFFFFFF
 CF_TRUE_CLOSED, CF_PRED_CLOSED, CF_TRUE_OVERFLOW, CF_PRED_OVERFLOW = 1, 2, 4, 8
 # column order of the device-derived per-class metrics (OCTM_M_* in include/octm.h)

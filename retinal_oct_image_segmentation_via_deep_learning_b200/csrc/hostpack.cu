@@ -16,17 +16,25 @@
 
 namespace octm {
 
-static void pack_scalar(const uint8_t* src, uint8_t* dst, size_t b, size_t e) {
-    for (size_t i = b; i + 2 <= e; i += 2) dst[i >> 1] = static_cast<uint8_t>((src[i] & 15u) | (src[i + 1] << 4));
+// Both packers return the OR of the labels they read: a value >= 16 means that some label has no 4-bit code.
+static uint32_t pack_scalar(const uint8_t* src, uint8_t* dst, size_t b, size_t e) {
+    uint32_t seen = 0;
+    for (size_t i = b; i + 2 <= e; i += 2) {
+        seen |= src[i] | src[i + 1];
+        dst[i >> 1] = static_cast<uint8_t>((src[i] & 15u) | (src[i + 1] << 4));
+    }
+    return seen;
 }
 
-__attribute__((target("avx2"))) static void pack_avx2(const uint8_t* src, uint8_t* dst, size_t b, size_t e) {
+__attribute__((target("avx2"))) static uint32_t pack_avx2(const uint8_t* src, uint8_t* dst, size_t b, size_t e) {
     size_t i = b;
     const __m256i lo8 = _mm256_set1_epi16(0x00ff);
+    __m256i seen = _mm256_setzero_si256();
     const bool aligned = (reinterpret_cast<uintptr_t>(dst + (b >> 1)) & 31u) == 0;
     for (; i + 64 <= e; i += 64) {
         const __m256i a = _mm256_loadu_si256(reinterpret_cast<const __m256i*>(src + i));
         const __m256i c = _mm256_loadu_si256(reinterpret_cast<const __m256i*>(src + i + 32));
+        seen = _mm256_or_si256(seen, _mm256_or_si256(a, c));
         // per 16-bit lane (even byte, odd byte): even | odd << 4 in the low byte
         __m256i pa = _mm256_and_si256(_mm256_or_si256(a, _mm256_srli_epi16(a, 4)), lo8);
         __m256i pc = _mm256_and_si256(_mm256_or_si256(c, _mm256_srli_epi16(c, 4)), lo8);
@@ -34,8 +42,9 @@ __attribute__((target("avx2"))) static void pack_avx2(const uint8_t* src, uint8_
         if (aligned) _mm256_stream_si256(reinterpret_cast<__m256i*>(dst + (i >> 1)), p);      // written once, read by DMA
         else _mm256_storeu_si256(reinterpret_cast<__m256i*>(dst + (i >> 1)), p);
     }
-    pack_scalar(src, dst, i, e);
+    const uint32_t tail = pack_scalar(src, dst, i, e);
     _mm_sfence();
+    return tail | (_mm256_testz_si256(seen, _mm256_set1_epi8(static_cast<char>(0xf0))) ? 0u : 16u);
 }
 
 // 16 packed bytes -> 32 labels
@@ -79,13 +88,21 @@ extern "C" int octm_host_pack_nibbles(const uint8_t* src, uint8_t* dst, size_t n
     const size_t even = n_labels & ~static_cast<size_t>(1);
     size_t per = ((even / threads) + 63) & ~static_cast<size_t>(63);
     if (per < (1u << 16)) per = 1u << 16;                      // not worth a thread below 64 KB
-    auto work = [&](size_t b, size_t e) { have_avx2 ? octm::pack_avx2(src, dst, b, e) : octm::pack_scalar(src, dst, b, e); };
+    std::vector<uint32_t> seen((even + per - 1) / per + 1, 0u);      // one slot per thread: no shared writes
+    auto work = [&](size_t t, size_t b, size_t e) {
+        seen[t] = have_avx2 ? octm::pack_avx2(src, dst, b, e) : octm::pack_scalar(src, dst, b, e);
+    };
     std::vector<std::thread> pool;
-    for (size_t b = per; b < even; b += per) pool.emplace_back(work, b, b + per < even ? b + per : even);
-    work(0, per < even ? per : even);
+    for (size_t b = per; b < even; b += per) pool.emplace_back(work, b / per, b, b + per < even ? b + per : even);
+    work(0, 0, per < even ? per : even);
     for (auto& t : pool) t.join();
-    if (n_labels & 1) dst[n_labels >> 1] = src[n_labels - 1] & 15u;
-    return OCTM_OK;
+    uint32_t any = 0;
+    for (uint32_t v : seen) any |= v;
+    if (n_labels & 1) {
+        any |= src[n_labels - 1];
+        dst[n_labels >> 1] = src[n_labels - 1] & 15u;
+    }
+    return any >= 16u ? OCTM_PACK_WIDE_LABEL : OCTM_OK;
 }
 
 extern "C" int octm_unpack_nibbles_u8(const uint8_t* packed, int64_t n_labels, uint8_t* labels, void* stream) {

@@ -903,10 +903,12 @@ def evaluate_host(y_true, y_pred, num_classes, *, contours=True, device=None, ch
         freed = [None, None]
         starts = list(range(0, n, chunk_items))
         ready = {}
+        packed = {}        # chunk -> sent two labels per byte (False: a label >= 16 sent it as it is)
 
         def issue_copy(ci):
             s0, e0 = starts[ci], min(n, starts[ci] + chunk_items)
             bt, bp = bufs[ci & 1]
+            packed[ci] = use_pack
             if use_pack:
                 b = ci & 1
                 if h2d_done[b] is not None:
@@ -914,12 +916,17 @@ def evaluate_host(y_true, y_pred, num_classes, *, contours=True, device=None, ch
                 m = (e0 - s0) * h * w
                 for k, src in ((0, ht), (1, hp)):
                     rc = lib.octm_host_pack_nibbles(src[s0:e0].data_ptr(), hpk[2 * b + k].data_ptr(), m, int(pack_threads))
+                    if rc == _lib.PACK_WIDE_LABEL:
+                        # no 4-bit code for this label: the chunk goes as it is, so that validate / the label pass
+                        # see exactly what pack=False gives them
+                        packed[ci] = False
+                        break
                     if rc != 0:
                         raise _lib.OctmError("octm_host_pack_nibbles failed")
             with torch.cuda.stream(copy):
                 if freed[ci & 1] is not None:
                     copy.wait_event(freed[ci & 1])               # kernels of chunk ci-2 are done with it
-                if use_pack:
+                if packed[ci]:
                     nb = (m + 1) // 2
                     dpk[2 * b][:nb].copy_(hpk[2 * b][:nb], non_blocking=True)
                     dpk[2 * b + 1][:nb].copy_(hpk[2 * b + 1][:nb], non_blocking=True)
@@ -952,7 +959,7 @@ def evaluate_host(y_true, y_pred, num_classes, *, contours=True, device=None, ch
                 issue_copy(ci + 1)                               # overlaps the kernels launched below
             bt, bp = bufs[ci & 1]
             compute.wait_event(ready.pop(ci))
-            if use_pack:
+            if packed.pop(ci):
                 expand(ci)
             parts.append(evaluate(bt[:e0 - s0], bp[:e0 - s0], num_classes, contours=contours, max_pts=max_pts,
                                   validate=validate, surface_dice=surface_dice, components=components,

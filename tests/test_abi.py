@@ -87,3 +87,23 @@ def test_host_nibble_packer(lib):
         if n & 1:
             ref[-1] = src[-1]
         assert np.array_equal(dst[:(n + 1) // 2], ref) and (dst[(n + 1) // 2:] == 0xAA).all()
+
+    # A label >= 16 has no 4-bit code: the packer must say so (OCTM_PACK_WIDE_LABEL = 1) wherever it sits, in the
+    # AVX2 body (64-label blocks), the scalar tail, the odd last label, and in the chunk of any thread (3 threads,
+    # at least 64 Ki labels each).
+    n = 3 * (1 << 17) + 37
+    base = rng.integers(0, 16, n, dtype=np.uint8)
+    dst = np.empty((n + 1) // 2, np.uint8)
+    assert so.octm_host_pack_nibbles(base.ctypes.data, dst.ctypes.data, n, 3) == 0
+    tail = n - (n & 1) - (n - (n & 1)) % 64          # first label of the last thread's scalar tail
+    for at in (0, 1, 62, 63, 1 << 17, (1 << 17) + 5, 2 << 17, 3 << 17, tail, tail + 1, n - 2, n - 1):
+        for bad in (16, 17, 128, 255):
+            src = base.copy()
+            src[at] = bad
+            assert so.octm_host_pack_nibbles(src.ctypes.data, dst.ctypes.data, n, 3) == 1, (at, bad)
+            assert so.octm_host_pack_nibbles(src.ctypes.data, dst.ctypes.data, n, 1) == 1, (at, bad)
+    for n in (1, 2, 3, 64, 65):                      # scalar only, one AVX2 block, a block and a tail
+        for at in range(n):
+            src = np.zeros(n, np.uint8)
+            src[at] = 16
+            assert so.octm_host_pack_nibbles(src.ctypes.data, dst.ctypes.data, n, 0) == 1, (n, at)
