@@ -162,7 +162,8 @@ def boundary_error(bnd_true, bnd_pred):
 
     Integer positions (e.g. ``b_k(x)`` extracted from label maps) give exact int64 sums; floating
     positions (the soft-argmax rows a layer model such as SD-LayerNet's ``LayerEngine`` produces) give
-    float64 sums accumulated in a fixed order."""
+    float64 sums accumulated in a fixed order.  A NaN position makes its row's sums NaN and an infinite one inf (NaN
+    for inf - inf), as numpy's ``mean`` of the reference does."""
     if bnd_true.shape != bnd_pred.shape or bnd_true.dim() != 3:
         raise ValueError("expected two [N, Kb, W] tensors of equal shape")
     n, kb, w = bnd_true.shape
@@ -183,20 +184,43 @@ def boundary_error(bnd_true, bnd_pred):
     return sq, ab
 
 
+_I32_NEVER = 2**31 - 1       # an int32 threshold no row y < H reaches; its negation is reached by every row
+
+
+def _raster_rows(boundaries):
+    """Boundary rows (any device) -> ``(rows, dtype code)`` for ``octm_labels_from_boundaries``, contiguous, with the
+    same set of rows ``0 <= y < 2**31 - 1`` satisfying ``b <= y`` as the caller's values.  float16 / bfloat16 /
+    float32 rows are exact as float32, and bool / int8 / uint8 / int16 / uint16 / int32 as int32.  float64 rows become
+    ``ceil(b)`` (``y >= b`` <=> ``y >= ceil(b)`` for integer ``y``), and uint32 / int64 / uint64 stay as they are; both
+    are clamped to ``[-(2**31 - 1), 2**31 - 1]`` and sent as int32, NaN (boundary absent) as ``2**31 - 1``.  The kernel
+    counts ``2**31 - 1`` for no row and ``-(2**31 - 1)`` for every row, as it does +inf and -inf.  No device sync."""
+    b = boundaries
+    if b.is_floating_point() and b.dtype != torch.float64:
+        return b.to(torch.float32).contiguous(), _lib.DTYPE_F32
+    if b.dtype == torch.float64:
+        b = torch.nan_to_num(torch.ceil(b), nan=_I32_NEVER)
+    elif b.dtype == torch.uint64:
+        b = b.view(torch.int64)
+        b = torch.where(b < 0, _I32_NEVER, b)            # values >= 2**63
+    elif b.dtype in (torch.int64, torch.uint32):
+        b = b.to(torch.int64)
+    else:
+        return b.to(torch.int32).contiguous(), _lib.DTYPE_I32
+    return b.clamp(-_I32_NEVER, _I32_NEVER).to(torch.int32).contiguous(), _lib.DTYPE_I32
+
+
 def labels_from_boundaries(boundaries, height):
     """Boundary rows ``[N, Kb, W]`` (int or float, CUDA) -> uint8 label maps ``[N, height, W]``:
-    ``label[i, y, x] = #{k : b_k(i, x) <= y}``.  The inverse of the label pass's boundary rows on layered maps;
-    this is how boundary-curve annotations (Duke ``manualLayers``, HC-MS control points, the soft rows of a layer
-    model) become inputs of the mask metrics.  Rows may be unsorted, out of range or NaN (= boundary absent)."""
+    ``label[i, y, x] = #{k : b_k(i, x) <= y}`` on the values passed, float64 and int64 included (``_raster_rows``).
+    The inverse of the label pass's boundary rows on layered maps; this is how boundary-curve annotations (Duke
+    ``manualLayers``, HC-MS control points, the soft rows of a layer model) become inputs of the mask metrics.
+    Rows may be unsorted, out of range or NaN (= boundary absent)."""
     if not isinstance(boundaries, torch.Tensor) or not boundaries.is_cuda or boundaries.dim() != 3:
         raise TypeError("expected a CUDA tensor [N, Kb, W]")
     n, kb, w = boundaries.shape
     if kb > 15:
         raise ValueError("at most 15 boundaries (16 classes)")
-    if boundaries.is_floating_point():
-        b, dt = boundaries.to(torch.float32).contiguous(), _lib.DTYPE_F32
-    else:
-        b, dt = boundaries.to(torch.int32).contiguous(), _lib.DTYPE_I32
+    b, dt = _raster_rows(boundaries)
     out = torch.empty((n, int(height), w), dtype=torch.uint8, device=b.device)
     with torch.cuda.device(b.device):
         _lib.call("octm_labels_from_boundaries", _ptr(b), dt, n, kb, int(height), w, _ptr(out), _stream())
@@ -215,7 +239,9 @@ def boundary_metrics(bnd_true, bnd_pred):
 
 def topology_violations(positions):
     """``relu(pos[:, :-1] - pos[:, 1:])`` of ``LayerEngine.get_topology_violations`` (SD_Layer_Net/layer_engine.py:74-76),
-    reduced over the width: ``(sum_violation float64 [N, Kb-1], n_violations int32 [N, Kb-1])``."""
+    reduced over the width: ``(sum_violation float64 [N, Kb-1], n_violations int32 [N, Kb-1])``.  A column where
+    either position is NaN (boundary absent) counts in neither the sum nor the count, where the reference's ``relu``
+    would propagate the NaN."""
     if not isinstance(positions, torch.Tensor) or not positions.is_cuda or positions.dim() != 3:
         raise TypeError("positions must be a CUDA tensor [N, Kb, W]")
     pos = positions if positions.is_floating_point() else positions.to(torch.float64)

@@ -9,7 +9,9 @@ from retinal_oct_image_segmentation_via_deep_learning_b200 import suite, synth
 pytestmark = pytest.mark.gpu
 
 
-@pytest.mark.parametrize("n,h,w,kb", [(3, 60, 48, 4), (2, 496, 512, 7), (2, 33, 50, 3), (1, 17, 7, 15), (2, 40, 1032, 9)])
+@pytest.mark.parametrize("n,h,w,kb", [(3, 60, 48, 4), (2, 496, 512, 7), (2, 33, 50, 3), (1, 17, 7, 15), (2, 40, 1032, 9)]
+                         # V = 4 strips (w % 4 == 0) and byte columns at small and ragged widths, 0 to 15 boundaries
+                         + [(2, 37, w, kb) for w in (1, 3, 4, 8, 513, 2048) for kb in (0, 1, 15)])
 def test_int_boundaries(cuda, n, h, w, kb):
     rng = np.random.default_rng(n * 1000 + w)
     b = rng.integers(-3, h + 4, size=(n, kb, w)).astype(np.int32)           # unsorted, partly outside [0, H]
